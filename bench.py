@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of BASELINE.json ("x4 RRDBNet LR Mpix/s + degraded pairs/s at 1/2/4/8 B200, % of roofline").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--precision fp16|bf16]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--precision fp16|bf16] [--dump-outputs DIR]
 
 Our arm (default). One step = one RRDBNet x4 forward of the 64x3x128x128 LR batch of BASELINE.json configs[2], batch-
 sharded over the N ranks (64 / N images per rank: STRONG scaling, the configuration BASELINE names; no collective on the
@@ -18,6 +18,9 @@ data path). Rank 0 prints ONE JSON line:
   training      secondary, configs[3]: degradation + generator forward / L1 / backward (+ NCCL all-reduce) per GPU
 `--impl reference`: the reference's own CPU implementation of the path (oracle port; /root/reference does not exist on
 the GPU box) timed on the host cores, one 1x3x128x128 image per step.
+`--dump-outputs DIR`: after the timed steps, the SR batch of the last timed step (rank 0's shard) goes to DIR/sr.npy in
+float32 (over 48 MiB: a fixed, seeded choice of whole images, 16 of the 64 at N = 1), so that two builds can be compared
+output for output: inputs and weights are seeded, identical in every run with the same arguments.
 """
 import argparse
 import json
@@ -163,6 +166,21 @@ def timed(fn, steps, D, fin=None, warm=0):
     ms = a.elapsed_time(b) / steps
     D.barrier()
     return ms
+
+
+DUMP_BYTES = 48 << 20   # the arrays of one --dump-outputs run stay under 64 MB
+
+
+def dump_output(out_dir, name, y):
+    """Writes y (images along dim 0) as out_dir/<name>.npy in float32. An output larger than DUMP_BYTES is cut to a
+    seeded choice of whole images, the same in every run; returns its shape and the images kept."""
+    n, per_image = y.shape[0], y[0].numel() * 4
+    idx = torch.arange(n)
+    if n * per_image > DUMP_BYTES:
+        idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_BYTES // per_image].sort().values
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), y.detach()[idx.to(y.device)].float().cpu().numpy())
+    return {name: {"shape": list(y.shape), "images": idx.tolist()}}
 
 
 # ------------------------------------------------------------------------------------------------- CPU baselines
@@ -609,7 +627,7 @@ def run_reference(args):
         og.generator_forward(x, sd)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        og.generator_forward(x, sd)
+        y = og.generator_forward(x, sd)
     dt = (time.perf_counter() - t0) / args.steps
     val = 128 * 128 / dt / 1e6
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": "LR Mpix/s", "n_gpus": args.gpus,
@@ -620,6 +638,8 @@ def run_reference(args):
             "cpu_baseline": {"value": val, "unit": "LR Mpix/s", "cores": torch.get_num_threads(), "kind": "port",
                              "sample": "1x3x128x128 fp32 forward per step, oracle port of model.py (reference tree is not on the GPU box)"},
             "e2e": {"value": val, "unit": "LR Mpix/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
+    if args.dump_outputs:
+        line["dump_outputs"] = dump_output(args.dump_outputs, "sr", y)
     try:  # secondary: the degradation half of the metric on the same host cores (numpy port, bounded sample)
         import resr_b200
         from oracle import kernels as ok
@@ -681,9 +701,11 @@ def run_ours(args):
         ms, ms_block, ms_pipe = D.max_ms(ms, ms_block, ms_pipe)
         return {"n": n, "ms": ms, "ms_block": ms_block, "ms_pipe": ms_pipe, "clocks": clocks.summary(),
                 "h2d": x_host.numel() * 4, "d2h": y_hosts[0].numel() * 4,
-                "checksum": float(y_hosts[0][0, :, ::64, ::64].double().sum())}
+                "checksum": float(y_hosts[0][0, :, ::64, ::64].double().sum()), "y": state["y"]}
 
     head = forward_leg(n_strong)
+    dumped = dump_output(args.dump_outputs, "sr", head["y"]) if args.dump_outputs and rank == 0 else None
+    head["y"] = None
     weak = forward_leg(TOTAL_BATCH) if (world > 1 and not args.batch and not args.no_weak) else None
     # the other precision recipe on the same box, device-resident only (north_star names bf16; fp16 is the default)
     other = "bf16" if args.precision == "fp16" else "fp16"
@@ -735,6 +757,8 @@ def run_ours(args):
                                    "35,853,696 per LR pixel)",
                          "peak_source": peaks["source"] + " bf16_tflops_sustained (kernel timed inside a long step), x n_gpus"},
         }
+        if dumped is not None:
+            line["dump_outputs"] = dumped
         if weak is not None:
             wpx = world * weak["n"] * H * W
             line["weak"] = {"value": wpx / (weak["ms"] * 1e-3) / 1e6, "unit": "LR Mpix/s", "ms_per_step": weak["ms"],
@@ -836,7 +860,11 @@ DEGRADE_LAUNCHES = 15
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, metavar="K",
+                    help="timed steps of the headline leg (the one --dump-outputs writes); the secondary legs clamp it to "
+                         "their own counts: e2e max(4, min(K, 10)), other precision max(3, K // 2), degradation max(20, K) "
+                         "(large batch: 10), training max(5, min(K, 20)) (other precision: max(5, min(K, 10))), tiled 2 "
+                         "(3 for N > 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--precision", default="fp16", choices=["fp16", "bf16"],
@@ -850,7 +878,10 @@ def main():
     ap.add_argument("--no-tiled", action="store_true", help="skip the secondary tiled-inference leg (configs[4])")
     ap.add_argument("--no-degrade", action="store_true", help="skip the secondary degradation leg")
     ap.add_argument("--no-train", action="store_true", help="skip the secondary training-step leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the SR batch of the last timed step to DIR/sr.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

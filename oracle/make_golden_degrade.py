@@ -3,8 +3,14 @@
 degrade_ops.npz    per-op input/output pairs of imgproc.filter2d_torch / USMSharp / DiffJPEG / F.interpolate /
                    random_add_{gaussian,poisson}_noise_torch with the random tensors recorded
 degrade_block.npz  whole-block executions of train_realesrnet.py:267-377 (exec of the literal source lines) for
-                   several seeds: inputs, blur kernels, recorded plan, every stage output, final (lr, hr)
+                   several seeds: blur kernels, recorded plan, every stage output, final lr
+
+Each file stays under 1 MB. The input images are not stored: smooth_image regenerates them from their seeds, and
+load_ops / load_block check them bit for bit against the SHA-256 digest stored beside. The stage outputs of the block
+are stored on the sub-grid STAGE_GRID (every second row and column). The reference's hr crop is not stored either:
+it is hr[..., hr_top:hr_top + image_size, hr_left:hr_left + image_size] of the recorded plan.
 """
+import hashlib
 import math
 import os
 import random
@@ -66,6 +72,40 @@ def smooth_image(b, h, w, seed):
     return x.clamp(0, 1).contiguous()
 
 
+STAGE_GRID = (Ellipsis, slice(None, None, 2), slice(None, None, 2))
+OPS_INPUTS = {"f2d_x": (2, 48, 56, 1), "usm_x": (1, 72, 88, 2), "jpeg_x": (3, 40, 52, 4)}   # key: smooth_image arguments
+
+
+def digest(a):
+    return np.array(hashlib.sha256(np.ascontiguousarray(a, np.float32).tobytes()).hexdigest())
+
+
+def _regenerated(z, key, args):
+    x = smooth_image(*args).numpy()
+    if str(digest(x)) != str(z[key + "_sha256"]):
+        raise AssertionError(f"{key}: smooth_image{args} no longer reproduces the stored input")
+    return x
+
+
+def load_ops(path):
+    """degrade_ops.npz as a dict, with the input images regenerated and checked."""
+    z = dict(np.load(path))
+    for key, args in OPS_INPUTS.items():
+        z[key] = _regenerated(z, key, args)
+    return z
+
+
+def load_block(path):
+    """degrade_block.npz as a dict, with every seed's hr regenerated and checked and its hr crop cut out of it."""
+    z = dict(np.load(path))
+    for seed in z["seeds"]:
+        tag = f"s{seed}."
+        hr = _regenerated(z, tag + "hr", (2, 64, 72, 100 + int(seed)))
+        top, left, size = (int(z[tag + "plan.crop." + k]) for k in ("hr_top", "hr_left", "image_size"))
+        z[tag + "hr"], z[tag + "hr_crop"] = hr, hr[:, :, top:top + size, left:left + size]
+    return z
+
+
 def make_ops(imgproc, config, out_dir):
     z = {}
     torch.manual_seed(11)
@@ -96,6 +136,8 @@ def make_ops(imgproc, config, out_dir):
     z["jpeg_factor"] = qq.numpy()
     _, parts = od.jpeg(xj.numpy(), q.numpy(), return_parts=True)
     z["jpeg_qy_oracle"], z["jpeg_qcb_oracle"], z["jpeg_qcr_oracle"] = parts["y_q"], parts["cb_q"], parts["cr_q"]
+    for key in OPS_INPUTS:
+        z[key + "_sha256"] = digest(z.pop(key))
     np.savez_compressed(os.path.join(out_dir, "degrade_ops.npz"), **z)
     print("degrade_ops.npz written")
 
@@ -112,7 +154,7 @@ def flatten_plan(prefix, plan, z):
 
 def unflatten_plan(z, prefix):
     plan = {}
-    for key in z.files:
+    for key in z:
         if not key.startswith(prefix):
             continue
         parts = key[len(prefix):].split(".")
@@ -139,12 +181,14 @@ def make_block(imgproc, config, out_dir):
         k1, k2, sk = batch_kernels(imgproc, config, b, seed)
         plan, stages, lr, hr_c = oplan.record_reference_plan(hr, k1, k2, sk, seed)
         tag = f"s{seed}."
-        z[tag + "hr"], z[tag + "k1"], z[tag + "k2"], z[tag + "sk"] = hr.numpy(), k1.numpy(), k2.numpy(), sk.numpy()
+        assert np.array_equal(hr_c, hr.numpy()[:, :, plan["crop"]["hr_top"]:plan["crop"]["hr_top"] + config.image_size,
+                                               plan["crop"]["hr_left"]:plan["crop"]["hr_left"] + config.image_size])
+        z[tag + "hr_sha256"], z[tag + "k1"], z[tag + "k2"], z[tag + "sk"] = digest(hr.numpy()), k1.numpy(), k2.numpy(), sk.numpy()
         flatten_plan(tag + "plan.", plan, z)
         z[tag + "stage_names"] = np.array([s[0] for s in stages])
         for name, xin, yout in stages:
-            z[tag + "out." + name] = yout.astype(np.float32)
-        z[tag + "lr"], z[tag + "hr_crop"] = lr, hr_c
+            z[tag + "out." + name] = np.ascontiguousarray(yout.astype(np.float32)[STAGE_GRID])
+        z[tag + "lr"] = lr
         kept.append(seed)
         print(f"seed {seed}: blur1={plan['blur1']} r1={plan['resize1']['mode']}/{plan['resize1']['out_h']}x{plan['resize1']['out_w']} "
               f"n1={plan['noise1']['type']} blur2={plan['blur2']} r2={plan['resize2']['mode']}/{plan['resize2']['out_h']}x{plan['resize2']['out_w']} "
