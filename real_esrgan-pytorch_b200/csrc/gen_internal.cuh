@@ -101,6 +101,7 @@ struct resr_generator {
     cudaGraphExec_t step_exec = nullptr;
     const void* step_key[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
     int step_shape[3] = {0, 0, 0};
+    int step_precision = -1;      // recipe the graph was captured under: its kernels and pack formats are that recipe's
     bool step_graph_failed = false;
     // pipelined host path (generator.cu): copy streams, per-slot events, call counter
     cudaStream_t h2d_stream = nullptr, d2h_stream = nullptr;

@@ -564,6 +564,13 @@ int resr_generator_set_precision(resr_generator_t* g, int precision) {
         g->plan.valid = false;
         cudaFree(g->pack_jobs);   // the batched pack table carries the operand format
         g->pack_jobs = nullptr;
+        // the captured training step launches the old recipe's kernels: capture it again under the new one
+        if (g->step_exec) cudaGraphExecDestroy(g->step_exec);
+        g->step_exec = nullptr;
+        memset(g->step_key, 0, sizeof(g->step_key));
+        memset(g->step_shape, 0, sizeof(g->step_shape));
+        g->step_precision = -1;
+        g->step_graph_failed = false;
     }
     return RESR_OK;
 }

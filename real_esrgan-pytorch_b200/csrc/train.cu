@@ -749,7 +749,7 @@ int resr_generator_train_step_l1(resr_generator_t* g, const float* x, const floa
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const void* key[6] = {x, hr, y, grads_flat, loss_out, workspace};
     const bool same = g->step_exec && memcmp(key, g->step_key, sizeof(key)) == 0 && g->step_shape[0] == n && g->step_shape[1] == h &&
-                      g->step_shape[2] == w;
+                      g->step_shape[2] == w && g->step_precision == g->precision;
     if (same) {
         const cudaError_t e = cudaGraphLaunch(g->step_exec, s);
         if (e != cudaSuccess) return set_error(RESR_E_CUDA, "cudaGraphLaunch: %s", cudaGetErrorString(e));
@@ -780,6 +780,7 @@ int resr_generator_train_step_l1(resr_generator_t* g, const float* x, const floa
     if (ei != cudaSuccess) { cudaGetLastError(); g->step_exec = nullptr; g->step_graph_failed = true; return RESR_OK; }
     memcpy(g->step_key, key, sizeof(key));
     g->step_shape[0] = n; g->step_shape[1] = h; g->step_shape[2] = w;
+    g->step_precision = g->precision;
     return RESR_OK;
 }
 

@@ -5,6 +5,7 @@ import os
 import numpy as np
 import pytest
 import torch
+import torch.nn.functional as F
 
 from oracle import degrade as od
 from oracle import generator as og
@@ -222,3 +223,73 @@ def test_niqe_oracle_matches_reference_golden():
             r = np.array(sorted(map(tuple, ref_feat[b])))
             assert np.abs(a - r).max() <= 1e-6
         assert np.abs(score - g[f"niqe{ci}"]).max() <= 1e-5 * g[f"niqe{ci}"].max()
+
+
+def test_oracle_grads_without_formats_is_float64_autograd():
+    """grads() with no formats is float64 autograd of the oracle forward (l1_loss_and_grads casts to float32, so it is
+    only checked to fp32 accuracy)."""
+    sd = og.rich_state_dict(5)
+    torch.manual_seed(5)
+    x, hr = torch.rand(1, 3, 4, 6), torch.rand(1, 3, 16, 24)
+    loss, g, sr = og.grads(x, sd, lambda y: torch.nn.functional.l1_loss(y, hr.double()))
+    params = {k: v.double().requires_grad_(True) for k, v in sd.items()}
+    sr64 = og._forward(x.double(), params, 23)
+    loss64 = torch.nn.functional.l1_loss(sr64, hr.double())
+    loss64.backward()
+    assert loss.dtype == torch.float64 and torch.equal(loss, loss64.detach()) and torch.equal(sr, sr64.detach())
+    assert list(g) == list(sd) and all(torch.equal(g[k], params[k].grad) for k in sd)
+    loss32, g32, _ = og.l1_loss_and_grads(x, hr, sd)
+    assert abs(loss32.item() - loss.item()) <= 1e-5 * loss.item()
+    flat, flat32 = torch.cat([g[k].reshape(-1) for k in sd]), torch.cat([g32[k].reshape(-1).double() for k in sd])
+    assert float((flat32 - flat).norm() / flat.norm()) <= 1e-4
+
+
+def test_oracle_recipe_rounding_points():
+    """On one convolution: the forward multiplies operands rounded to the operand format (the bias is not rounded); the
+    output gradient is rounded to the gradient format, and the data and weight gradients multiply it with the weights
+    and the input rounded to the backward format."""
+    torch.manual_seed(6)
+    x = (torch.randn(2, 5, 6, 7, dtype=torch.float64) * 3).requires_grad_(True)
+    p = {"c.weight": torch.randn(4, 5, 3, 3, dtype=torch.float64).requires_grad_(True),
+         "c.bias": torch.randn(4, dtype=torch.float64).requires_grad_(True)}
+    r = torch.randn(2, 4, 6, 7, dtype=torch.float64)
+    q = lambda t, fmt: t.detach().to(fmt).double()
+    for ofmt, bfmt in ((torch.float16, torch.bfloat16), (torch.bfloat16, torch.bfloat16), (torch.float16, torch.float16)):
+        for t in (x, *p.values()):
+            t.grad = None
+        y = og.recipe_conv(ofmt, torch.bfloat16, bfmt)(x, p, "c")
+        (y * r).sum().backward()
+        rq = q(r, torch.bfloat16)
+        assert not torch.equal(q(x, ofmt), x.detach()) and not torch.equal(rq, r)
+        assert torch.allclose(y, F.conv2d(q(x, ofmt), q(p["c.weight"], ofmt), p["c.bias"].detach(), padding=1), rtol=1e-14, atol=1e-12)
+        gx = torch.nn.grad.conv2d_input(x.shape, q(p["c.weight"], bfmt), rq, padding=1)
+        gw = torch.nn.grad.conv2d_weight(q(x, bfmt), p["c.weight"].shape, rq, padding=1)
+        assert torch.allclose(x.grad, gx, rtol=1e-12, atol=1e-12)
+        assert torch.allclose(p["c.weight"].grad, gw, rtol=1e-12, atol=1e-12)
+        assert torch.equal(p["c.bias"].grad, rq.sum((0, 2, 3)))
+        if bfmt != ofmt:   # the backward format is not the forward one
+            assert not torch.allclose(x.grad, torch.nn.grad.conv2d_input(x.shape, q(p["c.weight"], ofmt), rq, padding=1), rtol=1e-6)
+    # backward format defaults to the operand format; no formats: the plain convolution
+    for t in (x, *p.values()):
+        t.grad = None
+    (og.recipe_conv(torch.float16, torch.bfloat16)(x, p, "c") * r).sum().backward()
+    assert torch.allclose(x.grad, torch.nn.grad.conv2d_input(x.shape, q(p["c.weight"], torch.float16), q(r, torch.bfloat16), padding=1),
+                          rtol=1e-12, atol=1e-12)
+    y = og.recipe_conv()(x, p, "c")
+    assert torch.equal(y, F.conv2d(x, p["c.weight"], p["c.bias"], padding=1))
+
+
+def test_rich_state_dict_adds_nonzero_biases_only():
+    sd0, sd = og.random_state_dict(3), og.rich_state_dict(3)
+    assert list(sd) == list(sd0)
+    for k in sd:
+        assert sd[k].dtype == torch.float32 and sd[k].shape == sd0[k].shape
+        if k.endswith(".weight"):
+            assert torch.equal(sd[k], sd0[k])
+        else:
+            cin = sd[k[:-len("bias")] + "weight"].shape[1]
+            assert bool((sd[k] != 0).all()), k
+            assert float(sd[k].abs().max()) <= 1.0 / (9 * cin) ** 0.5 or k == "conv4.bias"
+    assert sd["conv4.bias"].tolist() == pytest.approx([-0.02, 0.5, 1.02])
+    assert float(og.random_state_dict(3)["trunk.0.rdb1.conv1.bias"].abs().max()) == 0.0
+    assert not torch.equal(og.rich_state_dict(4)["trunk.0.rdb1.conv1.bias"], sd["trunk.0.rdb1.conv1.bias"])
