@@ -96,6 +96,26 @@ int resr_generator_forward_host_async(resr_generator_t* g, const float* x_host, 
 /* Waits for every queued async call of this handle (copies included). */
 int resr_generator_host_sync(resr_generator_t* g);
 
+/* A list of differently sized images as ONE packed forward. The reference's image loops (test.py, validate() in
+ * train_realesrnet.py / train_realesrgan.py, inference.py over a directory) pass images one at a time; each then pays the
+ * full chain of launches at a size that leaves most SMs idle. Here the images are packed into one N = 1 canvas with a
+ * zero LR pixel between neighbours, and every convolution writes 0 outside the images, so each result is that image's
+ * own forward (DESIGN.md §3.2, packed canvas).
+ *
+ * resr_canvas_pack: the deterministic shelf packer (host only, no device). hs / ws: count image sizes (1..16384 per side);
+ * max_width: widest canvas row of images, <= 0 for a near-square canvas. Returns each image's LR offset (x0, y0) and the
+ * canvas size, rounded up to a multiple of 16 rows and 128 columns. Rectangles plus a one-pixel gutter do not overlap.
+ * resr_generator_forward_many(_workspace_bytes): xs[i] is image i, fp32 NCHW [1,3,hs[i],ws[i]]; ys[i] receives
+ * clamp(G(xs[i]), 0, 1), fp32 NCHW [1,3,4hs[i],4ws[i]]. _u8: NHWC u8 [hs[i],ws[i],3] in, [4hs[i],4ws[i],3] out, with the
+ * conversions of resr_generator_forward_u8. The pointer and size ARRAYS are host memory, the images device memory;
+ * count is 1..65535. Plans are cached per canvas size beside the single-shape plan of resr_generator_forward. */
+int resr_canvas_pack(const int* hs, const int* ws, int count, int max_width, int* x0, int* y0, int* canvas_h, int* canvas_w);
+size_t resr_generator_forward_many_workspace_bytes(const resr_generator_t* g, const int* hs, const int* ws, int count);
+int resr_generator_forward_many(resr_generator_t* g, const float* const* xs, float* const* ys, const int* hs, const int* ws, int count,
+                                void* workspace, size_t workspace_bytes, void* stream);
+int resr_generator_forward_many_u8(resr_generator_t* g, const unsigned char* const* xs, unsigned char* const* ys, const int* hs,
+                                   const int* ws, int count, void* workspace, size_t workspace_bytes, void* stream);
+
 /* Number of kernels of this library that one resr_generator_forward launches (for bench accounting). */
 int resr_generator_launches_per_forward(void);
 /* Kernel policy of the 3x3 convolutions: 0 = single-CTA kernel only, 1 = CTA-pair kernel (tcgen05 cta_group::2) when

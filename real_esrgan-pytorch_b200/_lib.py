@@ -93,6 +93,11 @@ SIGNATURES = {
     "resr_generator_forward_host": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_size_t, c_void_p]),
     "resr_generator_forward_host_async": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_size_t, c_void_p]),
     "resr_generator_host_sync": (c_int, [c_void_p]),
+    "resr_canvas_pack": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "resr_generator_forward_many_workspace_bytes": (c_size_t, [c_void_p, c_void_p, c_void_p, c_int]),
+    "resr_generator_forward_many": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_size_t, c_void_p]),
+    "resr_generator_forward_many_u8": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_size_t,
+                                               c_void_p]),
     "resr_generator_launches_per_forward": (c_int, []),
     "resr_debug_wait_profile": (c_int, [c_void_p, c_int]),
     "resr_set_conv_pair_policy": (c_int, [c_int]),
@@ -180,6 +185,16 @@ def stream_ptr(device=None):
     """Current CUDA stream of `device` (default: the current device) as the `void* stream` of the C ABI."""
     import torch
     return c_void_p(torch.cuda.current_stream(device).cuda_stream)
+
+
+def canvas_pack(sizes, max_width=0):
+    """resr_canvas_pack: `sizes` is a sequence of (h, w) LR sizes. Returns ([(x0, y0)] in input order, (canvas_h, canvas_w))."""
+    n = len(sizes)
+    hs = (c_int * n)(*[int(h) for h, _ in sizes])
+    ws = (c_int * n)(*[int(w) for _, w in sizes])
+    x0, y0, ch, cw = (c_int * n)(), (c_int * n)(), c_int(), c_int()
+    check(lib().resr_canvas_pack(hs, ws, n, int(max_width), x0, y0, ctypes.byref(ch), ctypes.byref(cw)))
+    return list(zip(x0, y0)), (ch.value, cw.value)
 
 
 def ptr(t):

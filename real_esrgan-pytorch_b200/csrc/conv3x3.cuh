@@ -68,6 +68,12 @@ struct ConvArgs {
     float res2_scale;           // EP_ADD2
     float out16_scale;          // != 0: the 16-bit output stores out16_scale * v (the fp32 output keeps v): the next dense block's dY5
     float* out_nchw_raw;        // pre-clamp copy of the NCHW output (training: clamp backward needs it)
+    // ---- packed canvas of several images (N == 1; generator.cu resr_generator_forward_many): null = every pixel is valid
+    const uint32_t* vmask;      // bitmap of the valid LR pixels, row-major, vmask_words 32-bit words per LR row (non-null
+                                // selects the kernels' MASKED instantiation; the unmasked one is the code without canvas)
+    int vmask_words;
+    int vmask_shift;            // this layer's resolution: pixel (x, y) is valid iff LR bit (x >> shift, y >> shift) is set;
+                                // every output of an invalid pixel is written as 0, so a zero gutter between images stays zero
     int dbg_flags;            // experiments only: 1 = skip output stores, 2 = producer re-reads row 0, 4 = issue 1/4 of the MMAs
     unsigned long long* dbg;  // optional: CTA (0,0) writes phase timestamps (globaltimer ns) here, 16 slots
 };

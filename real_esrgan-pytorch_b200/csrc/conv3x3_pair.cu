@@ -228,7 +228,8 @@ __device__ __forceinline__ void tmem_init_bias(uint32_t taddr, const float* __re
 
 }  // namespace
 
-template <int NOUT>
+// MASKED: the packed-canvas variant (ConvArgs::vmask set); the other instantiation carries no mask code at all
+template <int NOUT, bool MASKED>
 __global__ void __launch_bounds__(512, 1)
 conv3x3_pair_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant__ CUtensorMap tmapO16,
                     const __grid_constant__ CUtensorMap tmapOF, const ConvArgs a) {
@@ -436,6 +437,11 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_cons
                 const uint32_t col2 = (S + slot) * NOUT;  // overflow twin (ring positions 0 and 1 only)
                 const bool dual = slot < 2;
                 const size_t pix = (static_cast<size_t>(valid ? n : 0) * a.H + y) * a.W + (valid ? x : 0);
+                bool inside = true;   // canvas pixel of an image (vmask), read before the accumulator wait like the residual
+                if (MASKED && emit) {
+                    const int lx = (valid ? x : 0) >> a.vmask_shift, ly = y >> a.vmask_shift;
+                    inside = (__ldg(a.vmask + static_cast<size_t>(ly) * a.vmask_words + (lx >> 5)) >> (lx & 31)) & 1u;
+                }
                 bool waited = false;
 #pragma unroll 1
                 for (int h = 0; h < NSUB; ++h) {
@@ -590,6 +596,10 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_cons
                             val[2 * i + 1] = fmaxf(val[2 * i + 1], t.y);
                         }
                     }
+                    if (MASKED && !inside) {   // gutter / canvas margin: 0 in every output, as the zero padding around an image
+#pragma unroll
+                        for (int i = 0; i < SUBW; ++i) val[i] = 0.f;
+                    }
                     if (a.out_nchw_raw && valid) {
                         const size_t plane = static_cast<size_t>(a.H) * a.W;
                         float* o = a.out_nchw_raw + static_cast<size_t>(n) * a.out_nchw_c * plane + static_cast<size_t>(y) * a.W + x;
@@ -730,11 +740,11 @@ bool conv3x3_pair_plan_smem(ConvArgs* a, int nout) {
     }
 }
 
-template <int NOUT>
+template <int NOUT, bool MASKED>
 static cudaError_t launch_pair_t(const ConvMaps& maps, const ConvArgs& args, dim3 grid, int threads, cudaStream_t stream) {
     static PerDevice<bool> attr;  // function attributes are per device
     if (!attr.cur()) {
-        cudaError_t e = cudaFuncSetAttribute(conv3x3_pair_kernel<NOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax);
+        cudaError_t e = cudaFuncSetAttribute(conv3x3_pair_kernel<NOUT, MASKED>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax);
         if (e != cudaSuccess) return e;
         attr.cur() = true;
     }
@@ -753,7 +763,7 @@ static cudaError_t launch_pair_t(const ConvMaps& maps, const ConvArgs& args, dim
     at[1].val.clusterDim.z = 1;
     cfg.attrs = at;
     cfg.numAttrs = 2;
-    return cudaLaunchKernelEx(&cfg, conv3x3_pair_kernel<NOUT>, maps.a, maps.o16, maps.of, args);
+    return cudaLaunchKernelEx(&cfg, conv3x3_pair_kernel<NOUT, MASKED>, maps.a, maps.o16, maps.of, args);
 }
 
 // `nout`: accumulator columns per output row and pair (64, 32, 16); `nslices` pair-slices cover Cout (blockIdx.y).
@@ -776,9 +786,15 @@ cudaError_t conv3x3_pair_launch(const ConvMaps& maps, const ConvArgs& args_in, i
     if (args.tail_ksteps != 1 && args.tail_ksteps != 2 && args.tail_ksteps != 4) args.tail_ksteps = 4;
     const dim3 grid(static_cast<unsigned>(2 * npairs), static_cast<unsigned>(nslices), 1);
     const int threads = 128 + 128 * args.nepi;
-    if (nout == 64) return launch_pair_t<64>(maps, args, grid, threads, stream);
-    if (nout == 32) return launch_pair_t<32>(maps, args, grid, threads, stream);
-    if (nout == 16) return launch_pair_t<16>(maps, args, grid, threads, stream);
+    if (args.vmask) {
+        if (nout == 64) return launch_pair_t<64, true>(maps, args, grid, threads, stream);
+        if (nout == 32) return launch_pair_t<32, true>(maps, args, grid, threads, stream);
+        if (nout == 16) return launch_pair_t<16, true>(maps, args, grid, threads, stream);
+        return cudaErrorInvalidValue;
+    }
+    if (nout == 64) return launch_pair_t<64, false>(maps, args, grid, threads, stream);
+    if (nout == 32) return launch_pair_t<32, false>(maps, args, grid, threads, stream);
+    if (nout == 16) return launch_pair_t<16, false>(maps, args, grid, threads, stream);
     return cudaErrorInvalidValue;
 }
 

@@ -241,7 +241,8 @@ __device__ __forceinline__ void mma_role(const ConvArgs& a, const RowRange rr, c
     }
 }
 
-template <int NOUT>
+// MASKED: the packed-canvas variant (ConvArgs::vmask set); the other instantiation carries no mask code at all
+template <int NOUT, bool MASKED>
 __global__ void __launch_bounds__(512, 1)
 conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant__ CUtensorMap tmapO16,
                   const __grid_constant__ CUtensorMap tmapOF,
@@ -416,6 +417,11 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_consta
                         for (int i = 0; i < NOUT / 4; ++i) resv[i] = rp[i];
                     }
                 }
+                bool inside = true;   // canvas pixel of an image (vmask), read before the accumulator wait like the residual
+                if (MASKED && emit) {
+                    const int lx = (valid ? x : 0) >> a.vmask_shift, ly = y >> a.vmask_shift;
+                    inside = (__ldg(a.vmask + static_cast<size_t>(ly) * a.vmask_words + (lx >> 5)) >> (lx & 31)) & 1u;
+                }
                 mbar_wait(acc_full + slot, static_cast<uint32_t>(v >> 4) & 1);
                 tc_fence_after();
                 float val[NOUT];
@@ -508,6 +514,10 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_consta
                         val[2 * i] = fmaxf(val[2 * i], t.x);
                         val[2 * i + 1] = fmaxf(val[2 * i + 1], t.y);
                     }
+                }
+                if (MASKED && !inside) {   // gutter / canvas margin: 0 in every output, as the zero padding around an image
+#pragma unroll
+                    for (int i = 0; i < NOUT; ++i) val[i] = 0.f;
                 }
                 if (a.out_nchw_raw && valid) {
                     const size_t plane = static_cast<size_t>(a.H) * a.W;
@@ -738,11 +748,11 @@ int conv3x3_make_tmap_f32(CUtensorMap* out, const void* base, int N, int H, int 
     return r == CUDA_SUCCESS ? 0 : static_cast<int>(r);
 }
 
-template <int NOUT>
+template <int NOUT, bool MASKED>
 static cudaError_t launch_t(const ConvMaps& maps, const ConvArgs& args, dim3 grid, int threads, cudaStream_t stream) {
     static PerDevice<bool> attr;  // function attributes are per device
     if (!attr.cur()) {
-        const cudaError_t e = cudaFuncSetAttribute(conv3x3_tc_kernel<NOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax);
+        const cudaError_t e = cudaFuncSetAttribute(conv3x3_tc_kernel<NOUT, MASKED>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax);
         if (e != cudaSuccess) return e;
         attr.cur() = true;
     }
@@ -757,7 +767,7 @@ static cudaError_t launch_t(const ConvMaps& maps, const ConvArgs& args, dim3 gri
     at[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = at;
     cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, conv3x3_tc_kernel<NOUT>, maps.a, maps.o16, maps.of, args);
+    return cudaLaunchKernelEx(&cfg, conv3x3_tc_kernel<NOUT, MASKED>, maps.a, maps.o16, maps.of, args);
 }
 
 cudaError_t conv3x3_launch(const ConvMaps& maps, const ConvArgs& args, int cout_slice, int nslices, int num_sms,
@@ -784,8 +794,13 @@ cudaError_t conv3x3_launch(const ConvMaps& maps, const ConvArgs& args, int cout_
         fixed.tail_ksteps = 4;
         return conv3x3_launch(maps, fixed, cout_slice, nslices, num_sms, stream);
     }
-    if (cout_slice == 32) return launch_t<32>(maps, args, grid, threads, stream);
-    if (cout_slice == 16) return launch_t<16>(maps, args, grid, threads, stream);
+    if (args.vmask) {
+        if (cout_slice == 32) return launch_t<32, true>(maps, args, grid, threads, stream);
+        if (cout_slice == 16) return launch_t<16, true>(maps, args, grid, threads, stream);
+        return cudaErrorInvalidValue;
+    }
+    if (cout_slice == 32) return launch_t<32, false>(maps, args, grid, threads, stream);
+    if (cout_slice == 16) return launch_t<16, false>(maps, args, grid, threads, stream);
     return cudaErrorInvalidValue;
 }
 

@@ -3,6 +3,8 @@
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
+#include <algorithm>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -210,6 +212,153 @@ __global__ void tensor_to_image_kernel(const float* __restrict__ x, unsigned cha
     }
 }
 
+// ------------------------------------------------------------------------------------------- packed canvas
+// resr_generator_forward_many runs a list of differently sized images as ONE N = 1 forward over a canvas that holds
+// them side by side with at least one zero LR pixel between neighbours (DESIGN.md §3.2). Every convolution writes 0 at
+// each canvas pixel outside an image (ConvArgs::vmask), so the gutters act as each image's own zero padding.
+
+// One image of a canvas call (device table in the workspace, sorted by (y0, x0): shelf by shelf, left to right).
+struct CanvasImage {
+    const void* src;   // fp32 NCHW [3, h, w] or u8 NHWC [h, w, 3]
+    void* dst;         // fp32 NCHW [3, 4h, 4w] or u8 NHWC [4h, 4w, 3]
+    int x0, y0, h, w;  // LR rectangle on the canvas
+};
+
+// Index of the image covering LR canvas pixel (x, y), or -1. Relies on the shelf layout of canvas_pack: the images of a
+// shelf share y0 and every later shelf starts below the bottom of every earlier image.
+__device__ __forceinline__ int canvas_owner(const CanvasImage* __restrict__ im, int count, int x, int y) {
+    int lo = 0, hi = count;   // first image with y0 > y
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (im[mid].y0 <= y) lo = mid + 1; else hi = mid;
+    }
+    if (lo == 0) return -1;
+    const int sy = im[lo - 1].y0;   // the shelf that may hold row y
+    int a = 0, b = lo;              // first image after (sy, x) in (y0, x0) order
+    while (a < b) {
+        const int mid = (a + b) >> 1;
+        if (im[mid].y0 < sy || (im[mid].y0 == sy && im[mid].x0 <= x)) a = mid + 1; else b = mid;
+    }
+    const int i = a - 1;
+    if (i < 0) return -1;
+    const CanvasImage& c = im[i];
+    return (x >= c.x0 && x < c.x0 + c.w && y >= c.y0 && y < c.y0 + c.h) ? i : -1;
+}
+
+__device__ __forceinline__ uint32_t pack2_16(float a, float b, int fmt) {
+    if (fmt == 1) {
+        __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
+        return *reinterpret_cast<uint32_t*>(&h);
+    }
+    __half2 h = __floats2half2_rn(a, b);
+    return *reinterpret_cast<uint32_t*>(&h);
+}
+
+// Canvas input: every LR canvas pixel gets its 64-channel 16-bit NHWC value -- the image's 3 channels converted as
+// nchw_to_nhwc16_kernel (fp32) / u8nhwc_to_nhwc16_kernel (u8: / 255 in fp32) do, zero in the gutters and margins -- and
+// the valid-pixel bitmap the convolution epilogues read. cw % 32 == 0 and the stride is a multiple of 32, so a warp
+// always covers 32 pixels of one row and its ballot is one bitmap word.
+__global__ void canvas_gather_kernel(const CanvasImage* __restrict__ im, int count, int cw, size_t npix, int u8, int fmt,
+                                     uint16_t* __restrict__ xin, uint32_t* __restrict__ vmask) {
+    for (size_t p = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; p < npix;
+         p += static_cast<size_t>(gridDim.x) * blockDim.x) {
+        const int y = static_cast<int>(p / cw), x = static_cast<int>(p % cw);
+        const int i = canvas_owner(im, count, x, y);
+        float v[3] = {0.f, 0.f, 0.f};
+        if (i >= 0) {
+            const CanvasImage c = im[i];
+            const size_t q = static_cast<size_t>(y - c.y0) * c.w + (x - c.x0);
+            if (u8) {
+                const unsigned char* s = static_cast<const unsigned char*>(c.src) + q * 3;
+#pragma unroll
+                for (int k = 0; k < 3; ++k) v[k] = __fdiv_rn(static_cast<float>(s[k]), 255.f);
+            } else {
+                const float* s = static_cast<const float*>(c.src) + q;
+                const size_t plane = static_cast<size_t>(c.h) * c.w;
+#pragma unroll
+                for (int k = 0; k < 3; ++k) v[k] = s[k * plane];
+            }
+        }
+        uint4* o = reinterpret_cast<uint4*>(xin + p * 64);
+        o[0] = make_uint4(pack2_16(v[0], v[1], fmt), pack2_16(v[2], 0.f, fmt), 0u, 0u);
+#pragma unroll
+        for (int k = 1; k < 8; ++k) o[k] = make_uint4(0u, 0u, 0u, 0u);
+        const unsigned word = __ballot_sync(0xffffffffu, i >= 0);
+        if ((threadIdx.x & 31) == 0) vmask[p >> 5] = word;
+    }
+}
+
+// Canvas output -> each image's own tensor: its 4h x 4w region of conv4's fp32 NCHW [1, 3, 4ch, 4cw] or u8 NHWC
+// [4ch, 4cw, 3] canvas. blockIdx.y = image.
+__global__ void canvas_scatter_kernel(const CanvasImage* __restrict__ im, const void* __restrict__ canvas, int ch, int cw, int u8) {
+    const CanvasImage c = im[blockIdx.y];
+    const int H4 = 4 * c.h, W4 = 4 * c.w;
+    const size_t W4c = static_cast<size_t>(4) * cw;
+    const size_t total = static_cast<size_t>(H4) * W4 * 3;
+    for (size_t e = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; e < total;
+         e += static_cast<size_t>(gridDim.x) * blockDim.x) {
+        if (u8) {
+            const size_t pix = e / 3;
+            const int k = static_cast<int>(e % 3);
+            const size_t yy = pix / W4, xx = pix % W4;
+            static_cast<unsigned char*>(c.dst)[e] =
+                static_cast<const unsigned char*>(canvas)[((4 * static_cast<size_t>(c.y0) + yy) * W4c + 4 * static_cast<size_t>(c.x0) + xx) * 3 + k];
+        } else {
+            const size_t xx = e % W4, t = e / W4;
+            const size_t yy = t % H4, k = t / H4;
+            static_cast<float*>(c.dst)[e] =
+                static_cast<const float*>(canvas)[(k * 4 * ch + 4 * static_cast<size_t>(c.y0) + yy) * W4c + 4 * static_cast<size_t>(c.x0) + xx];
+        }
+    }
+}
+
+// Shelf packer of resr_canvas_pack: images tallest first (ties: wider first, then input order), left to right on shelves
+// that are as tall as their first image. Neighbours keep one zero pixel between them, to the right and below; the canvas
+// edge needs none (the convolutions' tensor maps zero-fill outside the tensor). max_width <= 0 picks a near-square canvas.
+// The canvas size is rounded up to multiples of kCanvasRows x kCanvasCols, so varied lists share a few plans.
+static const int kCanvasRows = 16, kCanvasCols = 128, kCanvasMaxSide = 16384;
+static int canvas_pack(const int* hs, const int* ws, int count, int max_width, int* x0, int* y0, int* canvas_h, int* canvas_w) {
+    if (!hs || !ws || !x0 || !y0 || !canvas_h || !canvas_w || count <= 0) return set_error(RESR_E_INVALID, "canvas_pack: bad argument");
+    long long area = 0;
+    int wmax = 0;
+    for (int i = 0; i < count; ++i) {
+        if (hs[i] <= 0 || ws[i] <= 0 || hs[i] > kCanvasMaxSide || ws[i] > kCanvasMaxSide)
+            return set_error(RESR_E_INVALID, "canvas_pack: image %d has size %dx%d (1..%d per side)", i, hs[i], ws[i], kCanvasMaxSide);
+        area += static_cast<long long>(hs[i] + 1) * (ws[i] + 1);
+        wmax = std::max(wmax, ws[i]);
+    }
+    long long limit = max_width;
+    if (max_width <= 0) {
+        limit = std::max<long long>(static_cast<long long>(std::ceil(std::sqrt(static_cast<double>(area)))), wmax);
+        limit = (limit + kCanvasCols - 1) / kCanvasCols * kCanvasCols;   // the whole bucket is computed anyway
+    } else if (wmax > max_width) {
+        return set_error(RESR_E_INVALID, "canvas_pack: an image is %d wide, the width limit is %d", wmax, max_width);
+    }
+    std::vector<int> order(count);
+    for (int i = 0; i < count; ++i) order[i] = i;
+    std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return hs[a] != hs[b] ? hs[a] > hs[b] : ws[a] > ws[b]; });
+    long long x = 0, y = 0, shelf_h = 0, used_w = 0;
+    for (int i : order) {
+        if (x > 0 && x + ws[i] > limit) {   // next shelf, one gutter row below the tallest image of this one
+            y += shelf_h + 1;
+            x = 0;
+            shelf_h = 0;
+        }
+        x0[i] = static_cast<int>(x);
+        y0[i] = static_cast<int>(y);
+        shelf_h = std::max<long long>(shelf_h, hs[i]);
+        used_w = std::max(used_w, x + ws[i]);
+        x += ws[i] + 1;
+    }
+    const long long H = (y + shelf_h + kCanvasRows - 1) / kCanvasRows * kCanvasRows;
+    const long long W = (used_w + kCanvasCols - 1) / kCanvasCols * kCanvasCols;
+    if (H > kCanvasMaxSide || W > kCanvasMaxSide)
+        return set_error(RESR_E_INVALID, "canvas_pack: canvas %lldx%lld exceeds %d per side; split the list", H, W, kCanvasMaxSide);
+    *canvas_h = static_cast<int>(H);
+    *canvas_w = static_cast<int>(W);
+    return RESR_OK;
+}
+
 int grid_for(size_t total, int block) {
     size_t g = (total + block - 1) / block;
     if (g > 148 * 16) g = 148 * 16;
@@ -285,8 +434,8 @@ static WsLayout ws_layout(size_t N, size_t H, size_t W, int precision = 0) {
     return L;
 }
 
-static int build_plan(resr_generator* g, int N, int H, int W, void* ws, cudaStream_t s) {
-    Plan& p = g->plan;
+// vmask: valid-pixel bitmap of a packed canvas (N == 1, W % 32 == 0; W / 32 words per LR row), or null
+static int build_plan(resr_generator* g, Plan& p, int N, int H, int W, void* ws, const uint32_t* vmask, cudaStream_t s) {
     p.valid = false;
     p.steps.clear();
     p.N = N; p.H = H; p.W = W; p.ws = ws;
@@ -342,6 +491,7 @@ static int build_plan(resr_generator* g, int N, int H, int W, void* ws, cudaStre
         a.rows_total = static_cast<long long>(a.ncg) * q.H;
         a.wpack = g->wpack + cs.w_off;
         a.bias = g->bias + cs.b_off;
+        if (vmask) { a.vmask = vmask; a.vmask_words = W / 32; a.vmask_shift = s; }
         map_rc |= conv3x3_make_tmap_act(&st.maps.a, in16, N, q.H, q.W, cin_total, q.mode, q.BW, q.BN, cs.cin);
         return st;
     };
@@ -562,6 +712,7 @@ int resr_generator_set_precision(resr_generator_t* g, int precision) {
         g->precision = precision;
         g->loaded = false;        // the packed weights are in the old operand format: the caller reloads its parameters
         g->plan.valid = false;
+        g->canvas_plans.clear();
         cudaFree(g->pack_jobs);   // the batched pack table carries the operand format
         g->pack_jobs = nullptr;
         // the captured training step launches the old recipe's kernels: capture it again under the new one
@@ -577,6 +728,17 @@ int resr_generator_set_precision(resr_generator_t* g, int precision) {
 
 static int forward_any(resr_generator_t* g, const float* x, const unsigned char* x_u8, float* y, unsigned char* y_u8, int n, int h, int w,
                        void* workspace, size_t workspace_bytes, void* stream);
+
+// The 352 launches of a plan after its input layout kernel; conv4 writes y (fp32 NCHW) or y_u8 (u8 NHWC).
+static int run_plan(resr_generator_t* g, Plan& p, float* y, unsigned char* y_u8, cudaStream_t s) {
+    for (size_t i = 0; i < p.steps.size(); ++i) {
+        Step& st = p.steps[i];
+        if (i + 1 == p.steps.size()) { st.a.out_nchw = y; st.a.out_u8 = y_u8; }
+        const cudaError_t e = conv3x3_run(st.maps, st.a, st.cfg, g->num_sms, s);
+        if (e != cudaSuccess) return set_error(RESR_E_CUDA, "conv %d launch: %s", st.conv, cudaGetErrorString(e));
+    }
+    return RESR_OK;
+}
 
 int resr_generator_forward(resr_generator_t* g, const float* x, float* y, int n, int h, int w, void* workspace,
                            size_t workspace_bytes, void* stream) {
@@ -628,20 +790,114 @@ static int forward_any(resr_generator_t* g, const float* x, const unsigned char*
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     Plan& p = g->plan;
     if (!p.valid || p.N != n || p.H != h || p.W != w || p.ws != workspace || p.pair_policy != conv3x3_set_pair_policy(-1)) {
-        const int rc = build_plan(g, n, h, w, workspace, s);
+        const int rc = build_plan(g, p, n, h, w, workspace, nullptr, s);
         if (rc != RESR_OK) return rc;
     }
     const size_t total = static_cast<size_t>(n) * h * w * 8;
     if (x_u8) u8nhwc_to_nhwc16_kernel<<<grid_for(total, 256), 256, 0, s>>>(x_u8, p.xin, static_cast<size_t>(n) * h * w, 3, 64, g->precision == 1 ? 1 : 0);
     else nchw_to_nhwc16_kernel<<<grid_for(total, 256), 256, 0, s>>>(x, p.xin, n, 3, h, w, 64, g->precision == 1 ? 1 : 0);
-    const Table& T = table();
-    for (size_t i = 0; i < p.steps.size(); ++i) {
-        Step& st = p.steps[i];
-        if (i + 1 == p.steps.size()) { st.a.out_nchw = y; st.a.out_u8 = y_u8; }
-        const cudaError_t e = conv3x3_run(st.maps, st.a, st.cfg, g->num_sms, s);
-        if (e != cudaSuccess) return set_error(RESR_E_CUDA, "conv %d launch: %s", st.conv, cudaGetErrorString(e));
-    }
+    return run_plan(g, p, y, y_u8, s);
+}
+
+// Workspace of a canvas call: the N = 1 forward of the canvas, then conv4's canvas output (fp32 NCHW; the u8 output
+// takes a quarter of it), the valid-pixel bitmap and the per-image table.
+struct ManyLayout {
+    int ch, cw;
+    size_t out, vmask, table, total;
+};
+static int many_layout(const resr_generator_t* g, const int* hs, const int* ws, int count, int* x0, int* y0, ManyLayout* L) {
+    const int rc = canvas_pack(hs, ws, count, 0, x0, y0, &L->ch, &L->cw);
+    if (rc != RESR_OK) return rc;
+    const size_t P = static_cast<size_t>(L->ch) * L->cw;
+    size_t o = ws_layout(1, L->ch, L->cw, g->precision).total;
+    L->out = o;
+    o = align_up(o + P * 48 * 4, 1024);
+    L->vmask = o;
+    o = align_up(o + P / 8, 1024);
+    L->table = o;
+    L->total = align_up(o + static_cast<size_t>(count) * sizeof(CanvasImage), 1024);
     return RESR_OK;
+}
+
+static const int kCanvasPlans = 8;      // canvas plans a handle keeps (each ~0.4 MB of host memory)
+static const int kCanvasMaxImages = 65535;
+
+static int forward_many_any(resr_generator_t* g, const void* const* xs, void* const* ys, const int* hs, const int* ws, int count,
+                            int u8, void* workspace, size_t workspace_bytes, void* stream) {
+    if (!g || !workspace || !xs || !ys || !hs || !ws) return set_error(RESR_E_INVALID, "null argument");
+    if (count <= 0 || count > kCanvasMaxImages) return set_error(RESR_E_INVALID, "forward_many: count %d (1..%d)", count, kCanvasMaxImages);
+    for (int i = 0; i < count; ++i)
+        if (!xs[i] || !ys[i]) return set_error(RESR_E_INVALID, "forward_many: null image pointer %d", i);
+    if (!g->loaded) return set_error(RESR_E_INVALID, "resr_generator_load_params has not been called");
+    if ((reinterpret_cast<uintptr_t>(workspace) & 1023) != 0) return set_error(RESR_E_INVALID, "workspace must be 1024-byte aligned");
+    std::vector<int> x0(count), y0(count);
+    ManyLayout L;
+    const int rc = many_layout(g, hs, ws, count, x0.data(), y0.data(), &L);
+    if (rc != RESR_OK) return rc;
+    if (workspace_bytes < L.total) return set_error(RESR_E_NOMEM, "workspace too small (need %zu)", L.total);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    uint8_t* base = static_cast<uint8_t*>(workspace);
+    uint32_t* vmask = reinterpret_cast<uint32_t*>(base + L.vmask);
+    CanvasImage* table_d = reinterpret_cast<CanvasImage*>(base + L.table);
+
+    // plans are cached by canvas geometry next to the single-shape plan (g->plan)
+    const int policy = conv3x3_set_pair_policy(-1);
+    Plan* p = nullptr;
+    for (Plan& c : g->canvas_plans)
+        if (c.valid && c.H == L.ch && c.W == L.cw && c.ws == workspace && c.pair_policy == policy) p = &c;
+    if (!p) {
+        if (static_cast<int>(g->canvas_plans.size()) >= kCanvasPlans) g->canvas_plans.erase(g->canvas_plans.begin());
+        g->canvas_plans.emplace_back();
+        p = &g->canvas_plans.back();
+        const int brc = build_plan(g, *p, 1, L.ch, L.cw, workspace, vmask, s);
+        if (brc != RESR_OK) {
+            g->canvas_plans.pop_back();
+            return brc;
+        }
+    }
+
+    std::vector<CanvasImage> tab(count);
+    size_t most = 0;
+    for (int i = 0; i < count; ++i) {
+        tab[i] = CanvasImage{xs[i], ys[i], x0[i], y0[i], hs[i], ws[i]};
+        most = std::max(most, static_cast<size_t>(hs[i]) * ws[i] * 48);
+    }
+    std::sort(tab.begin(), tab.end(), [](const CanvasImage& a, const CanvasImage& b) { return a.y0 != b.y0 ? a.y0 < b.y0 : a.x0 < b.x0; });
+    // (pageable source: the copy is staged before the call returns, so `tab` may go out of scope)
+    if (cudaMemcpyAsync(table_d, tab.data(), tab.size() * sizeof(CanvasImage), cudaMemcpyHostToDevice, s) != cudaSuccess)
+        return set_error(RESR_E_CUDA, "forward_many: table copy failed");
+    const size_t npix = static_cast<size_t>(L.ch) * L.cw;
+    canvas_gather_kernel<<<grid_for(npix, 256), 256, 0, s>>>(table_d, count, L.cw, npix, u8, g->precision == 1 ? 1 : 0, p->xin, vmask);
+    const int rrc = run_plan(g, *p, u8 ? nullptr : reinterpret_cast<float*>(base + L.out), u8 ? base + L.out : nullptr, s);
+    if (rrc != RESR_OK) return rrc;
+    const int gx = static_cast<int>(std::min<size_t>(128, (most + 2047) / 2048));
+    canvas_scatter_kernel<<<dim3(gx, count), 256, 0, s>>>(table_d, base + L.out, L.ch, L.cw, u8);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return set_error(RESR_E_CUDA, "forward_many: %s", cudaGetErrorString(e));
+    return RESR_OK;
+}
+
+int resr_canvas_pack(const int* hs, const int* ws, int count, int max_width, int* x0, int* y0, int* canvas_h, int* canvas_w) {
+    return canvas_pack(hs, ws, count, max_width, x0, y0, canvas_h, canvas_w);
+}
+
+size_t resr_generator_forward_many_workspace_bytes(const resr_generator_t* g, const int* hs, const int* ws, int count) {
+    if (!g || !hs || !ws || count <= 0 || count > kCanvasMaxImages) return 0;
+    std::vector<int> x0(count), y0(count);
+    ManyLayout L;
+    return many_layout(g, hs, ws, count, x0.data(), y0.data(), &L) == RESR_OK ? L.total : 0;
+}
+
+int resr_generator_forward_many(resr_generator_t* g, const float* const* xs, float* const* ys, const int* hs, const int* ws, int count,
+                                void* workspace, size_t workspace_bytes, void* stream) {
+    return forward_many_any(g, reinterpret_cast<const void* const*>(xs), reinterpret_cast<void* const*>(ys), hs, ws, count, 0, workspace,
+                            workspace_bytes, stream);
+}
+
+int resr_generator_forward_many_u8(resr_generator_t* g, const unsigned char* const* xs, unsigned char* const* ys, const int* hs,
+                                   const int* ws, int count, void* workspace, size_t workspace_bytes, void* stream) {
+    return forward_many_any(g, reinterpret_cast<const void* const*>(xs), reinterpret_cast<void* const*>(ys), hs, ws, count, 1, workspace,
+                            workspace_bytes, stream);
 }
 
 int resr_generator_forward_host(resr_generator_t* g, const float* x_host, float* y_host, int n, int h, int w,

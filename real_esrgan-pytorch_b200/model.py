@@ -18,6 +18,8 @@ __all__ = ["ResidualDenseBlock", "ResidualResidualDenseBlock", "Generator", "pla
 
 
 _PRECISIONS = {"fp16": 0, "bf16": 1}
+# LR pixels per packed canvas of infer_many: cfg3's 64 x 128 x 128 batch, about 8 GB of workspace in the fp16 recipe
+CANVAS_MAX_PIXELS = 1 << 20
 
 
 def _conv(cin: int, cout: int) -> nn.Conv2d:
@@ -242,6 +244,9 @@ class Generator(nn.Module):
 
     def _get_workspace(self, n: int, h: int, w: int, device, extra: int = 0) -> torch.Tensor:
         need = _lib.lib().resr_generator_workspace_bytes_for(self._native(), n, h, w) + extra
+        return self._workspace_of(need, device)
+
+    def _workspace_of(self, need: int, device) -> torch.Tensor:
         ws = self._workspace
         if ws is None or ws.numel() < need + 1024 or ws.device != device:
             ws = torch.empty(need + 1024, dtype=torch.uint8, device=device)
@@ -371,6 +376,72 @@ class Generator(nn.Module):
 
     def host_sync(self):
         _lib.check(_lib.lib().resr_generator_host_sync(self._native()))
+
+    # ------------------------------------------------------------------ lists of differently sized images
+    @torch.no_grad()
+    def infer_many(self, images, max_pixels: int = CANVAS_MAX_PIXELS):
+        """SR of a list of differently sized images ([1, 3, h, w] or [3, h, w] fp32 CUDA tensors), returned in input order
+        with infer()'s shape per image ([1, 3, 4h, 4w] or [3, 4h, 4w]). The loops of the reference's test.py, validate()
+        and inference.py over a folder run one image per forward; here consecutive images are packed into canvases of at
+        most `max_pixels` LR pixels (an image larger than that runs alone) and each canvas is one forward
+        (resr_generator_forward_many). Every result is its image's own forward, up to fp32 summation order."""
+        xs = []
+        for x in images:
+            if x.dim() not in (3, 4) or x.size(-3) != 3 or (x.dim() == 4 and x.size(0) != 1):
+                raise ValueError(f"expected a [1, 3, H, W] or [3, H, W] image, got {tuple(x.shape)}")
+            self._check_device(x)
+            xs.append(x.detach().float().contiguous())
+        ys = [torch.empty(x.shape[:-2] + (4 * x.size(-2), 4 * x.size(-1)), dtype=torch.float32, device=x.device) for x in xs]
+        self._run_many(xs, ys, [tuple(x.shape[-2:]) for x in xs], max_pixels, "resr_generator_forward_many")
+        return ys
+
+    @torch.no_grad()
+    def infer_u8_many(self, images_u8, max_pixels: int = CANVAS_MAX_PIXELS):
+        """infer_u8 for a list of differently sized uint8 [h, w, 3] CUDA images: a list of [4h, 4w, 3] uint8 results in
+        input order, each equal to infer_u8 of its image up to fp32 summation order (packing as in infer_many)."""
+        xs = []
+        for x in images_u8:
+            if x.dim() != 3 or x.size(2) != 3 or x.dtype != torch.uint8:
+                raise ValueError(f"expected a uint8 [H, W, 3] image, got {tuple(x.shape)} {x.dtype}")
+            self._check_device(x)
+            xs.append(x.contiguous())
+        ys = [torch.empty((4 * x.size(0), 4 * x.size(1), 3), dtype=torch.uint8, device=x.device) for x in xs]
+        self._run_many(xs, ys, [tuple(x.shape[:2]) for x in xs], max_pixels, "resr_generator_forward_many_u8")
+        return ys
+
+    def _check_device(self, x):
+        if not x.is_cuda:
+            raise _lib.ResrError("resr_b200.Generator runs on a CUDA (sm_100a) device only; there is no CPU path")
+        if x.device != self._device():
+            raise _lib.ResrError(f"input on {x.device} but the generator lives on {self._device()}")
+
+    def _run_many(self, xs, ys, sizes, max_pixels, fn):
+        if not xs:
+            return
+        self._ensure_packed()
+        h = self._native()
+        dev = xs[0].device
+        groups, cur, px = [], [], 0
+        for i, (hh, ww) in enumerate(sizes):   # consecutive images, up to max_pixels LR pixels per canvas
+            if cur and px + hh * ww > max_pixels:
+                groups.append(cur)
+                cur, px = [], 0
+            cur.append(i)
+            px += hh * ww
+        groups.append(cur)
+        call = getattr(_lib.lib(), fn)
+        with torch.cuda.device(dev):
+            for idx in groups:
+                n = len(idx)
+                hs = (ctypes.c_int * n)(*[sizes[i][0] for i in idx])
+                ws_ = (ctypes.c_int * n)(*[sizes[i][1] for i in idx])
+                need = _lib.lib().resr_generator_forward_many_workspace_bytes(h, hs, ws_, n)
+                if need == 0:
+                    raise _lib.ResrError(f"no canvas for these {n} images: {_lib.lib().resr_last_error().decode()}")
+                wp, wbytes = self._aligned(self._workspace_of(need, dev))
+                xp = (ctypes.c_void_p * n)(*[xs[i].data_ptr() for i in idx])
+                yp = (ctypes.c_void_p * n)(*[ys[i].data_ptr() for i in idx])
+                _lib.check(call(h, xp, yp, hs, ws_, n, wp, wbytes, _lib.stream_ptr(dev)))
 
 
 # ----------------------------------------------------------------------------------------------------------------------
