@@ -161,6 +161,8 @@ int resr_nchw_to_nhwc16(const float* x, void* out16, int n, int c, int h, int w,
  * Hot path 2 — second-order degradation synthesis (train_realesrnet.py:267-377 and the imgproc.py ops it calls).
  * Images: fp32 NCHW contiguous, device memory. Random decisions and random tensors are INPUTS (drawn by the
  * caller: torch RNG on the host side, or recorded from the reference for parity).
+ * filter2d, USM, resize, JPEG and crop return RESR_E_INVALID for an empty or negative size (batch, channels, planes,
+ * input or output height / width) before they touch the device.
  * ---------------------------------------------------------------------------------------------------------- */
 
 /* imgproc.filter2d_torch (imgproc.py:1089-1121): reflect-pad k/2, cross-correlation; kernel [kernel_batch,k,k] with

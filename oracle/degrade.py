@@ -212,7 +212,19 @@ def rgb_to_gray(img):
     return ((f32(0.2989) * r + f32(0.587) * g).astype(f32) + f32(0.114) * bl).astype(f32)
 
 
-def gaussian_noise_apply(img, sigma, gray, noise_color, noise_gray):
+def noise_post(out, clip=True, rounds=False):
+    """The clip / rounds tail of both noise ops; imgproc.py:1048-1055, 1080-1085."""
+    out = out.astype(f32)
+    if clip and rounds:
+        return (np.clip(np.rint(out * f32(255)), 0, 255) / f32(255)).astype(f32)
+    if clip:
+        return np.clip(out, 0, 1).astype(f32)
+    if rounds:
+        return (np.rint(out * f32(255)) / f32(255)).astype(f32)
+    return out
+
+
+def gaussian_noise_apply(img, sigma, gray, noise_color, noise_gray, clip=True, rounds=False):
     """imgproc.py:829-863 + 1029-1057 with the random tensors fed in:
     sigma[B], gray[B] (0/1), noise_color = randn(B,3,H,W), noise_gray = randn(H,W) (or None when sum(gray) == 0)."""
     b = img.shape[0]
@@ -222,7 +234,7 @@ def gaussian_noise_apply(img, sigma, gray, noise_color, noise_gray):
         g = gray.astype(f32).reshape(b, 1, 1, 1)
         ng = (noise_gray.astype(f32)[None, None] * s / f32(255)).astype(f32)  # ONE field shared by the batch
         noise = (noise * (f32(1) - g) + ng * g).astype(f32)
-    return np.clip(img + noise, 0, 1).astype(f32)
+    return noise_post(img + noise, clip, rounds)
 
 
 def unique_count_u8(q):
@@ -248,7 +260,7 @@ def poisson_rates(img, gray_any):
     return out
 
 
-def poisson_noise_apply(img, scale, gray, samples_color, samples_gray):
+def poisson_noise_apply(img, scale, gray, samples_color, samples_gray, clip=True, rounds=False):
     """imgproc.py:866-916 + 1060-1086 with the Poisson draws fed in: samples_color = poisson(q * vals) [B,3,H,W],
     samples_gray = poisson(q_gray * vals_gray) [B,1,H,W] or None."""
     b = img.shape[0]
@@ -259,7 +271,7 @@ def poisson_noise_apply(img, scale, gray, samples_color, samples_gray):
         ng = (samples_gray.astype(f32) / r["vals_g"] - r["qg"]).astype(f32)
         noise = (noise * (f32(1) - g) + ng * g).astype(f32)
     noise = (noise * scale.astype(f32).reshape(b, 1, 1, 1)).astype(f32)
-    return np.clip(img + noise, 0, 1).astype(f32)
+    return noise_post(img + noise, clip, rounds)
 
 
 # --------------------------------------------------------------------------------------------- JPEG (a12)

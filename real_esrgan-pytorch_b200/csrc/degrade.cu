@@ -582,9 +582,19 @@ __global__ void __launch_bounds__(128) usm_fused51_kernel(const float* __restric
     }
 }
 
+static int usm_taps_count(int radius) { return radius % 2 == 0 ? radius + 1 : radius; }  // imgproc.py:1518-1519
+
+// Argument checks of the USM entry points, made before anything touches the device
+static int usm_check_args(int B, int C, int H, int W, int radius) {
+    const int k = usm_taps_count(radius);
+    if (B <= 0 || C <= 0) return set_error(RESR_E_INVALID, "USM batch %d / channels %d must be positive", B, C);
+    if (k < 1 || k > kUsmMaxTaps) return set_error(RESR_E_INVALID, "USM radius %d out of range", radius);
+    if (k / 2 >= H || k / 2 >= W) return set_error(RESR_E_INVALID, "USM reflect padding %d needs a larger image (%dx%d)", k / 2, H, W);
+    return RESR_OK;
+}
+
 static int usm_set_taps(int radius, int sigma, int* k_out) {
-    if (radius % 2 == 0) radius += 1;  // imgproc.py:1518-1519
-    if (radius > kUsmMaxTaps) return set_error(RESR_E_INVALID, "USM radius %d too large", radius);
+    radius = usm_taps_count(radius);
     double sg = sigma;
     if (sg <= 0) sg = 0.3 * ((radius - 1) * 0.5 - 1) + 0.8;  // cv2.getGaussianKernel
     double taps[kUsmMaxTaps], sum = 0;
@@ -610,9 +620,9 @@ static int usm_set_taps(int radius, int sigma, int* k_out) {
 static int usm_impl(const float* x, float* out, float* ws, int B, int C, int H, int W, int radius, int sigma, float weight,
                     float threshold, cudaStream_t s, float* soft_out = nullptr) {
     int k = 0;
-    const int rc = usm_set_taps(radius, sigma, &k);
+    int rc = usm_check_args(B, C, H, W, radius);
+    if (rc == RESR_OK) rc = usm_set_taps(radius, sigma, &k);
     if (rc != RESR_OK) return rc;
-    if (k / 2 >= H || k / 2 >= W) return set_error(RESR_E_INVALID, "USM reflect padding %d needs a larger image (%dx%d)", k / 2, H, W);
     const size_t E = static_cast<size_t>(B) * C * H * W;
     float* tmp = ws;
     float* res = ws + E;
@@ -1049,8 +1059,9 @@ static constexpr int kJpegWarps = 8;
 
 __global__ void __launch_bounds__(32 * kJpegWarps) jpeg_kernel(const float* __restrict__ x, float* __restrict__ out,
                                                                const float* __restrict__ quality, float* __restrict__ factor_out,
-                                                               int B, int H, int W, int clamp_in, float* __restrict__ qy,
-                                                               float* __restrict__ qcb, float* __restrict__ qcr) {
+                                                               int B, int H, int W, int clamp_in, int vec_ok,
+                                                               float* __restrict__ qy, float* __restrict__ qcb,
+                                                               float* __restrict__ qcr) {
     grid_dep_wait();      // programmatic dependent launch: everything the previous kernel wrote is visible from here on
     grid_dep_launch();    // the next kernel of the chain may be scheduled behind this one
     __shared__ __align__(16) float s_pix[kJpegWarps][6][64];   // samples -> dequantised coefficients -> reconstruction
@@ -1090,7 +1101,6 @@ __global__ void __launch_bounds__(32 * kJpegWarps) jpeg_kernel(const float* __re
     const int nmcu = B * mh * mw;
     const size_t HW = static_cast<size_t>(H) * W;
     const int py = lane >> 1, px0 = (lane & 1) * 8;   // this lane's 8 consecutive pixels of the MCU
-    const bool vec_ok = (W & 3) == 0;
     for (int m = blockIdx.x * kJpegWarps + warp; m < nmcu; m += gridDim.x * kJpegWarps) {
         const int b = m / (mh * mw);
         const int my = (m / mw) % mh, mx = m % mw;
@@ -1282,7 +1292,9 @@ static int jpeg_impl(const float* x, float* out, const float* quality, float* fa
     const int nmcu = B * ((H + 15) / 16) * ((W + 15) / 16);
     int grid = (nmcu + kJpegWarps - 1) / kJpegWarps;
     if (grid > 148 * 8) grid = 148 * 8;   // beyond that, warps loop over MCUs
-    launch_pdl(jpeg_kernel, grid, 32 * kJpegWarps, 0, s, x, out, quality, factor_out, B, H, W, clamp_in, qy, qcb, qcr);
+    // float4 rows need W % 4 == 0 AND 16-byte aligned bases: a contiguous view with a storage offset reaches here as is
+    const int vec_ok = (W & 3) == 0 && ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(out)) & 15) == 0;
+    launch_pdl(jpeg_kernel, grid, 32 * kJpegWarps, 0, s, x, out, quality, factor_out, B, H, W, clamp_in, vec_ok, qy, qcb, qcr);
     RESR_LAUNCH_CHECK("jpeg");
     return RESR_OK;
 }
@@ -1314,6 +1326,7 @@ extern "C" {
 int resr_filter2d(const float* image, const float* kernel, float* out, int b, int c, int h, int w, int k, int kernel_batch,
                   void* stream) {
     if (!image || !kernel || !out) return set_error(RESR_E_INVALID, "null argument");
+    if (b <= 0 || c <= 0) return set_error(RESR_E_INVALID, "filter2d batch %d / channels %d must be positive", b, c);
     if (kernel_batch != 1 && kernel_batch != b) return set_error(RESR_E_INVALID, "kernel batch %d must be 1 or %d", kernel_batch, b);
     return filter2d_impl(image, kernel, out, b, c, h, w, k, kernel_batch != 1, static_cast<cudaStream_t>(stream));
 }
@@ -1341,7 +1354,7 @@ int resr_usm_sharp_backward(const float* image, const float* grad_out, float* gr
     // recompute the forward quantities the gradient needs (residual, soft mask); the sharpened image itself lands in `t`
     const int rc = usm_impl(image, t, ws, b, c, h, w, radius, sigma, weight, threshold, s, soft);
     if (rc != RESR_OK) return rc;
-    int k = radius % 2 == 0 ? radius + 1 : radius;
+    const int k = usm_taps_count(radius);
     launch_pdl(usm_gsh_kernel, grid1d(E), 256, 0, s, grad_out, image, ws + E, soft, gsh, E, weight);
     launch_pdl(usm_adjoint_kernel, grid1d(E), 256, 0, s, gsh, t, b * c, h, w, k, 0, nullptr, nullptr, nullptr, weight);
     launch_pdl(usm_adjoint_kernel, grid1d(E), 256, 0, s, t, grad_in, b * c, h, w, k, 1, grad_out, soft, gsh, weight);
@@ -1352,6 +1365,7 @@ int resr_usm_sharp_backward(const float* image, const float* grad_out, float* gr
 int resr_resize(const float* image, float* out, int planes, int h_in, int w_in, int h_out, int w_out, int mode,
                 double scale_h, double scale_w, void* stream) {
     if (!image || !out) return set_error(RESR_E_INVALID, "null argument");
+    if (planes <= 0 || h_in <= 0 || w_in <= 0) return set_error(RESR_E_INVALID, "bad resize input %d x %d x %d", planes, h_in, w_in);
     return resize_impl(image, out, planes, h_in, w_in, h_out, w_out, mode, scale_h, scale_w, static_cast<cudaStream_t>(stream));
 }
 
@@ -1463,12 +1477,14 @@ int resr_jpeg(const float* image, float* out, const float* quality, float* facto
     if (!image || !out || !quality) return set_error(RESR_E_INVALID, "null argument");
     if ((q_y != nullptr) != (q_cb != nullptr) || (q_y != nullptr) != (q_cr != nullptr))
         return set_error(RESR_E_INVALID, "pass all three coefficient dumps or none");
+    if (b <= 0 || h <= 0 || w <= 0) return set_error(RESR_E_INVALID, "bad JPEG image %d x 3 x %d x %d", b, h, w);
     return jpeg_impl(image, out, quality, factor_out, b, h, w, clamp_input, q_y, q_cb, q_cr, static_cast<cudaStream_t>(stream));
 }
 
 int resr_crop(const float* image, float* out, int planes, int h_in, int w_in, int top, int left, int h_out, int w_out,
               int round_to_u8, void* stream) {
     if (!image || !out) return set_error(RESR_E_INVALID, "null argument");
+    if (planes <= 0 || h_out <= 0 || w_out <= 0) return set_error(RESR_E_INVALID, "bad crop size %d x %d x %d", planes, h_out, w_out);
     if (top < 0 || left < 0 || top + h_out > h_in || left + w_out > w_in) return set_error(RESR_E_INVALID, "crop window out of range");
     const size_t total = static_cast<size_t>(planes) * h_out * w_out;
     if (!round_to_u8 && h_out == h_in && w_out == w_in) {  // the window is the whole image (cfg2: HR is already 256^2)
