@@ -18,7 +18,7 @@ $(LIB): $(OBJS)
 	@mkdir -p $(PKG)/lib
 	$(NVCC) -shared -o $@ $(OBJS) -cudart static
 
-# development variants (A/B runs on one box through RESR_LIB_PATH): make variant NAME=prof DEFS=-DRESR_PROFILE_WAITS
+# development variants (same-box A/B through RESR_LIB_PATH, tools/ab.sh): make variant NAME=v1 [DEFS=-D...]
 variant:
 	@mkdir -p build/variants/$(NAME)
 	for f in $(SRCS); do $(NVCC) $(NVFLAGS) $(DEFS) -c $$f -o build/variants/$(NAME)/$$(basename $$f .cu).o || exit 1; done

@@ -123,9 +123,6 @@ int resr_generator_launches_per_forward(void);
  * column groups exist (tests use it to push small / awkward shapes through the pair kernel). Returns the previous policy;
  * a value outside 0..2 only queries. Takes effect for plans built afterwards (new shapes / workspaces). */
 int resr_set_conv_pair_policy(int policy);
-/* Development aid: wait-time counters of the CTA-pair convolution kernel (16 x u64 clock cycles summed over CTAs; all
- * zero unless the library was built with -DRESR_PROFILE_WAITS). out16_host may be NULL; reset != 0 clears them. */
-int resr_debug_wait_profile(unsigned long long* out16_host, int reset);
 
 /* One 3x3 convolution through the same tensor-core kernel (test / building block).
  * in16: NHWC 16-bit activations [n,h,w,c_total]; the first `cin` channels are convolved.
@@ -149,8 +146,6 @@ typedef struct resr_conv_desc {
     int res16, res16_fmt;    /* res16 = 1: res1 / res2 are 16-bit tensors of format res16_fmt (0 fp16, 1 bf16) */
     float* out_nchw;
     int out_nchw_c;
-    int dbg_flags;           /* experiments only (0 in production) */
-    unsigned long long* dbg; /* optional device buffer of 16 u64: phase timestamps of CTA (0,0), or NULL */
 } resr_conv_desc;
 int resr_conv3x3(const resr_conv_desc* d, void* stream);
 

@@ -28,8 +28,6 @@ class ConvDesc(Structure):
         ("res16", c_int), ("res16_fmt", c_int),
         ("out_nchw", c_void_p),
         ("out_nchw_c", c_int),
-        ("dbg_flags", c_int),
-        ("dbg", c_void_p),
     ]
 
 
@@ -99,7 +97,6 @@ SIGNATURES = {
     "resr_generator_forward_many_u8": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_size_t,
                                                c_void_p]),
     "resr_generator_launches_per_forward": (c_int, []),
-    "resr_debug_wait_profile": (c_int, [c_void_p, c_int]),
     "resr_set_conv_pair_policy": (c_int, [c_int]),
     "resr_conv3x3": (c_int, [POINTER(ConvDesc), c_void_p]),
     "resr_nchw_to_nhwc16": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),

@@ -30,7 +30,8 @@ struct ConvArgs {
     int reverse;    // pair kernel: traverse the work back to front (rows bottom-up, column groups last to first, dy taps
                     // flipped when the weights are gathered). Consecutive layers alternate direction, so a launch starts
                     // on the data its predecessor touched last -- what is still in the 126 MB L2.
-    int epi_bufs;   // pair kernel: staging tiles per epilogue group (2 = a pass never waits for the previous pass's TMA store)
+    int epi_bufs;   // staging tiles per epilogue group (2 = a pass never waits for the previous pass's TMA store; the
+                    // single-CTA kernel uses 1)
     int fmt_in;     // MMA operand format: 0 fp16, 1 bf16
     long long rows_total;  // ncg * H
     long long rows_total_pair;  // ceil(ncg / 2) * H: work units of the CTA-pair kernel (filled by its launcher)
@@ -74,20 +75,12 @@ struct ConvArgs {
     int vmask_words;
     int vmask_shift;            // this layer's resolution: pixel (x, y) is valid iff LR bit (x >> shift, y >> shift) is set;
                                 // every output of an invalid pixel is written as 0, so a zero gutter between images stays zero
-    int dbg_flags;            // experiments only: 1 = skip output stores, 2 = producer re-reads row 0, 4 = issue 1/4 of the MMAs
-    unsigned long long* dbg;  // optional: CTA (0,0) writes phase timestamps (globaltimer ns) here, 16 slots
 };
 
-// K16 steps of the last 64-channel chunk that hold real input channels.
-inline int conv3x3_tail_ksteps(int cin) {
-#ifdef RESR_NO_TAILSKIP
-    (void)cin;
-    return 4;
-#else
-    const int r = cin % 64;
-    return r == 0 || r > 32 ? 4 : (r > 16 ? 2 : 1);
-#endif
-}
+// Fills the launch geometry of an N x H x W convolution: N / H / W, the lane split BW x BN, mode (-1: automatic, i.e. 0
+// when a tile is one image row; lanes that span images always take mode 1), nxs, ncg, rows_total, and tail_ksteps from
+// the real input channels `cin` (0: every 64-channel chunk is full).
+void conv3x3_init_geometry(ConvArgs* args, int N, int H, int W, int cin, int mode);
 
 struct ConvMaps {
     CUtensorMap a;    // activations (load)
@@ -95,30 +88,16 @@ struct ConvMaps {
     CUtensorMap of;   // fp32 output (store)
 };
 
-// Launch one convolution. `cout_slice` is 32 or 16 (channels per CTA slice), `nslices` slices cover Cout.
-cudaError_t conv3x3_launch(const ConvMaps& maps, const ConvArgs& args, int cout_slice, int nslices, int num_sms,
-                           cudaStream_t stream);
-
-// Fills nstages / nepi from the shared-memory budget. Returns false if the configuration does not fit.
-bool conv3x3_plan_smem(ConvArgs* args, int cout_slice);
-
-// ---- CTA-pair kernel (conv3x3_pair.cu): tcgen05 cta_group::2, M = 256; reads the same weight packs.
-// nout: accumulator columns per output row of a pair (64 = two 32-channel pack slices per pair, 32, or 16).
-bool conv3x3_pair_plan_smem(ConvArgs* args, int nout);
-cudaError_t conv3x3_pair_launch(const ConvMaps& maps, const ConvArgs& args, int nout, int nslices, int num_sms,
-                                cudaStream_t stream);
-
-// Development builds (-DRESR_PROFILE_WAITS): copies / resets the pair kernel's wait-time counters (16 x u64 cycles).
-int conv3x3_wait_profile(unsigned long long* out16, int reset);
-
 // Kernel choice for one convolution whose weights are packed in `pack_nout`-channel slices (`pack_nslices` of them).
 struct ConvLaunchCfg {
     int pair;     // 1: CTA-pair kernel, 0: single-CTA kernel
     int nout;     // channels per launch slice
     int nslices;  // blockIdx.y extent
 };
-// Picks the kernel (pairs whenever there are at least two column groups to pair up; RESR_CONV_PAIR=0 forces the
-// single-CTA kernel), fills args->nstages / nepi. Returns false if the configuration does not fit in shared memory.
+// Picks the kernel: the CTA-pair kernel (conv3x3_pair.cu: tcgen05 cta_group::2, M = 256, same weight packs) whenever
+// there are at least two column groups to pair up and enough rows, the single-CTA kernel (conv3x3_tc.cu) otherwise;
+// RESR_CONV_PAIR=0 forces the single-CTA kernel. Fills args->nstages / nepi / epi_bufs. Returns false if the
+// configuration does not fit in shared memory.
 int conv3x3_set_pair_policy(int policy);  // returns the previous policy; -1 only queries
 bool conv3x3_choose(ConvArgs* args, int pack_nout, int pack_nslices, ConvLaunchCfg* cfg);
 cudaError_t conv3x3_run(const ConvMaps& maps, const ConvArgs& args, const ConvLaunchCfg& cfg, int num_sms, cudaStream_t stream);
@@ -129,8 +108,5 @@ int conv3x3_make_tmap_act(CUtensorMap* out, const void* base, int N, int H, int 
 int conv3x3_make_tmap_out16(CUtensorMap* out, const void* base, int N, int H, int W, int C, int nout, int BW, int BN,
                             int up2);  // N,H,W = geometry of the CONVOLUTION (destination is 2H x 2W when up2)
 int conv3x3_make_tmap_f32(CUtensorMap* out, const void* base, int N, int H, int W, int C, int BW, int BN);
-
-// Chooses the lane split for an image width.
-void conv3x3_pick_tile(int W, int* BW, int* BN);
 
 }  // namespace resr

@@ -20,80 +20,18 @@
 //     position is 0 or 1 therefore have their sum in two slots; the epilogue adds them.
 //   * The weight packs are the ones conv3x3_tc.cu uses ([slice32][chunk][dx][(dy, co) x 64 ch], 128B-swizzled): each
 //     CTA bulk-copies the row blocks that make up its half.
-#include <cuda_bf16.h>
-#include <cuda_fp16.h>
-
 #include <cstdlib>
-#include <cstring>
 
-#include "conv3x3.cuh"
-#include "device_state.h"
-#include "ptx.cuh"
+#include "conv3x3_common.cuh"
 
 namespace resr {
 
-// Wait-time profile (development builds with -DRESR_PROFILE_WAITS): cycles each role spends blocked, summed over CTAs.
-//   [0] MMA warp total  [1] .. waiting for activation stages  [2] .. waiting for free accumulator slots  [3] steps
-//   [4] producer total  [5] .. waiting for empty stages
-//   [6] epilogue (group 0, warp 0) total  [7] .. waiting for accumulators  [8] .. waiting for its staging tile
-__device__ unsigned long long g_wait_prof[16];
-#ifdef RESR_PROFILE_WAITS
-#define PROF_DECL(name) long long name = 0
-#define PROF_T0(t) const long long t = clock64()
-#define PROF_ADD(acc, t) acc += clock64() - t
-#define PROF_FLUSH(idx, v) do { if ((threadIdx.x & 31) == 0) atomicAdd(&g_wait_prof[idx], static_cast<unsigned long long>(v)); } while (0)
-#else
-#define PROF_DECL(name)
-#define PROF_T0(t)
-#define PROF_ADD(acc, t)
-#define PROF_FLUSH(idx, v)
-#endif
-
 namespace {
-
-constexpr int kStageBytes = 17408;  // 136 rows x 128 B (mode 0 uses BW + 2 rows, mode 1 uses 128)
-constexpr int kMaxStages = 12;
-constexpr int kMiscBytes = 1024;
-constexpr int kSmemMax = 232448;    // 227 KB opt-in limit per CTA
-constexpr int kTileFBytes = 16384;  // 128 px x 32 fp32
-
-struct RowRange {   // 32-bit on purpose: 64-bit divisions are ~100-instruction subroutines and every role decodes its strips
-    int g0, g1;     // (the launcher refuses problems with rows_total * grid >= 2^31)
-};
-
-// K-major, 128B-swizzled operand descriptor: constant high word (SBO = 1024 B, version 1, SWIZZLE_128B) + low word.
-constexpr uint32_t kDescHi = (1024u >> 4) | (1u << 14) | (2u << 29);
-__device__ __forceinline__ uint64_t desc_of(uint32_t lo) { return (static_cast<uint64_t>(kDescHi) << 32) | lo; }
-
-// one staging buffer of an epilogue group: [fp32 tile][16-bit tile]
-__host__ __device__ inline int epi_buf_bytes_pair(const ConvArgs& a, int subw) {
-    const int f = a.has_outf ? kTileFBytes : 0;
-    const int h = a.has_out16 ? 128 * subw * 2 : 0;
-    return f + (h + 1023) / 1024 * 1024;
-}
-__host__ __device__ inline int epi_group_bytes_pair(const ConvArgs& a, int subw) {
-    return (a.epi_bufs == 2 ? 2 : 1) * epi_buf_bytes_pair(a, subw);
-}
 
 template <int S>
 __device__ __forceinline__ uint32_t ring_slot(uint32_t v) { return (S - v % S) % S; }
 template <int S>
 __device__ __forceinline__ uint32_t ring_parity(uint32_t v) { return (v / S) & 1u; }
-
-__device__ __forceinline__ void unpack16x8(const uint4 q, int fmt, float (&f)[8]) {
-    const uint32_t w4[4] = {q.x, q.y, q.z, q.w};
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        if (fmt == 1) {
-            f[2 * i] = __uint_as_float(w4[i] << 16);
-            f[2 * i + 1] = __uint_as_float(w4[i] & 0xFFFF0000u);
-        } else {
-            const float2 h = __half22float2(*reinterpret_cast<const __half2*>(&w4[i]));
-            f[2 * i] = h.x;
-            f[2 * i + 1] = h.y;
-        }
-    }
-}
 
 // MMAs [I0, I1) of one pipeline stage (i = dx * KS + ks), straight-line. One N = 3 * NOUT instruction per K16 step.
 template <int NOUT, int KS, int I0, int I1>
@@ -137,8 +75,6 @@ __device__ __forceinline__ void mma_role(const ConvArgs& a, const RowRange rr, c
     bool full_ready = false, slot_ready = false;
     uint32_t vnew = 1;               // virtual index of the NEWEST accumulator the next row touches (out row r+1)
     uint32_t acq = 0;                // accumulators acquired so far (virtual indices < acq)
-    PROF_DECL(p_full); PROF_DECL(p_slot); PROF_DECL(p_steps);
-    PROF_T0(p_t0);
     for (int g = rr.g0; g < rr.g1;) {
         const int ya = g % H;
         const int yb = min(H, ya + (rr.g1 - g));
@@ -149,12 +85,10 @@ __device__ __forceinline__ void mma_role(const ConvArgs& a, const RowRange rr, c
             if (slot_ready && acq == vnew) {
                 ++acq;
             } else {
-                PROF_T0(p_t);
                 while (static_cast<int>(vnew - acq) >= 0) {
                     mbar_wait_a(slotfree_a + (ring_slot<S>(acq) << 3), ring_parity<S>(acq));
                     ++acq;
                 }
-                PROF_ADD(p_slot, p_t);
             }
             slot_ready = false;
             tc_fence_after();
@@ -162,11 +96,8 @@ __device__ __forceinline__ void mma_role(const ConvArgs& a, const RowRange rr, c
             const uint32_t d0 = tbase + s0 * NOUT;   // the three dy blocks land on s0, s0+1, s0+2 (possibly overflow slots)
             uint32_t b_lo = w_lo;
             for (int st = 0; st < nsteps; ++st, b_lo += b_step) {
-                if (!full_ready) { PROF_T0(p_t); mbar_wait_a(full_a + (stage << 3), phase); PROF_ADD(p_full, p_t); }
+                if (!full_ready) mbar_wait_a(full_a + (stage << 3), phase);
                 tc_fence_after();
-#ifdef RESR_PROFILE_WAITS
-                ++p_steps;
-#endif
                 const bool last = (st == nsteps - 1);
                 const int ks = (st >= nsteps - (MODE == 0 ? 1 : 3)) ? a.tail_ksteps : 4;  // steps of the last K chunk
                 if (elect_one()) {
@@ -199,33 +130,12 @@ __device__ __forceinline__ void mma_role(const ConvArgs& a, const RowRange rr, c
         if (elect_one()) umma2_commit_mc(empty_a + (pending_empty << 3), 3);
         __syncwarp();
     }
-#ifdef RESR_PROFILE_WAITS
-    PROF_FLUSH(0, clock64() - p_t0); PROF_FLUSH(1, p_full); PROF_FLUSH(2, p_slot); PROF_FLUSH(3, p_steps);
-#endif
 }
 
-template <int W>
-__device__ __forceinline__ void tmem_ld_w(uint32_t taddr, float* v) {
-    if (W == 32) tmem_ld32(taddr, v); else tmem_ld16(taddr, v);
-}
 template <int W>
 __device__ __forceinline__ void tmem_zero_w(uint32_t taddr) {
     if (W == 32) tmem_st_zero32(taddr); else tmem_st_zero16(taddr);
 }
-// Re-arm an accumulator with the layer's BIAS instead of zero: the MMAs then accumulate on top of it and the epilogue
-// needs no bias add (32 FADDs + their shared loads per pass for 8 vector loads; the epilogue warps are issue-bound:
-// 41.0 -> 39.8 ms per cfg3 forward, same-box A/B in profiles/r02_epilogue_ab.txt).
-template <int W>
-__device__ __forceinline__ void tmem_init_bias(uint32_t taddr, const float* __restrict__ bias_w) {
-    float b[W];
-#pragma unroll
-    for (int i = 0; i < W / 4; ++i) {
-        const float4 q = reinterpret_cast<const float4*>(bias_w)[i];
-        b[4 * i] = q.x; b[4 * i + 1] = q.y; b[4 * i + 2] = q.z; b[4 * i + 3] = q.w;
-    }
-    if (W == 32) tmem_st32(taddr, b); else tmem_st16(taddr, b);
-}
-
 }  // namespace
 
 // MASKED: the packed-canvas variant (ConvArgs::vmask set); the other instantiation carries no mask code at all
@@ -248,7 +158,7 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_cons
     const int slice = blockIdx.y;
     const uint32_t rank = cluster_ctarank();
     const uint32_t wbytes = static_cast<uint32_t>(a.nchunks) * 3u * WHALF;
-    const int epi_bytes = epi_group_bytes_pair(a, SUBW);
+    const int epi_bytes = epi_group_bytes(a, SUBW);
 
     uint8_t* wsm = smem;
     uint8_t* stg = smem + wbytes;
@@ -336,8 +246,6 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_cons
         const int ndx = a.mode == 0 ? 1 : 3;
         const uint32_t tx_bytes = a.mode == 0 ? (a.BW + 2) * 128 : 128 * 128;
         const uint32_t full0 = map_to_cta(smem_u32(full), 0);  // the leader's stage barriers
-        PROF_DECL(p_empty);
-        PROF_T0(p_t0);
         const int ncg2 = (a.ncg + 1) >> 1;
         for (int g = rr.g0; g < rr.g1;) {
             const int cg2 = g / H;
@@ -350,7 +258,7 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_cons
             for (int r = ra; r <= rb; ++r) {
                 for (int c = 0; c < a.nchunks; ++c) {
                     for (int dx = 0; dx < ndx; ++dx) {
-                        { PROF_T0(p_t); mbar_wait(empty + stage, phase ^ 1); PROF_ADD(p_empty, p_t); }
+                        mbar_wait(empty + stage, phase ^ 1);
                         if (elect_one()) {
                             // rank 1 does not arrive: its bytes are counted by the leader's expect_tx (the transaction count
                             // may go negative for a moment; the phase cannot complete before the leader's own arrive, and
@@ -366,9 +274,6 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_cons
             }
             g += yb - ya;
         }
-#ifdef RESR_PROFILE_WAITS
-        PROF_FLUSH(4, clock64() - p_t0); PROF_FLUSH(5, p_empty);
-#endif
     } else if (warp == 1) {
         // ------------------------------------------------------------------ MMA issuer (leader CTA only)
         mbar_wait(wbar, 0);   // this CTA's half of the weights is resident
@@ -386,10 +291,7 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_cons
         const int q = warp & 3;        // TMEM lane quadrant this warp may access
         const int m = q * 32 + lane;   // M row == TMEM lane == pixel of this CTA's tile
         const bool lead_warp = ((warp - 4) & 3) == 0;
-        uint8_t* const tile_base = epi + gi * epi_bytes;
-        const int buf_bytes = epi_buf_bytes_pair(a, SUBW);
-        const bool two_bufs = a.epi_bufs == 2;
-        uint32_t pass = 0;   // staged passes of this group so far (selects the staging buffer)
+        EpiGroup grp{epi + gi * epi_bytes, epi_buf_bytes(a, SUBW), a.epi_bufs == 2, 0, gi, m, lead_warp};
         const uint32_t lane_base = tbase + (static_cast<uint32_t>(q * 32) << 16);
         const uint32_t free0 = map_to_cta(smem_u32(slot_free), 0);  // the leader's slot barriers
         const int img_in_tile = m / a.BW;
@@ -410,8 +312,6 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_cons
                 for (int s = s_lo; s < s_hi; ++s) mbar_arrive_cluster(free0 + (s << 3));
         }
         grid_dep_wait();  // residual reads / output writes below touch buffers of the previous kernel
-        PROF_DECL(p_acc); PROF_DECL(p_tile); PROF_DECL(p_drain); PROF_DECL(p_math); PROF_DECL(p_store); PROF_DECL(p_rows);
-        PROF_T0(p_t0);
         uint32_t v0 = 0;
         const int ncg2 = (a.ncg + 1) >> 1;
         for (int g = rr.g0; g < rr.g1;) {
@@ -421,9 +321,6 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_cons
             const int yb = min(H, ya + (rr.g1 - g));
             const int n0 = (cg / a.nxs) * a.BN;
             const int x0 = (cg % a.nxs) * a.BW;
-            const int n = n0 + img_in_tile;
-            const int x = x0 + x_in_tile;
-            const bool valid = (n < a.N) && (x < a.W);
             const int ra = max(ya - 1, 0), rb = min(yb, H - 1);
             const int n_acc = rb - ra + 3;
             for (int j = 0; j < n_acc; ++j) {
@@ -436,47 +333,19 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_cons
                 const uint32_t col = slot * NOUT;
                 const uint32_t col2 = (S + slot) * NOUT;  // overflow twin (ring positions 0 and 1 only)
                 const bool dual = slot < 2;
-                const size_t pix = (static_cast<size_t>(valid ? n : 0) * a.H + y) * a.W + (valid ? x : 0);
-                bool inside = true;   // canvas pixel of an image (vmask), read before the accumulator wait like the residual
-                if (MASKED && emit) {
-                    const int lx = (valid ? x : 0) >> a.vmask_shift, ly = y >> a.vmask_shift;
-                    inside = (__ldg(a.vmask + static_cast<size_t>(ly) * a.vmask_words + (lx >> 5)) >> (lx & 31)) & 1u;
-                }
+                const EpiPixel px = epi_pixel<MASKED>(a, n0, x0, n0 + img_in_tile, x0 + x_in_tile, y, emit);
                 bool waited = false;
 #pragma unroll 1
                 for (int h = 0; h < NSUB; ++h) {
                     const int ls = slice * NSUB + h;   // logical 32-channel slice (channel offsets, per-slice flags)
-                    const bool use_res1 = a.has_res1 && !((a.slice_nores_mask >> ls) & 1u);
-                    const bool use_outf = a.has_outf && !((a.slice_noutf_mask >> ls) & 1u);
-                    const bool use_o16 = a.has_out16 && !((a.slice_no16_mask >> ls) & 1u);
-                    const bool staged = use_o16 || use_outf;
-                    float4 resv[SUBW / 4];   // fp32 residual, or (res16) SUBW 16-bit values in the first SUBW / 8 entries
-                    if (emit && use_res1) {
-                        // requested before the wait for the accumulator: the latency hides behind the row's MMAs
-                        if (a.res16) {
-                            const uint4* rp = reinterpret_cast<const uint4*>(static_cast<const uint16_t*>(a.res1) + pix * a.res1_cstride +
-                                                                             a.res_choff + ls * SUBW);
-#pragma unroll
-                            for (int i = 0; i < SUBW / 8; ++i) {
-                                const uint4 q4 = rp[i];
-                                resv[i] = make_float4(__uint_as_float(q4.x), __uint_as_float(q4.y), __uint_as_float(q4.z), __uint_as_float(q4.w));
-                            }
-                        } else {
-                            const float4* rp = reinterpret_cast<const float4*>(static_cast<const float*>(a.res1) + pix * a.res1_cstride +
-                                                                               a.res_choff + ls * SUBW);
-#pragma unroll
-                            for (int i = 0; i < SUBW / 4; ++i) resv[i] = rp[i];
-                        }
-                    }
+                    float4 resv[SUBW / 4];
+                    if (emit && slice_on(a.has_res1, a.slice_nores_mask, ls)) epi_load_res1<SUBW>(a, px.pix, ls, resv);
                     if (!waited) {
-                        PROF_T0(p_t);
                         mbar_wait(acc_full + slot, ring_parity<S>(v));
-                        PROF_ADD(p_acc, p_t);
                         tc_fence_after();
                         waited = true;
                     }
                     float val[SUBW];
-                    PROF_T0(p_td);
                     tmem_ld_w<SUBW>(lane_base + col + h * SUBW, val);
                     if (dual) {
                         float val2[SUBW];
@@ -495,216 +364,13 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_cons
                         __syncwarp();
                         if (lane == 0) mbar_arrive_cluster(free0 + (slot << 3));
                     }
-                    PROF_ADD(p_drain, p_td);
-                    if (!emit) continue;
-                    PROF_T0(p_tm);
-#ifdef RESR_PROFILE_WAITS
-                    ++p_rows;
-#endif
-
-                    // (no bias add here: the accumulator was armed with the bias, tmem_init_bias)
-                    if (use_res1 && a.res16) {  // widen the 16-bit residual in place (consumed below as fp32)
-                        float wide[SUBW];
-#pragma unroll
-                        for (int i = 0; i < SUBW / 8; ++i) {
-                            float f8[8];
-                            unpack16x8(make_uint4(__float_as_uint(resv[i].x), __float_as_uint(resv[i].y), __float_as_uint(resv[i].z),
-                                                  __float_as_uint(resv[i].w)), a.res16_fmt, f8);
-#pragma unroll
-                            for (int e = 0; e < 8; ++e) wide[8 * i + e] = f8[e];
-                        }
-#pragma unroll
-                        for (int i = 0; i < SUBW / 4; ++i) resv[i] = make_float4(wide[4 * i], wide[4 * i + 1], wide[4 * i + 2], wide[4 * i + 3]);
-                    }
-                    if (use_res1) {
-#pragma unroll
-                        for (int i = 0; i < SUBW / 4; ++i) {
-                            const float4 r4 = resv[i];
-                            if (a.ep_mode == EP_SKIP || a.ep_mode == EP_ADD2) {
-                                val[4 * i + 0] = __fadd_rn(r4.x, val[4 * i + 0]);
-                                val[4 * i + 1] = __fadd_rn(r4.y, val[4 * i + 1]);
-                                val[4 * i + 2] = __fadd_rn(r4.z, val[4 * i + 2]);
-                                val[4 * i + 3] = __fadd_rn(r4.w, val[4 * i + 3]);
-                            } else {   // v * 0.2 + r: separately rounded product and sum (reference order), two lanes per instruction
-                                const float2 p01 = __fmul2_rn(make_float2(val[4 * i + 0], val[4 * i + 1]), make_float2(0.2f, 0.2f));
-                                const float2 p23 = __fmul2_rn(make_float2(val[4 * i + 2], val[4 * i + 3]), make_float2(0.2f, 0.2f));
-                                const float2 s01 = __fadd2_rn(p01, make_float2(r4.x, r4.y));
-                                const float2 s23 = __fadd2_rn(p23, make_float2(r4.z, r4.w));
-                                val[4 * i + 0] = s01.x; val[4 * i + 1] = s01.y; val[4 * i + 2] = s23.x; val[4 * i + 3] = s23.y;
-                            }
-                        }
-                    }
-                    PROF_ADD(p_math, p_tm);
-                    uint8_t* const tileR = tile_base + ((two_bufs && (pass & 1u)) ? buf_bytes : 0);  // fp32 output tile
-                    uint8_t* const tile16 = tileR + (a.has_outf ? kTileFBytes : 0);                  // 16-bit output tile
-                    if (staged) {
-                        // the staging buffer is free once the TMA stores that last used it have read it: the previous pass's
-                        // (one buffer) or the pass before that (two buffers: the wait is normally already satisfied)
-                        PROF_T0(p_t);
-                        if (lead_warp) { if (two_bufs) tma_store_wait_read1(); else tma_store_wait_read(); }
-                        named_bar_sync(1 + gi, 128);
-                        PROF_ADD(p_tile, p_t);
-                        ++pass;
-                    }
-                    PROF_T0(p_ts);
-                    if (a.ep_mode == EP_RRDB) {
-                        if (a.res16) {
-                            // plain (coherent) loads: in the inference trunk res2 is the RRDB input held in the very buffer
-                            // this launch overwrites -- each element is read by the thread that later stores its replacement
-                            const uint4* r2 = reinterpret_cast<const uint4*>(static_cast<const uint16_t*>(a.res2) + pix * a.res2_cstride +
-                                                                             a.res_choff + ls * SUBW);
-#pragma unroll
-                            for (int i = 0; i < SUBW / 8; ++i) {
-                                float f8[8];
-                                unpack16x8(r2[i], a.res16_fmt, f8);
-#pragma unroll
-                                for (int e = 0; e < 8; e += 2) {
-                                    const float2 pp = __fmul2_rn(make_float2(val[8 * i + e], val[8 * i + e + 1]), make_float2(0.2f, 0.2f));
-                                    const float2 ss = __fadd2_rn(pp, make_float2(f8[e], f8[e + 1]));
-                                    val[8 * i + e] = ss.x; val[8 * i + e + 1] = ss.y;
-                                }
-                            }
-                        } else {
-                            const float4* r2 = reinterpret_cast<const float4*>(static_cast<const float*>(a.res2) + pix * a.res2_cstride +
-                                                                               a.res_choff + ls * SUBW);
-#pragma unroll
-                            for (int i = 0; i < SUBW / 4; ++i) {
-                                const float4 r4 = __ldg(r2 + i);
-                                val[4 * i + 0] = __fadd_rn(__fmul_rn(val[4 * i + 0], 0.2f), r4.x);
-                                val[4 * i + 1] = __fadd_rn(__fmul_rn(val[4 * i + 1], 0.2f), r4.y);
-                                val[4 * i + 2] = __fadd_rn(__fmul_rn(val[4 * i + 2], 0.2f), r4.z);
-                                val[4 * i + 3] = __fadd_rn(__fmul_rn(val[4 * i + 3], 0.2f), r4.w);
-                            }
-                        }
-                    }
-                    if (a.ep_mode == EP_ADD2 && a.res2) {
-                        const float4* r2 = reinterpret_cast<const float4*>(static_cast<const float*>(a.res2) + pix * a.res2_cstride + a.res_choff + ls * SUBW);
-#pragma unroll
-                        for (int i = 0; i < SUBW / 4; ++i) {
-                            const float4 r4 = __ldg(r2 + i);
-                            val[4 * i + 0] = fmaf(a.res2_scale, r4.x, val[4 * i + 0]);
-                            val[4 * i + 1] = fmaf(a.res2_scale, r4.y, val[4 * i + 1]);
-                            val[4 * i + 2] = fmaf(a.res2_scale, r4.z, val[4 * i + 2]);
-                            val[4 * i + 3] = fmaf(a.res2_scale, r4.w, val[4 * i + 3]);
-                        }
-                    }
-                    if (a.lrelu) {   // max(v, 0.2 v) == (v > 0 ? v : 0.2 v) for every finite v; the product is one packed FMUL2 per pair
-#pragma unroll
-                        for (int i = 0; i < SUBW / 2; ++i) {
-                            const float2 t = __fmul2_rn(make_float2(val[2 * i], val[2 * i + 1]), make_float2(0.2f, 0.2f));
-                            val[2 * i] = fmaxf(val[2 * i], t.x);
-                            val[2 * i + 1] = fmaxf(val[2 * i + 1], t.y);
-                        }
-                    }
-                    if (MASKED && !inside) {   // gutter / canvas margin: 0 in every output, as the zero padding around an image
-#pragma unroll
-                        for (int i = 0; i < SUBW; ++i) val[i] = 0.f;
-                    }
-                    if (a.out_nchw_raw && valid) {
-                        const size_t plane = static_cast<size_t>(a.H) * a.W;
-                        float* o = a.out_nchw_raw + static_cast<size_t>(n) * a.out_nchw_c * plane + static_cast<size_t>(y) * a.W + x;
-#pragma unroll
-                        for (int c = 0; c < SUBW; ++c) {
-                            const int cc = ls * SUBW + c;
-                            if (cc < a.out_nchw_c) o[static_cast<size_t>(cc) * plane] = val[c];
-                        }
-                    }
-                    if (a.clamp01) {
-#pragma unroll
-                        for (int i = 0; i < SUBW; ++i) val[i] = fminf(fmaxf(val[i], 0.f), 1.f);
-                    }
-                    if (use_outf) {  // fp32 master (SUBW == 32 only)
-#pragma unroll
-                        for (int i = 0; i < SUBW / 4; ++i)
-                            *reinterpret_cast<float4*>(tileR + m * 128 + ((i ^ (m & 7)) << 4)) =
-                                make_float4(val[4 * i], val[4 * i + 1], val[4 * i + 2], val[4 * i + 3]);
-                    }
-                    if (use_o16 && a.mask16) {  // LeakyReLU backward: slope 1 where the saved activation is > 0, else 0.2
-                        const uint4* mk = reinterpret_cast<const uint4*>(static_cast<const uint16_t*>(a.mask16) + pix * a.mask16_cstride +
-                                                                         a.mask16_choff + ls * SUBW);
-#pragma unroll
-                        for (int i = 0; i < SUBW / 8; ++i) {
-                            const uint4 q4 = __ldg(mk + i);
-                            const uint32_t w4[4] = {q4.x, q4.y, q4.z, q4.w};
-#pragma unroll
-                            for (int e = 0; e < 8; ++e) {
-                                const uint32_t h16 = (w4[e >> 1] >> ((e & 1) * 16)) & 0xFFFFu;
-                                const bool pos = ((h16 & 0x8000u) == 0) && ((h16 & 0x7FFFu) != 0);
-                                if (!pos) val[8 * i + e] = __fmul_rn(val[8 * i + e], 0.2f);
-                            }
-                        }
-                    }
-                    if (use_o16 && a.out16_scale != 0.f) {
-#pragma unroll
-                        for (int i = 0; i < SUBW; ++i) val[i] = __fmul_rn(val[i], a.out16_scale);
-                    }
-                    if (use_o16) {
-                        uint32_t pk[SUBW / 2];
-#pragma unroll
-                        for (int i = 0; i < SUBW / 2; ++i) {
-                            if (a.out16_fmt == 1) {
-                                __nv_bfloat162 hh = __floats2bfloat162_rn(val[2 * i], val[2 * i + 1]);
-                                pk[i] = *reinterpret_cast<uint32_t*>(&hh);
-                            } else {
-                                pk[i] = pack_f16x2_sat(val[2 * i], val[2 * i + 1]);  // saturate, never inf
-                            }
-                        }
-                        // (Storing the pixel's channels straight from registers instead -- no staging tile, no proxy fence, no
-                        // block barrier -- was tried and is slower: 45.5 vs 43.0 ms per cfg3 forward, profiles/r02_direct_store_ab.txt.)
-                        uint4* dst = reinterpret_cast<uint4*>(tile16 + m * (SUBW * 2));
-#pragma unroll
-                        for (int i = 0; i < SUBW / 8; ++i) dst[i] = make_uint4(pk[4 * i], pk[4 * i + 1], pk[4 * i + 2], pk[4 * i + 3]);
-                    }
-                    if (staged) {
-                        fence_proxy_async_smem();
-                        named_bar_sync(1 + gi, 128);
-                        if (lead_warp) {
-                            if (elect_one()) {
-                                if (use_outf) tma_store_4d(&tmapOF, tileR, a.outf_choff + ls * SUBW, x0, y, n0);
-                                if (use_o16) {
-                                    const int c0 = a.out16_choff + (a.out16_slice_fixed ? 0 : ls * SUBW);
-                                    if (!a.out16_up2) {
-                                        tma_store_4d(&tmapO16, tile16, c0, x0, y, n0);
-                                    } else {
-#pragma unroll
-                                        for (int s = 0; s < 4; ++s) tma_store_5d(&tmapO16, tile16, c0, s & 1, x0, 2 * y + (s >> 1), n0);
-                                    }
-                                }
-                                tma_store_commit();
-                            }
-                            __syncwarp();
-                        }
-                    }
-                    PROF_ADD(p_store, p_ts);
-                    if (a.out_nchw && valid) {
-                        const size_t plane = static_cast<size_t>(a.H) * a.W;
-                        float* o = a.out_nchw + static_cast<size_t>(n) * a.out_nchw_c * plane + static_cast<size_t>(y) * a.W + x;
-#pragma unroll
-                        for (int c = 0; c < SUBW; ++c) {
-                            const int cc = ls * SUBW + c;
-                            if (cc < a.out_nchw_c) o[static_cast<size_t>(cc) * plane] = val[c];
-                        }
-                    }
-                    if (a.out_u8 && valid) {   // clamp01 has been applied: v * 255 lies in [0, 255], the cast truncates
-                        unsigned char* o = a.out_u8 + ((static_cast<size_t>(n) * a.H + y) * a.W + x) * a.out_nchw_c;
-#pragma unroll
-                        for (int c = 0; c < SUBW; ++c) {
-                            const int cc = ls * SUBW + c;
-                            if (cc < a.out_nchw_c) o[cc] = static_cast<unsigned char>(fminf(fmaxf(__fmul_rn(val[c], 255.f), 0.f), 255.f));
-                        }
-                    }
+                    if (emit) epi_pass<SUBW, MASKED>(a, &tmapO16, &tmapOF, grp, px, ls, val, resv);
                 }
             }
             v0 += n_acc;
             g += yb - ya;
         }
         if (lead_warp) tma_store_wait_all();
-#ifdef RESR_PROFILE_WAITS
-        if (warp == 4) {
-            PROF_FLUSH(6, clock64() - p_t0); PROF_FLUSH(7, p_acc); PROF_FLUSH(8, p_tile);
-            PROF_FLUSH(9, p_drain); PROF_FLUSH(10, p_math); PROF_FLUSH(11, p_store); PROF_FLUSH(12, p_rows);
-        }
-#endif
     }
 
     // no CTA of the pair may exit while its peer can still signal its barriers / read its shared memory
@@ -715,20 +381,18 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_cons
 
 // --------------------------------------------------------------------------------------------- host side
 
-bool conv3x3_pair_plan_smem(ConvArgs* a, int nout) {
-    const int subw = nout == 64 ? 32 : nout;
-    const int wbytes = a->nchunks * 3 * (3 * nout / 2) * 128;
-    int nepi = a->has_outf ? 2 : 3;
-    const char* env = getenv("RESR_CONV_NEPI");
-    if (env) nepi = atoi(env);
-    if (nepi < 1) nepi = 1;
-    if (nepi > 3) nepi = 3;
-    static const int env_bufs = getenv("RESR_CONV_EPI_BUFS") ? atoi(getenv("RESR_CONV_EPI_BUFS")) : 2;
-    for (;; --nepi) {
+// Fills nepi / epi_bufs / nstages from the shared-memory budget of a CTA that keeps `wbytes` of weights resident and
+// stages `subw` channels per epilogue pass; `max_bufs` (1 or 2) staging buffers per epilogue group at most. Returns
+// false if the configuration does not fit.
+static bool plan_smem(ConvArgs* a, int wbytes, int subw, int max_bufs) {
+    // The per-row epilogue latency (TMEM drain, staging, TMA store; ~1.6k cycles, more with an fp32 output tile) is hidden
+    // by running several epilogue groups on consecutive rows. Three groups whenever they fit beside at least four
+    // stages (8 KB of shared memory each without an fp32 tile); two with the 24 KB fp32 variant.
+    for (int nepi = a->has_outf ? 2 : 3;; --nepi) {
         a->nepi = nepi;
-        for (int bufs = env_bufs == 2 ? 2 : 1; bufs >= 1; --bufs) {
+        for (int bufs = max_bufs; bufs >= 1; --bufs) {
             a->epi_bufs = bufs;
-            const int fixed = 1024 + wbytes + nepi * epi_group_bytes_pair(*a, subw) + kMiscBytes;
+            const int fixed = 1024 + wbytes + nepi * epi_group_bytes(*a, subw) + kMiscBytes;
             int ns = (kSmemMax - fixed) / kStageBytes;
             if (ns > kMaxStages) ns = kMaxStages;
             // two staging tiles per group only where they do not eat into the activation ring (>= 6 stages left)
@@ -738,73 +402,6 @@ bool conv3x3_pair_plan_smem(ConvArgs* a, int nout) {
             }
         }
     }
-}
-
-template <int NOUT, bool MASKED>
-static cudaError_t launch_pair_t(const ConvMaps& maps, const ConvArgs& args, dim3 grid, int threads, cudaStream_t stream) {
-    static PerDevice<bool> attr;  // function attributes are per device
-    if (!attr.cur()) {
-        cudaError_t e = cudaFuncSetAttribute(conv3x3_pair_kernel<NOUT, MASKED>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax);
-        if (e != cudaSuccess) return e;
-        attr.cur() = true;
-    }
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = grid;
-    cfg.blockDim = dim3(threads, 1, 1);
-    cfg.dynamicSmemBytes = kSmemMax;  // the full 227 KB: exactly one CTA (one 512-column TMEM allocation) per SM
-    cfg.stream = stream;
-    cudaLaunchAttribute at[2];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    at[1].id = cudaLaunchAttributeClusterDimension;
-    at[1].val.clusterDim.x = 2;
-    at[1].val.clusterDim.y = 1;
-    at[1].val.clusterDim.z = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = 2;
-    return cudaLaunchKernelEx(&cfg, conv3x3_pair_kernel<NOUT, MASKED>, maps.a, maps.o16, maps.of, args);
-}
-
-// `nout`: accumulator columns per output row and pair (64, 32, 16); `nslices` pair-slices cover Cout (blockIdx.y).
-cudaError_t conv3x3_pair_launch(const ConvMaps& maps, const ConvArgs& args_in, int nout, int nslices, int num_sms,
-                                cudaStream_t stream) {
-    ConvArgs args = args_in;
-    const int subw = nout == 64 ? 32 : nout;
-    const int wbytes = args.nchunks * 3 * (3 * nout / 2) * 128;
-    const int smem = 1024 + wbytes + args.nstages * kStageBytes + args.nepi * epi_group_bytes_pair(args, subw) + kMiscBytes;
-    if (args.nstages < 2 || args.nepi < 1 || args.nepi > 3 || smem > kSmemMax) return cudaErrorInvalidConfiguration;
-    if (args.has_outf && subw != 32) return cudaErrorInvalidConfiguration;
-    const long long ncg2 = (args.ncg + 1) / 2;
-    args.rows_total_pair = ncg2 * args.H;
-    long long npairs = (num_sms / 2) / nslices;
-    const long long min_rows = 4;  // do not shred tiny problems into 1-row strips (2 halo rows each)
-    const long long cap = (args.rows_total_pair + min_rows - 1) / min_rows;
-    if (npairs > cap) npairs = cap;
-    if (npairs < 1) npairs = 1;
-    if (args.rows_total_pair * (npairs + 1) >= (1ll << 31)) return cudaErrorInvalidValue;   // the kernel's strip arithmetic is 32-bit
-    if (args.tail_ksteps != 1 && args.tail_ksteps != 2 && args.tail_ksteps != 4) args.tail_ksteps = 4;
-    const dim3 grid(static_cast<unsigned>(2 * npairs), static_cast<unsigned>(nslices), 1);
-    const int threads = 128 + 128 * args.nepi;
-    if (args.vmask) {
-        if (nout == 64) return launch_pair_t<64, true>(maps, args, grid, threads, stream);
-        if (nout == 32) return launch_pair_t<32, true>(maps, args, grid, threads, stream);
-        if (nout == 16) return launch_pair_t<16, true>(maps, args, grid, threads, stream);
-        return cudaErrorInvalidValue;
-    }
-    if (nout == 64) return launch_pair_t<64, false>(maps, args, grid, threads, stream);
-    if (nout == 32) return launch_pair_t<32, false>(maps, args, grid, threads, stream);
-    if (nout == 16) return launch_pair_t<16, false>(maps, args, grid, threads, stream);
-    return cudaErrorInvalidValue;
-}
-
-int conv3x3_wait_profile(unsigned long long* out16, int reset) {
-    if (out16 && cudaMemcpyFromSymbol(out16, g_wait_prof, sizeof(unsigned long long) * 16) != cudaSuccess) return -1;
-    if (reset) {
-        unsigned long long z[16] = {0};
-        if (cudaMemcpyToSymbol(g_wait_prof, z, sizeof(z)) != cudaSuccess) return -1;
-    }
-    return 0;
 }
 
 // 0: never pair, 1: pair when the problem is large enough (default), 2: pair whenever two column groups exist
@@ -817,8 +414,7 @@ int conv3x3_set_pair_policy(int policy) {
 }
 
 bool conv3x3_choose(ConvArgs* a, int pack_nout, int pack_nslices, ConvLaunchCfg* cfg) {
-    const int env_pair = conv3x3_set_pair_policy(-1);
-    static const int env_n64 = getenv("RESR_CONV_PAIR_N64") ? atoi(getenv("RESR_CONV_PAIR_N64")) : 1;
+    const int policy = conv3x3_set_pair_policy(-1);
     cfg->pair = 0;
     cfg->nout = pack_nout;
     cfg->nslices = pack_nslices;
@@ -826,23 +422,40 @@ bool conv3x3_choose(ConvArgs* a, int pack_nout, int pack_nslices, ConvLaunchCfg*
     // 256 pair-rows over 74 pairs) the launch is dominated by its prologue and the two halo rows per strip, and the
     // single-CTA kernel is as fast or faster (measured 25.6 vs 26.4 ms per training step). RESR_CONV_PAIR=2 forces pairs.
     const long long pair_rows = static_cast<long long>((a->ncg + 1) / 2) * a->H;
-    const bool big_enough = pair_rows >= 6 * 74 || env_pair == 2;
-    if (env_pair && a->ncg >= 2 && big_enough) {
+    const bool big_enough = pair_rows >= 6 * 74 || policy == 2;
+    if (policy && a->ncg >= 2 && big_enough) {
         ConvArgs t = *a;
         int nout = pack_nout, nslices = pack_nslices;
-        if (env_n64 && pack_nout == 32 && pack_nslices % 2 == 0) { nout = 64; nslices = pack_nslices / 2; }
-        if (conv3x3_pair_plan_smem(&t, nout)) {
+        // two 32-channel pack slices per pair: the 192 -> 64 convolution of a dense block is ONE N = 192 MMA per K step
+        if (pack_nout == 32 && pack_nslices % 2 == 0) { nout = 64; nslices = pack_nslices / 2; }
+        if (plan_smem(&t, conv3x3_weight_bytes(t, nout, 2), nout == 64 ? 32 : nout, 2)) {
             *a = t;
             cfg->pair = 1; cfg->nout = nout; cfg->nslices = nslices;
             return true;
         }
     }
-    return conv3x3_plan_smem(a, pack_nout);
+    return plan_smem(a, conv3x3_weight_bytes(*a, pack_nout, 1), pack_nout, 1);   // the single-CTA kernel stages in one buffer
 }
 
-cudaError_t conv3x3_run(const ConvMaps& maps, const ConvArgs& args, const ConvLaunchCfg& cfg, int num_sms, cudaStream_t stream) {
-    if (cfg.pair) return conv3x3_pair_launch(maps, args, cfg.nout, cfg.nslices, num_sms, stream);
-    return conv3x3_launch(maps, args, cfg.nout, cfg.nslices, num_sms, stream);
+cudaError_t conv3x3_run(const ConvMaps& maps, const ConvArgs& args_in, const ConvLaunchCfg& cfg, int num_sms, cudaStream_t stream) {
+    ConvArgs args = args_in;
+    if (args.tail_ksteps != 1 && args.tail_ksteps != 2 && args.tail_ksteps != 4) args.tail_ksteps = 4;
+    if (!cfg.pair) return conv3x3_tc_launch(maps, args, cfg.nout, cfg.nslices, num_sms, stream);
+    // `nout`: accumulator columns per output row and pair (64, 32, 16); `nslices` pair-slices cover Cout (blockIdx.y)
+    const int nout = cfg.nout, nslices = cfg.nslices;
+    if (args.has_outf && nout == 16) return cudaErrorInvalidConfiguration;   // the fp32 tile holds 32 channels
+    args.rows_total_pair = static_cast<long long>((args.ncg + 1) / 2) * args.H;
+    const long long units = args.rows_total_pair;
+    if (args.vmask) {
+        if (nout == 64) return conv3x3_launch_grid<conv3x3_pair_kernel<64, true>>(maps, args, 64, 2, units, nslices, num_sms, stream);
+        if (nout == 32) return conv3x3_launch_grid<conv3x3_pair_kernel<32, true>>(maps, args, 32, 2, units, nslices, num_sms, stream);
+        if (nout == 16) return conv3x3_launch_grid<conv3x3_pair_kernel<16, true>>(maps, args, 16, 2, units, nslices, num_sms, stream);
+        return cudaErrorInvalidValue;
+    }
+    if (nout == 64) return conv3x3_launch_grid<conv3x3_pair_kernel<64, false>>(maps, args, 64, 2, units, nslices, num_sms, stream);
+    if (nout == 32) return conv3x3_launch_grid<conv3x3_pair_kernel<32, false>>(maps, args, 32, 2, units, nslices, num_sms, stream);
+    if (nout == 16) return conv3x3_launch_grid<conv3x3_pair_kernel<16, false>>(maps, args, 16, 2, units, nslices, num_sms, stream);
+    return cudaErrorInvalidValue;
 }
 
 }  // namespace resr

@@ -15,41 +15,18 @@
 //     shared-memory descriptor by dx * 128 B; mode 1 issues one TMA load per dx (used when the lanes span images).
 //   * Weights of the CTA's Cout slice stay resident in shared memory for the whole launch (bulk copies).
 //   * CTAs are persistent over a contiguous range of (column group, row) work; grid = #SMs / #slices.
-//   * Epilogue: one or two groups of 4 warps take alternate output rows: TMEM -> registers -> bias / LeakyReLU /
-//     residual -> shared-memory staging tile -> TMA store (coalesced NHWC writes, also the 2x nearest-upsampled
-//     variant); the fp32 residual tile arrives by TMA load while the row's MMAs are still running.
+//   * Epilogue (conv3x3_common.cuh, shared with the CTA-pair kernel): one to three groups of 4 warps take alternate
+//     output rows: TMEM -> registers -> residual / LeakyReLU -> shared-memory staging tile -> TMA store (coalesced NHWC
+//     writes, also the 2x nearest-upsampled variant). Each thread reads its pixel's residual channels straight into
+//     registers, issued before the wait for the accumulator so that the latency hides behind the row's MMAs.
 //
 // Warp roles: warp 0 lane 0 = TMA producer, warp 1 lane 0 = MMA issuer, warp 2 = TMEM allocator,
-// warps 4-7 (and 8-11) = epilogue groups.
-#include <cuda_bf16.h>
-#include <cuda_fp16.h>
-
-#include <cstdlib>
-#include <cstring>
-
-#include "conv3x3.cuh"
-#include "device_state.h"
-#include "ptx.cuh"
-
-// Kernel perturbation flags for bottleneck experiments (tools/power_probe.py); compiled out of the product build.
-#ifdef RESR_EXPERIMENTS
-#define DBGF(x) ((a.dbg_flags & (x)) != 0)
-#else
-#define DBGF(x) false
-#endif
+// warps 4-7 (8-11, 12-15) = epilogue groups.
+#include "conv3x3_common.cuh"
 
 namespace resr {
 
-static constexpr int kStageBytes = 17408;  // 136 rows x 128 B (mode 0 uses 130 rows, mode 1 uses 128)
-static constexpr int kMaxStages = 12;
 static constexpr int kSlots = 16;          // TMEM accumulator ring
-static constexpr int kMiscBytes = 1024;
-static constexpr int kSmemMax = 232448;    // 227 KB opt-in limit per CTA
-static constexpr int kTileFBytes = 16384;  // 128 px x 32 fp32
-
-struct RowRange {   // 32-bit on purpose: 64-bit divisions are ~100-instruction subroutines and every role decodes its strips
-    int g0, g1;     // (the launcher refuses problems with rows_total * grid >= 2^31)
-};
 
 __device__ __forceinline__ RowRange cta_rows(const ConvArgs& a) {
     RowRange r;
@@ -59,25 +36,7 @@ __device__ __forceinline__ RowRange cta_rows(const ConvArgs& a) {
     return r;
 }
 
-__device__ __forceinline__ unsigned long long gtimer() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-    return t;
-}
-#define RESR_DBG(slot) do { if (a.dbg && blockIdx.x == 0 && blockIdx.y == 0 && (threadIdx.x & 31) == 0) a.dbg[slot] = gtimer(); } while (0)
-
 __device__ __forceinline__ uint32_t slot_of(uint32_t v) { return (16u - (v & 15u)) & 15u; }
-
-__host__ __device__ inline int epi_group_bytes(const ConvArgs& a, int nout) {
-    const int f = a.has_outf ? kTileFBytes : 0;  // fp32 output tile (TMA store)
-    const int h = a.has_out16 ? 128 * nout * 2 : 0;
-    return f + (h + 1023) / 1024 * 1024;
-}
-
-
-// K-major, 128B-swizzled operand descriptor: constant high word (SBO = 1024 B, version 1, SWIZZLE_128B) + low word.
-static constexpr uint32_t kDescHi = (1024u >> 4) | (1u << 14) | (2u << 29);
-__device__ __forceinline__ uint64_t desc_of(uint32_t lo) { return (static_cast<uint64_t>(kDescHi) << 32) | lo; }
 
 // All MMAs of one pipeline stage, straight-line. SPLIT: 0 = one N=3*NOUT MMA at d0; 1 / 2 = ring seam (slot 14 / 15),
 // the (dy=0,1 | dy=2) resp. (dy=0 | dy=1,2) column blocks go to d0 and to the start of the ring. NDX: horizontal taps
@@ -127,35 +86,6 @@ __device__ __forceinline__ void issue_half(int ks, uint32_t s0, uint32_t d0, uin
 #undef RESR_HALF
 }
 
-// Re-arm an accumulator slot with the layer's BIAS instead of zero (see conv3x3_pair.cu tmem_init_bias): the MMAs
-// accumulate on top of it and the epilogue needs no bias add.
-template <int W>
-__device__ __forceinline__ void tmem_init_bias_w(uint32_t taddr, const float* __restrict__ bias_w) {
-    float b[W];
-#pragma unroll
-    for (int i = 0; i < W / 4; ++i) {
-        const float4 q = reinterpret_cast<const float4*>(bias_w)[i];
-        b[4 * i] = q.x; b[4 * i + 1] = q.y; b[4 * i + 2] = q.z; b[4 * i + 3] = q.w;
-    }
-    if (W == 32) tmem_st32(taddr, b); else tmem_st16(taddr, b);
-}
-
-// eight 16-bit values (fp16 or bf16) of a uint4 -> fp32
-__device__ __forceinline__ void unpack16x8(const uint4 q, int fmt, float (&f)[8]) {
-    const uint32_t w4[4] = {q.x, q.y, q.z, q.w};
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        if (fmt == 1) {
-            f[2 * i] = __uint_as_float(w4[i] << 16);
-            f[2 * i + 1] = __uint_as_float(w4[i] & 0xFFFF0000u);
-        } else {
-            const float2 h = __half22float2(*reinterpret_cast<const __half2*>(&w4[i]));
-            f[2 * i] = h.x;
-            f[2 * i + 1] = h.y;
-        }
-    }
-}
-
 // The MMA-issuing warp. The tensor core is fed by ONE instruction stream with a shallow queue, so every non-MMA
 // instruction of this warp is tensor-pipe idle time (tools/mma_bench3.cu): the loop keeps 32-bit incremental
 // bookkeeping, probes the NEXT step's barriers (non-blocking test_wait) between the two halves of the current step's
@@ -175,7 +105,6 @@ __device__ __forceinline__ void mma_role(const ConvArgs& a, const RowRange rr, c
     const uint32_t b_step = (MODE == 0 ? 3 : 1) * WT;
     const int nstages = a.nstages;
     const int H = a.H;
-    const bool dbg_quarter = DBGF(4), dbg_nomma = DBGF(16);
     int stage = 0;
     uint32_t phase = 0;
     uint32_t a_lo = s_lo;
@@ -207,9 +136,9 @@ __device__ __forceinline__ void mma_role(const ConvArgs& a, const RowRange rr, c
                 if (!full_ready) mbar_wait_a(full_a + (stage << 3), phase);
                 tc_fence_after();
                 const bool last = (st == nsteps - 1);
-                const int ks = dbg_quarter ? 1 : ((st >= nsteps - (MODE == 0 ? 1 : 3)) ? a.tail_ksteps : 4);  // steps of the last K chunk
+                const int ks = (st >= nsteps - (MODE == 0 ? 1 : 3)) ? a.tail_ksteps : 4;  // steps of the last K chunk
                 if (elect_one()) {
-                    if (!dbg_nomma) issue_half<NOUT, MODE == 0 ? 3 : 1, 0>(ks, s0, d0, tbase, a_lo, b_lo, idesc3, idesc2, idesc1);
+                    issue_half<NOUT, MODE == 0 ? 3 : 1, 0>(ks, s0, d0, tbase, a_lo, b_lo, idesc3, idesc2, idesc1);
                     if (pending_empty >= 0) umma_commit_a(empty_a + (pending_empty << 3));
                 }
                 __syncwarp();
@@ -220,7 +149,7 @@ __device__ __forceinline__ void mma_role(const ConvArgs& a, const RowRange rr, c
                 full_ready = mbar_test_wait_a(full_a + (stage << 3), phase);
                 if (last && r < rb) slot_ready = mbar_test_wait_a(slotfree_a + (((0u - (vnew + 1)) & 15u) << 3), ((vnew + 1) >> 4) & 1u);
                 if (elect_one()) {
-                    if (!dbg_nomma) issue_half<NOUT, MODE == 0 ? 3 : 1, 1>(ks, s0, d0, tbase, a_cur, b_lo, idesc3, idesc2, idesc1);
+                    issue_half<NOUT, MODE == 0 ? 3 : 1, 1>(ks, s0, d0, tbase, a_cur, b_lo, idesc3, idesc2, idesc1);
                     if (last) {
                         umma_commit_a(accfull_a + (((s0 + 2) & 15u) << 3));      // row r-1 has its last contribution
                         if (r == rb) {                                            // strip end: rows rb, rb+1 get no more
@@ -256,7 +185,6 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_consta
     const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);
     const int lane = threadIdx.x & 31;
     const int slice = blockIdx.y;
-    if (threadIdx.x == 0) RESR_DBG(0);  // kernel entry
     const uint32_t wbytes = static_cast<uint32_t>(a.nchunks) * 3u * WTILE;
     const int epi_bytes = epi_group_bytes(a, NOUT);
 
@@ -296,7 +224,6 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_consta
     __syncthreads();
     tc_fence_after();
     const uint32_t tbase = *tmem_ptr;
-    if (threadIdx.x == 0) RESR_DBG(1);  // setup done (barriers, TMEM)
     // Programmatic dependent launch: the next kernel in the stream may take over SMs as soon as CTAs of this grid
     // retire (it parks in griddepcontrol.wait until this whole grid has completed and flushed).
     grid_dep_launch();
@@ -314,7 +241,6 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_consta
         }
         __syncwarp();
         grid_dep_wait();
-        RESR_DBG(2);  // previous grid complete
         int stage = 0;
         uint32_t phase = 0;
         const int ndx = a.mode == 0 ? 1 : 3;
@@ -331,13 +257,8 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_consta
                     for (int dx = 0; dx < ndx; ++dx) {
                         mbar_wait(empty + stage, phase ^ 1);
                         if (elect_one()) {
-                            if (DBGF(32)) {
-                                mbar_arrive(full + stage);
-                            } else {
-                                mbar_expect_tx(full + stage, tx_bytes);
-                                tma_load_4d(stg + stage * kStageBytes, &tmapA, full + stage, c * 64,
-                                            a.mode == 0 ? x0 - 1 : x0 + dx - 1, DBGF(2) ? 0 : r, DBGF(2) ? 0 : n0);
-                            }
+                            mbar_expect_tx(full + stage, tx_bytes);
+                            tma_load_4d(stg + stage * kStageBytes, &tmapA, full + stage, c * 64, a.mode == 0 ? x0 - 1 : x0 + dx - 1, r, n0);
                         }
                         __syncwarp();
                         if (++stage == a.nstages) { stage = 0; phase ^= 1; }
@@ -349,31 +270,24 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_consta
     } else if (warp == 1) {
         // ------------------------------------------------------------------ MMA issuer (whole warp, one elected lane issues)
         mbar_wait(wbar, 0);
-        RESR_DBG(3);  // weights resident
         tc_fence_after();
         if (a.mode == 0) mma_role<NOUT, 0>(a, rr, tbase, smem_u32(wsm), smem_u32(stg), smem_u32(full), smem_u32(empty), smem_u32(acc_full), smem_u32(slot_free));
         else mma_role<NOUT, 1>(a, rr, tbase, smem_u32(wsm), smem_u32(stg), smem_u32(full), smem_u32(empty), smem_u32(acc_full), smem_u32(slot_free));
-        RESR_DBG(5);  // all MMAs issued
     } else if (warp >= 4) {
         // ------------------------------------------------------------------ epilogue groups
         const int gi = (warp - 4) >> 2;
         const int q = warp & 3;        // TMEM lane quadrant this warp may access
         const int m = q * 32 + lane;   // M row == TMEM lane == pixel of the tile
         const bool lead_warp = ((warp - 4) & 3) == 0;  // first warp of the group issues its TMA traffic
-        // per-slice output selection (backward: only the top slice produces the masked 16-bit dY, the others
-        // accumulate into the fp32 gradient buffer)
-        const bool use_res1 = a.has_res1 && !((a.slice_nores_mask >> slice) & 1u);
-        const bool use_outf = a.has_outf && !((a.slice_noutf_mask >> slice) & 1u);
-        const bool use_o16 = a.has_out16 && !((a.slice_no16_mask >> slice) & 1u);
-        const bool staged = use_o16 || use_outf;
-        uint8_t* tileR = epi + gi * epi_bytes;                       // fp32 output tile (TMA store)
-        uint8_t* tile16 = tileR + (a.has_outf ? kTileFBytes : 0);  // 16-bit output tile (TMA store)
+        // per-slice residual selection (backward: slices whose input gradient is not accumulated skip res1)
+        const bool use_res1 = slice_on(a.has_res1, a.slice_nores_mask, slice);
+        EpiGroup grp{epi + gi * epi_bytes, 0, false, 0, gi, m, lead_warp};   // one staging buffer per group
         const uint32_t lane_base = tbase + (static_cast<uint32_t>(q * 32) << 16);
         const int img_in_tile = m / a.BW;
         const int x_in_tile = m % a.BW;
         {   // zero this group's share of the accumulator ring, then hand the slots to the MMA issuer
             const int s_lo = gi * kSlots / a.nepi, s_hi = (gi + 1) * kSlots / a.nepi;
-            for (int s = s_lo; s < s_hi; ++s) tmem_init_bias_w<NOUT>(lane_base + s * NOUT, bias_s);
+            for (int s = s_lo; s < s_hi; ++s) tmem_init_bias<NOUT>(lane_base + s * NOUT, bias_s);
             tmem_st_wait();
             tc_fence_before();
             for (int s = s_lo; s < s_hi; ++s) mbar_arrive(slot_free + s);
@@ -386,278 +300,57 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_consta
             const int yb = min(H, ya + (rr.g1 - g));
             const int n0 = (cg / a.nxs) * a.BN;
             const int x0 = (cg % a.nxs) * a.BW;
-            const int n = n0 + img_in_tile;
-            const int x = x0 + x_in_tile;
-            const bool valid = (n < a.N) && (x < a.W);
             const int ra = max(ya - 1, 0), rb = min(yb, H - 1);
             const int n_acc = rb - ra + 3;
             for (int j = 0; j < n_acc; ++j) {
                 const uint32_t v = v0 + j;
                 if (static_cast<int>(v % static_cast<uint32_t>(a.nepi)) != gi) continue;
                 const int y = ra - 1 + j;
-                const bool emit = (y >= ya) && (y < yb) && !DBGF(8);
+                const bool emit = (y >= ya) && (y < yb);
                 const uint32_t slot = slot_of(v);
-                float4 resv[NOUT / 4];   // fp32 residual, or (res16) NOUT 16-bit values in the first NOUT / 8 entries
-                if (emit && use_res1) {
-                    // this row's residual: contiguous bytes per thread, requested before the wait for the accumulator so
-                    // the latency hides behind the row's MMAs
-                    const size_t pix = (static_cast<size_t>(valid ? n : 0) * a.H + y) * a.W + (valid ? x : 0);
-                    if (a.res16) {
-                        const uint4* rp = reinterpret_cast<const uint4*>(static_cast<const uint16_t*>(a.res1) + pix * a.res1_cstride +
-                                                                         a.res_choff + slice * NOUT);
-#pragma unroll
-                        for (int i = 0; i < NOUT / 8; ++i) {
-                            const uint4 q4 = rp[i];
-                            resv[i] = make_float4(__uint_as_float(q4.x), __uint_as_float(q4.y), __uint_as_float(q4.z), __uint_as_float(q4.w));
-                        }
-                    } else {
-                        const float4* rp = reinterpret_cast<const float4*>(static_cast<const float*>(a.res1) + pix * a.res1_cstride +
-                                                                           a.res_choff + slice * NOUT);
-#pragma unroll
-                        for (int i = 0; i < NOUT / 4; ++i) resv[i] = rp[i];
-                    }
-                }
-                bool inside = true;   // canvas pixel of an image (vmask), read before the accumulator wait like the residual
-                if (MASKED && emit) {
-                    const int lx = (valid ? x : 0) >> a.vmask_shift, ly = y >> a.vmask_shift;
-                    inside = (__ldg(a.vmask + static_cast<size_t>(ly) * a.vmask_words + (lx >> 5)) >> (lx & 31)) & 1u;
-                }
+                const EpiPixel px = epi_pixel<MASKED>(a, n0, x0, n0 + img_in_tile, x0 + x_in_tile, y, emit);
+                float4 resv[NOUT / 4];
+                if (emit && use_res1) epi_load_res1<NOUT>(a, px.pix, slice, resv);
                 mbar_wait(acc_full + slot, static_cast<uint32_t>(v >> 4) & 1);
                 tc_fence_after();
                 float val[NOUT];
-                if (NOUT == 32) tmem_ld32(lane_base + slot * NOUT, val); else tmem_ld16(lane_base + slot * NOUT, val);
+                tmem_ld_w<NOUT>(lane_base + slot * NOUT, val);
                 tmem_ld_wait();
-                tmem_init_bias_w<NOUT>(lane_base + slot * NOUT, bias_s);
+                tmem_init_bias<NOUT>(lane_base + slot * NOUT, bias_s);
                 tmem_st_wait();
                 tc_fence_before();
                 mbar_arrive(slot_free + slot);
-                if (!emit) continue;
-
-                // (no bias add here: the accumulator was armed with the bias)
-                if (use_res1 && a.res16) {  // widen the 16-bit residual in place (consumed below as fp32)
-                    float wide[NOUT];
-#pragma unroll
-                    for (int i = 0; i < NOUT / 8; ++i) {
-                        float f8[8];
-                        unpack16x8(make_uint4(__float_as_uint(resv[i].x), __float_as_uint(resv[i].y), __float_as_uint(resv[i].z),
-                                              __float_as_uint(resv[i].w)), a.res16_fmt, f8);
-#pragma unroll
-                        for (int e = 0; e < 8; ++e) wide[8 * i + e] = f8[e];
-                    }
-#pragma unroll
-                    for (int i = 0; i < NOUT / 4; ++i) resv[i] = make_float4(wide[4 * i], wide[4 * i + 1], wide[4 * i + 2], wide[4 * i + 3]);
-                }
-                if (use_res1) {
-#pragma unroll
-                    for (int i = 0; i < NOUT / 4; ++i) {
-                        const float4 r4 = resv[i];
-                        if (a.ep_mode == EP_SKIP || a.ep_mode == EP_ADD2) {
-                            val[4 * i + 0] = __fadd_rn(r4.x, val[4 * i + 0]);
-                            val[4 * i + 1] = __fadd_rn(r4.y, val[4 * i + 1]);
-                            val[4 * i + 2] = __fadd_rn(r4.z, val[4 * i + 2]);
-                            val[4 * i + 3] = __fadd_rn(r4.w, val[4 * i + 3]);
-                        } else {
-                            val[4 * i + 0] = __fadd_rn(__fmul_rn(val[4 * i + 0], 0.2f), r4.x);
-                            val[4 * i + 1] = __fadd_rn(__fmul_rn(val[4 * i + 1], 0.2f), r4.y);
-                            val[4 * i + 2] = __fadd_rn(__fmul_rn(val[4 * i + 2], 0.2f), r4.z);
-                            val[4 * i + 3] = __fadd_rn(__fmul_rn(val[4 * i + 3], 0.2f), r4.w);
-                        }
-                    }
-                }
-                if (staged) {  // the output tiles are free once the previous row's TMA stores have read them
-                    if (lead_warp) tma_store_wait_read();
-                    named_bar_sync(1 + gi, 128);
-                }
-                if (a.ep_mode == EP_RRDB) {
-                    const size_t pix = (static_cast<size_t>(valid ? n : 0) * a.H + y) * a.W + (valid ? x : 0);
-                    if (a.res16) {
-                        // plain (coherent) loads: in the inference trunk res2 is the RRDB input held in the very buffer
-                        // this launch overwrites -- each element is read by the thread that later stores its replacement
-                        const uint4* r2 = reinterpret_cast<const uint4*>(static_cast<const uint16_t*>(a.res2) + pix * a.res2_cstride +
-                                                                         a.res_choff + slice * NOUT);
-#pragma unroll
-                        for (int i = 0; i < NOUT / 8; ++i) {
-                            float f8[8];
-                            unpack16x8(r2[i], a.res16_fmt, f8);
-#pragma unroll
-                            for (int e = 0; e < 8; ++e) val[8 * i + e] = __fadd_rn(__fmul_rn(val[8 * i + e], 0.2f), f8[e]);
-                        }
-                    } else {
-                        const float4* r2 = reinterpret_cast<const float4*>(static_cast<const float*>(a.res2) + pix * a.res2_cstride +
-                                                                           a.res_choff + slice * NOUT);
-#pragma unroll
-                        for (int i = 0; i < NOUT / 4; ++i) {
-                            const float4 r4 = __ldg(r2 + i);
-                            val[4 * i + 0] = __fadd_rn(__fmul_rn(val[4 * i + 0], 0.2f), r4.x);
-                            val[4 * i + 1] = __fadd_rn(__fmul_rn(val[4 * i + 1], 0.2f), r4.y);
-                            val[4 * i + 2] = __fadd_rn(__fmul_rn(val[4 * i + 2], 0.2f), r4.z);
-                            val[4 * i + 3] = __fadd_rn(__fmul_rn(val[4 * i + 3], 0.2f), r4.w);
-                        }
-                    }
-                }
-                if (a.ep_mode == EP_ADD2 && a.res2) {
-                    const size_t pix = (static_cast<size_t>(valid ? n : 0) * a.H + y) * a.W + (valid ? x : 0);
-                    const float4* r2 = reinterpret_cast<const float4*>(static_cast<const float*>(a.res2) + pix * a.res2_cstride + a.res_choff + slice * NOUT);
-#pragma unroll
-                    for (int i = 0; i < NOUT / 4; ++i) {
-                        const float4 r4 = __ldg(r2 + i);
-                        val[4 * i + 0] = fmaf(a.res2_scale, r4.x, val[4 * i + 0]);
-                        val[4 * i + 1] = fmaf(a.res2_scale, r4.y, val[4 * i + 1]);
-                        val[4 * i + 2] = fmaf(a.res2_scale, r4.z, val[4 * i + 2]);
-                        val[4 * i + 3] = fmaf(a.res2_scale, r4.w, val[4 * i + 3]);
-                    }
-                }
-                if (a.lrelu) {   // max(v, 0.2 v) == (v > 0 ? v : 0.2 v); the product is one packed FMUL2 per pair
-#pragma unroll
-                    for (int i = 0; i < NOUT / 2; ++i) {
-                        const float2 t = __fmul2_rn(make_float2(val[2 * i], val[2 * i + 1]), make_float2(0.2f, 0.2f));
-                        val[2 * i] = fmaxf(val[2 * i], t.x);
-                        val[2 * i + 1] = fmaxf(val[2 * i + 1], t.y);
-                    }
-                }
-                if (MASKED && !inside) {   // gutter / canvas margin: 0 in every output, as the zero padding around an image
-#pragma unroll
-                    for (int i = 0; i < NOUT; ++i) val[i] = 0.f;
-                }
-                if (a.out_nchw_raw && valid) {
-                    const size_t plane = static_cast<size_t>(a.H) * a.W;
-                    float* o = a.out_nchw_raw + static_cast<size_t>(n) * a.out_nchw_c * plane + static_cast<size_t>(y) * a.W + x;
-#pragma unroll
-                    for (int c = 0; c < NOUT; ++c) {
-                        const int cc = slice * NOUT + c;
-                        if (cc < a.out_nchw_c) o[static_cast<size_t>(cc) * plane] = val[c];
-                    }
-                }
-                if (a.clamp01) {
-#pragma unroll
-                    for (int i = 0; i < NOUT; ++i) val[i] = fminf(fmaxf(val[i], 0.f), 1.f);
-                }
-                if (use_outf) {  // fp32 master
-#pragma unroll
-                    for (int i = 0; i < NOUT / 4; ++i)
-                        *reinterpret_cast<float4*>(tileR + m * 128 + ((i ^ (m & 7)) << 4)) =
-                            make_float4(val[4 * i], val[4 * i + 1], val[4 * i + 2], val[4 * i + 3]);
-                }
-                if (use_o16 && a.mask16) {  // LeakyReLU backward: slope 1 where the saved activation is > 0, else 0.2
-                    const size_t pix = (static_cast<size_t>(valid ? n : 0) * a.H + y) * a.W + (valid ? x : 0);
-                    const uint4* mk = reinterpret_cast<const uint4*>(static_cast<const uint16_t*>(a.mask16) + pix * a.mask16_cstride +
-                                                                     a.mask16_choff + slice * NOUT);
-#pragma unroll
-                    for (int i = 0; i < NOUT / 8; ++i) {
-                        const uint4 q4 = __ldg(mk + i);
-                        const uint32_t w4[4] = {q4.x, q4.y, q4.z, q4.w};
-#pragma unroll
-                        for (int e = 0; e < 8; ++e) {
-                            const uint32_t h16 = (w4[e >> 1] >> ((e & 1) * 16)) & 0xFFFFu;
-                            const bool pos = ((h16 & 0x8000u) == 0) && ((h16 & 0x7FFFu) != 0);
-                            if (!pos) val[8 * i + e] = __fmul_rn(val[8 * i + e], 0.2f);
-                        }
-                    }
-                }
-                if (use_o16 && a.out16_scale != 0.f) {
-#pragma unroll
-                    for (int i = 0; i < NOUT; ++i) val[i] = __fmul_rn(val[i], a.out16_scale);
-                }
-                if (use_o16) {
-                    uint32_t pk[NOUT / 2];
-#pragma unroll
-                    for (int i = 0; i < NOUT / 2; ++i) {
-                        if (a.out16_fmt == 1) {
-                            __nv_bfloat162 h = __floats2bfloat162_rn(val[2 * i], val[2 * i + 1]);
-                            pk[i] = *reinterpret_cast<uint32_t*>(&h);
-                        } else {
-
-                            pk[i] = pack_f16x2_sat(val[2 * i], val[2 * i + 1]);  // saturate, never inf
-                        }
-                    }
-                    // rotate the 16-byte chunk order per lane so that a quarter-warp does not hammer two bank groups
-                    uint4* dst = reinterpret_cast<uint4*>(tile16 + m * (NOUT * 2));
-#pragma unroll
-                    for (int i = 0; i < NOUT / 8; ++i) dst[i] = make_uint4(pk[4 * i], pk[4 * i + 1], pk[4 * i + 2], pk[4 * i + 3]);
-                }
-                if (staged) {
-                    fence_proxy_async_smem();
-                    named_bar_sync(1 + gi, 128);
-                    if (lead_warp) {
-                      if (elect_one()) {
-                        if (use_outf && !DBGF(1) && !DBGF(64)) tma_store_4d(&tmapOF, tileR, a.outf_choff + slice * NOUT, x0, y, n0);
-                        if (use_o16 && !DBGF(1) && !(DBGF(128) && a.has_res1)) {
-                            const int c0 = a.out16_choff + (a.out16_slice_fixed ? 0 : slice * NOUT);
-                            if (!a.out16_up2) {
-                                tma_store_4d(&tmapO16, tile16, c0, x0, y, n0);
-                            } else {
-#pragma unroll
-                                for (int s = 0; s < 4; ++s) tma_store_5d(&tmapO16, tile16, c0, s & 1, x0, 2 * y + (s >> 1), n0);
-                            }
-                        }
-                        tma_store_commit();
-                      }
-                      __syncwarp();
-                    }
-                }
-                if (a.out_nchw && valid) {
-                    const size_t plane = static_cast<size_t>(a.H) * a.W;
-                    float* o = a.out_nchw + static_cast<size_t>(n) * a.out_nchw_c * plane + static_cast<size_t>(y) * a.W + x;
-#pragma unroll
-                    for (int c = 0; c < NOUT; ++c) {
-                        const int cc = slice * NOUT + c;
-                        if (cc < a.out_nchw_c) o[static_cast<size_t>(cc) * plane] = val[c];
-                    }
-                }
-                if (a.out_u8 && valid) {   // clamp01 has been applied: v * 255 lies in [0, 255], the cast truncates
-                    unsigned char* o = a.out_u8 + ((static_cast<size_t>(n) * a.H + y) * a.W + x) * a.out_nchw_c;
-#pragma unroll
-                    for (int c = 0; c < NOUT; ++c) {
-                        const int cc = slice * NOUT + c;
-                        if (cc < a.out_nchw_c) o[cc] = static_cast<unsigned char>(fminf(fmaxf(__fmul_rn(val[c], 255.f), 0.f), 255.f));
-                    }
-                }
+                if (emit) epi_pass<NOUT, MASKED>(a, &tmapO16, &tmapOF, grp, px, slice, val, resv);
             }
             v0 += n_acc;
             g += yb - ya;
         }
         if (lead_warp) tma_store_wait_all();
-        if (gi == 0 && lead_warp) RESR_DBG(6);  // epilogue group 0 drained
     }
 
     tc_fence_before();
     __syncthreads();
-    if (threadIdx.x == 0) RESR_DBG(7);  // CTA done
     if (warp == 2) tmem_dealloc(tbase, 512);
 }
 
 // --------------------------------------------------------------------------------------------- host side
 
-bool conv3x3_plan_smem(ConvArgs* a, int cout_slice) {
-    const int wbytes = a->nchunks * 3 * (3 * cout_slice) * 128;
-    // The per-row epilogue latency (TMEM drain, staging, TMA store; ~1.6k cycles, more with an fp32 output tile) is hidden
-    // by running several epilogue groups on consecutive rows. Three groups whenever they fit beside at least four
-    // stages (8 KB of shared memory each without an fp32 tile); two with the 24 KB fp32 variant.
-    int nepi = a->has_outf ? 2 : 3;
-    const char* env = getenv("RESR_CONV_NEPI");
-    if (env) nepi = atoi(env);
-    if (nepi < 1) nepi = 1;
-    if (nepi > 3) nepi = 3;
-    for (;; --nepi) {
-        a->nepi = nepi;
-        const int fixed = 1024 + wbytes + nepi * epi_group_bytes(*a, cout_slice) + kMiscBytes;
-        int ns = (kSmemMax - fixed) / kStageBytes;
-        if (ns > kMaxStages) ns = kMaxStages;
-        if (ns >= 4 || nepi == 1) {
-            a->nstages = ns;
-            return ns >= 2;
-        }
-    }
-}
-
-void conv3x3_pick_tile(int W, int* BW, int* BN) {
-    if (W == 64 || W == 32 || W == 16 || W == 8) {
-        *BW = W;
-        *BN = 128 / W;
+void conv3x3_init_geometry(ConvArgs* a, int N, int H, int W, int cin, int mode) {
+    a->N = N; a->H = H; a->W = W;
+    if (W == 64 || W == 32 || W == 16 || W == 8) {   // BN images of W columns share one 128-lane tile
+        a->BW = W;
+        a->BN = 128 / W;
     } else {
-        *BW = 128;
-        *BN = 1;
+        a->BW = 128;
+        a->BN = 1;
     }
+    a->mode = a->BN != 1 ? 1 : (mode >= 0 ? mode : 0);   // lanes that span images need one load per dx
+    a->nxs = (W + a->BW - 1) / a->BW;
+    a->ncg = ((N + a->BN - 1) / a->BN) * a->nxs;
+    a->rows_total = static_cast<long long>(a->ncg) * H;
+    // K16 steps of the last 64-channel chunk that hold real input channels; the zero-weight rest is not issued
+    const int r = cin % 64;
+    a->tail_ksteps = r == 0 || r > 32 ? 4 : (r > 16 ? 2 : 1);
 }
 
 typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -692,13 +385,8 @@ int conv3x3_make_tmap_act(CUtensorMap* out, const void* base, int N, int H, int 
     const cuuint32_t estr[4] = {1, 1, 1, 1};
     // L2 promotion: 128 B fetches suit full 64-channel chunks (128 B per pixel); a layer whose last chunk holds only 32
     // channels (Cin = 96 / 160) would drag the other half of every 128-byte line in from DRAM (ncu: 278 MB read for the
-    // 201 MB a 96-channel layer needs), so those maps promote to 64 B. RESR_TMAP_PROMO = 0 / 1 / 2 / 3 forces none / 64 / 128 / 256.
-    static const int env_promo = getenv("RESR_TMAP_PROMO") ? atoi(getenv("RESR_TMAP_PROMO")) : -1;
-    CUtensorMapL2promotion promo = (cdim % 64 != 0) ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B : CU_TENSOR_MAP_L2_PROMOTION_L2_128B;
-    if (env_promo == 0) promo = CU_TENSOR_MAP_L2_PROMOTION_NONE;
-    else if (env_promo == 1) promo = CU_TENSOR_MAP_L2_PROMOTION_L2_64B;
-    else if (env_promo == 2) promo = CU_TENSOR_MAP_L2_PROMOTION_L2_128B;
-    else if (env_promo == 3) promo = CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
+    // 201 MB a 96-channel layer needs), so those maps promote to 64 B.
+    const CUtensorMapL2promotion promo = (cdim % 64 != 0) ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B : CU_TENSOR_MAP_L2_PROMOTION_L2_128B;
     const CUresult r = enc(out, CU_TENSOR_MAP_DATA_TYPE_UINT16, 4, const_cast<void*>(base), dims, strides, box, estr,
                            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, promo, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     return r == CUDA_SUCCESS ? 0 : static_cast<int>(r);
@@ -748,59 +436,16 @@ int conv3x3_make_tmap_f32(CUtensorMap* out, const void* base, int N, int H, int 
     return r == CUDA_SUCCESS ? 0 : static_cast<int>(r);
 }
 
-template <int NOUT, bool MASKED>
-static cudaError_t launch_t(const ConvMaps& maps, const ConvArgs& args, dim3 grid, int threads, cudaStream_t stream) {
-    static PerDevice<bool> attr;  // function attributes are per device
-    if (!attr.cur()) {
-        const cudaError_t e = cudaFuncSetAttribute(conv3x3_tc_kernel<NOUT, MASKED>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax);
-        if (e != cudaSuccess) return e;
-        attr.cur() = true;
-    }
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = grid;
-    cfg.blockDim = dim3(threads, 1, 1);
-    cfg.dynamicSmemBytes = kSmemMax;  // always the full 227 KB: exactly one CTA (one 512-column TMEM allocation) per SM
-    cfg.stream = stream;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, conv3x3_tc_kernel<NOUT, MASKED>, maps.a, maps.o16, maps.of, args);
-}
-
-cudaError_t conv3x3_launch(const ConvMaps& maps, const ConvArgs& args, int cout_slice, int nslices, int num_sms,
-                           cudaStream_t stream) {
-    const int wbytes = args.nchunks * 3 * (3 * cout_slice) * 128;
-    const int smem = 1024 + wbytes + args.nstages * kStageBytes + args.nepi * epi_group_bytes(args, cout_slice) + kMiscBytes;
-    if (args.nstages < 2 || args.nepi < 1 || args.nepi > 3 || smem > kSmemMax) return cudaErrorInvalidConfiguration;
-    long long gx = num_sms / nslices;
-    const long long min_rows = 4;  // do not shred tiny problems into 1-row strips (2 halo rows each)
-    const long long cap = (args.rows_total + min_rows - 1) / min_rows;
-    if (gx > cap) gx = cap;
-    if (gx < 1) gx = 1;
-    if (args.rows_total * (gx + 1) >= (1ll << 31)) return cudaErrorInvalidValue;   // the kernel's strip arithmetic is 32-bit
-    const dim3 grid(static_cast<unsigned>(gx), static_cast<unsigned>(nslices), 1);
-    const int threads = 128 + 128 * args.nepi;
-    static const int env_flags = getenv("RESR_CONV_DBGFLAGS") ? atoi(getenv("RESR_CONV_DBGFLAGS")) : 0;  // experiments only
-    if (env_flags && !(args.dbg_flags & 0x40000000)) {
-        ConvArgs fixed = args;
-        fixed.dbg_flags |= env_flags | 0x40000000;
-        return conv3x3_launch(maps, fixed, cout_slice, nslices, num_sms, stream);
-    }
-    if (args.tail_ksteps != 1 && args.tail_ksteps != 2 && args.tail_ksteps != 4) {
-        ConvArgs fixed = args;
-        fixed.tail_ksteps = 4;
-        return conv3x3_launch(maps, fixed, cout_slice, nslices, num_sms, stream);
-    }
+cudaError_t conv3x3_tc_launch(const ConvMaps& maps, const ConvArgs& args, int nout, int nslices, int num_sms,
+                              cudaStream_t stream) {
+    const long long units = args.rows_total;
     if (args.vmask) {
-        if (cout_slice == 32) return launch_t<32, true>(maps, args, grid, threads, stream);
-        if (cout_slice == 16) return launch_t<16, true>(maps, args, grid, threads, stream);
+        if (nout == 32) return conv3x3_launch_grid<conv3x3_tc_kernel<32, true>>(maps, args, 32, 1, units, nslices, num_sms, stream);
+        if (nout == 16) return conv3x3_launch_grid<conv3x3_tc_kernel<16, true>>(maps, args, 16, 1, units, nslices, num_sms, stream);
         return cudaErrorInvalidValue;
     }
-    if (cout_slice == 32) return launch_t<32, false>(maps, args, grid, threads, stream);
-    if (cout_slice == 16) return launch_t<16, false>(maps, args, grid, threads, stream);
+    if (nout == 32) return conv3x3_launch_grid<conv3x3_tc_kernel<32, false>>(maps, args, 32, 1, units, nslices, num_sms, stream);
+    if (nout == 16) return conv3x3_launch_grid<conv3x3_tc_kernel<16, false>>(maps, args, 16, 1, units, nslices, num_sms, stream);
     return cudaErrorInvalidValue;
 }
 

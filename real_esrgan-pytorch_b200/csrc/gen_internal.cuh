@@ -128,7 +128,6 @@ struct resr_generator {
     float* bias = nullptr;
     bool loaded = false;
     int num_sms = 148;
-    int force_mode = -1;
     int precision = 0;            // inference recipe: 0 = fp16 operands / fp16 residual stream, 1 = bf16 operands + fp32 residual masters
     resr::Plan plan;
     std::vector<resr::Plan> canvas_plans;  // packed-canvas plans of resr_generator_forward_many, oldest first (a few shapes)

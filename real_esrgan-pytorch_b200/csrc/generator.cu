@@ -457,15 +457,6 @@ static int build_plan(resr_generator* g, Plan& p, int N, int H, int W, void* ws,
     uint16_t* t4 = reinterpret_cast<uint16_t*>(base + L.t4);
     p.xin = xin;
 
-    struct Geo { int H, W, BW, BN, mode; };
-    Geo geo[3];
-    for (int s = 0; s < 3; ++s) {
-        geo[s].H = H << s;
-        geo[s].W = W << s;
-        conv3x3_pick_tile(geo[s].W, &geo[s].BW, &geo[s].BN);
-        geo[s].mode = geo[s].BN == 1 ? 0 : 1;
-        if (g->force_mode >= 0) geo[s].mode = (geo[s].BN == 1) ? g->force_mode : 1;
-    }
     // (one-time hygiene: no layer reads a channel that has not been written, the activation tensor maps end at Cin).
     // Issued on the CALLER's stream: ordered after whatever forward is still in flight on this workspace and capturable
     // into a CUDA graph (the legacy default stream is neither).
@@ -476,33 +467,28 @@ static int build_plan(resr_generator* g, Plan& p, int N, int H, int W, void* ws,
     // in16: source activations [N, H<<s, W<<s, cin_total]
     auto make_step = [&](int conv, int s, const void* in16, int cin_total) {
         const ConvSpec& cs = T.c[conv];
-        const Geo& q = geo[s];
         Step st;
         memset(&st, 0, sizeof(st));
         st.conv = conv;
         ConvArgs& a = st.a;
-        a.N = N; a.H = q.H; a.W = q.W; a.BW = q.BW; a.BN = q.BN;
-        a.nxs = (q.W + q.BW - 1) / q.BW;
-        a.ncg = ((N + q.BN - 1) / q.BN) * a.nxs;
+        conv3x3_init_geometry(&a, N, H << s, W << s, cs.cin, -1);
         a.nchunks = cs.nchunks;
-        a.tail_ksteps = conv3x3_tail_ksteps(cs.cin);
-        a.mode = q.mode;
         a.fmt_in = prec == 1 ? 1 : cs.fmt;
-        a.rows_total = static_cast<long long>(a.ncg) * q.H;
         a.wpack = g->wpack + cs.w_off;
         a.bias = g->bias + cs.b_off;
         if (vmask) { a.vmask = vmask; a.vmask_words = W / 32; a.vmask_shift = s; }
-        map_rc |= conv3x3_make_tmap_act(&st.maps.a, in16, N, q.H, q.W, cin_total, q.mode, q.BW, q.BN, cs.cin);
+        map_rc |= conv3x3_make_tmap_act(&st.maps.a, in16, N, a.H, a.W, cin_total, a.mode, a.BW, a.BN, cs.cin);
         return st;
     };
-    auto set_out16 = [&](Step& st, int s, void* dst, int c_total, int choff, int fmt, int up2) {
-        const Geo& q = geo[s];
+    auto set_out16 = [&](Step& st, void* dst, int c_total, int choff, int fmt, int up2) {
+        const ConvArgs& a = st.a;
         st.a.has_out16 = 1; st.a.out16_fmt = prec == 1 ? 1 : fmt; st.a.out16_choff = choff; st.a.out16_up2 = up2;
-        map_rc |= conv3x3_make_tmap_out16(&st.maps.o16, dst, N, q.H, q.W, c_total, T.c[st.conv].nout, q.BW, q.BN, up2);
+        map_rc |= conv3x3_make_tmap_out16(&st.maps.o16, dst, N, a.H, a.W, c_total, T.c[st.conv].nout, a.BW, a.BN, up2);
     };
     auto set_outf = [&](Step& st, float* dst) {
+        const ConvArgs& a = st.a;
         st.a.has_outf = 1; st.a.outf_choff = 0; st.a.outf = static_cast<float*>(dst); st.a.outf_cstride = 64;
-        map_rc |= conv3x3_make_tmap_f32(&st.maps.of, dst, N, geo[0].H, geo[0].W, 64, geo[0].BW, geo[0].BN);
+        map_rc |= conv3x3_make_tmap_f32(&st.maps.of, dst, N, a.H, a.W, 64, a.BW, a.BN);
     };
     auto set_res1 = [&](Step& st, const float* src) {
         st.a.has_res1 = 1; st.a.res_choff = 0; st.a.res1 = src; st.a.res1_cstride = 64;
@@ -511,8 +497,7 @@ static int build_plan(resr_generator* g, Plan& p, int N, int H, int W, void* ws,
         if (!conv3x3_choose(&st.a, T.c[st.conv].nout, T.c[st.conv].nslices, &st.cfg)) map_rc |= 1 << 20;
         // serpentine order: every other pair-kernel launch walks its rows / column groups back to front, so that it starts
         // on what the previous layer touched last (L2-resident) instead of on what it touched first (long evicted)
-        static const int serp = getenv("RESR_CONV_SERPENTINE") ? atoi(getenv("RESR_CONV_SERPENTINE")) : 1;
-        st.a.reverse = (serp && st.cfg.pair) ? static_cast<int>(p.steps.size() & 1) : 0;
+        st.a.reverse = st.cfg.pair ? static_cast<int>(p.steps.size() & 1) : 0;
         p.steps.push_back(st);
     };
 
@@ -526,7 +511,7 @@ static int build_plan(resr_generator* g, Plan& p, int N, int H, int W, void* ws,
         Step st = make_step(conv, 0, xin, 64);
         st.a.ep_mode = EP_PLAIN;
         set_outf(st, F0);
-        set_out16(st, 0, cbuf[0], 192, 0, 0, 0);
+        set_out16(st, cbuf[0], 192, 0, 0, 0);
         push(st);
         ++conv;
     }
@@ -536,7 +521,7 @@ static int build_plan(resr_generator* g, Plan& p, int N, int H, int W, void* ws,
             for (int k = 0; k < 4; ++k) {  // model.py:90-93
                 Step st = make_step(conv, 0, cin_buf, 192);
                 st.a.ep_mode = EP_PLAIN; st.a.lrelu = 1;
-                set_out16(st, 0, cin_buf, 192, 64 + 32 * k, 0, 0);
+                set_out16(st, cin_buf, 192, 64 + 32 * k, 0, 0);
                 push(st);
                 ++conv;
             }
@@ -554,7 +539,7 @@ static int build_plan(resr_generator* g, Plan& p, int N, int H, int W, void* ws,
                 set_res16(st, cin_buf);
                 if (j == 2) { st.a.res2 = cbuf[0]; st.a.res2_cstride = 192; }
             }
-            set_out16(st, 0, cbuf[(j + 1) % 3], 192, 0, 0, 0);
+            set_out16(st, cbuf[(j + 1) % 3], 192, 0, 0, 0);
             push(st);
             ++conv;
         }
@@ -563,28 +548,28 @@ static int build_plan(resr_generator* g, Plan& p, int N, int H, int W, void* ws,
         Step st = make_step(conv, 0, cbuf[0], 192);
         st.a.ep_mode = EP_SKIP;
         set_res1(st, F0);
-        set_out16(st, 0, t1, 64, 0, 0, 1);
+        set_out16(st, t1, 64, 0, 0, 1);
         push(st);
         ++conv;
     }
     {   // upsampling1 conv + LeakyReLU (model.py:264), output written upsampled x2 again (model.py:265)
         Step st = make_step(conv, 1, t1, 64);
         st.a.lrelu = 1;
-        set_out16(st, 1, t2, 64, 0, 0, 1);
+        set_out16(st, t2, 64, 0, 0, 1);
         push(st);
         ++conv;
     }
     {   // upsampling2 conv + LeakyReLU (model.py:265)
         Step st = make_step(conv, 2, t2, 64);
         st.a.lrelu = 1;
-        set_out16(st, 2, t3, 64, 0, 0, 0);
+        set_out16(st, t3, 64, 0, 0, 0);
         push(st);
         ++conv;
     }
     {   // conv3 + LeakyReLU (model.py:267)
         Step st = make_step(conv, 2, t3, 64);
         st.a.lrelu = 1;
-        set_out16(st, 2, t4, 64, 0, 0, 0);
+        set_out16(st, t4, 64, 0, 0, 0);
         push(st);
         ++conv;
     }
@@ -615,11 +600,6 @@ int resr_generator_launches_per_forward(void) { return 1 + kNumConvs; }
 
 int resr_set_conv_pair_policy(int policy) { return conv3x3_set_pair_policy(policy); }
 
-int resr_debug_wait_profile(unsigned long long* out16_host, int reset) {
-    if (conv3x3_wait_profile(out16_host, reset) != 0) return set_error(RESR_E_CUDA, "wait profile copy failed");
-    return RESR_OK;
-}
-
 int resr_generator_tensor_span(int index, size_t* offset, size_t* count) {
     if (index < 0 || index >= 2 * kNumConvs || !offset || !count) return set_error(RESR_E_INVALID, "bad tensor index");
     const ConvSpec& c = table().c[index / 2];
@@ -641,10 +621,6 @@ int resr_generator_create(resr_generator_t** out, int in_channels, int out_chann
     if (prop.major != 10) return set_error(RESR_E_CUDA, "libresr needs an sm_100a device (found sm_%d%d)", prop.major, prop.minor);
     resr_generator* g = new resr_generator();
     g->num_sms = prop.multiProcessorCount;
-    if (getenv("RESR_NUM_SMS") && atoi(getenv("RESR_NUM_SMS")) > 0 && atoi(getenv("RESR_NUM_SMS")) < g->num_sms)
-        g->num_sms = atoi(getenv("RESR_NUM_SMS"));   // experiment knob: grids sized for a subset of the SMs (concurrent chains)
-    const char* fm = getenv("RESR_CONV_MODE");
-    if (fm) g->force_mode = atoi(fm);
     if (cudaMalloc(&g->wpack, table().pack_bytes) != cudaSuccess || cudaMalloc(&g->bias, table().bias_floats * 4) != cudaSuccess) {
         delete g;
         return set_error(RESR_E_CUDA, "cudaMalloc of packed weights failed");
@@ -1012,16 +988,9 @@ int resr_conv3x3(const resr_conv_desc* d, void* stream) {
     ConvMaps maps;
     memset(&a, 0, sizeof(a));
     memset(&maps, 0, sizeof(maps));
-    a.N = d->n; a.H = d->h; a.W = d->w;
-    conv3x3_pick_tile(d->w, &a.BW, &a.BN);
-    a.mode = d->mode >= 0 ? d->mode : (a.BN == 1 ? 0 : 1);
-    if (a.BN != 1) a.mode = 1;
-    a.nxs = (d->w + a.BW - 1) / a.BW;
-    a.ncg = ((d->n + a.BN - 1) / a.BN) * a.nxs;
+    conv3x3_init_geometry(&a, d->n, d->h, d->w, d->cin, d->mode);
     a.nchunks = nchunks;
-    a.tail_ksteps = conv3x3_tail_ksteps(d->cin);
     a.fmt_in = d->fmt_in;
-    a.rows_total = static_cast<long long>(a.ncg) * d->h;
     a.wpack = wp; a.bias = bp;
     a.ep_mode = d->ep_mode; a.lrelu = d->lrelu; a.clamp01 = d->clamp01;
     int rc = conv3x3_make_tmap_act(&maps.a, d->in16, d->n, d->h, d->w, d->c_total, a.mode, a.BW, a.BN, d->cin);
@@ -1039,8 +1008,6 @@ int resr_conv3x3(const resr_conv_desc* d, void* stream) {
     }
     a.res2 = d->res2; a.res2_cstride = d->res_cstride;
     a.out_nchw = d->out_nchw; a.out_nchw_c = d->out_nchw_c;
-    a.dbg = d->dbg;
-    a.dbg_flags = d->dbg_flags;
     ConvLaunchCfg cfg;
     if (!conv3x3_choose(&a, nout, nslices, &cfg)) rc |= 1 << 20;
     if (nout == 16 && (d->out16 || d->outf || d->res1)) rc |= 1 << 21;  // the 16-wide slice only feeds the NCHW output

@@ -197,16 +197,7 @@ static int egrid(size_t total) {
 
 // ================================================================================================ conv launcher
 
-struct Geo { int H, W, BW, BN, mode; };
-
-static Geo make_geo(const resr_generator* g, int H, int W) {
-    Geo q;
-    q.H = H; q.W = W;
-    conv3x3_pick_tile(W, &q.BW, &q.BN);
-    q.mode = q.BN == 1 ? 0 : 1;
-    if (g->force_mode >= 0 && q.BN == 1) q.mode = g->force_mode;
-    return q;
-}
+struct Geo { int H, W; };  // resolution of one convolution
 
 struct ConvIO {
     const void* in16 = nullptr; int in_c = 64;
@@ -228,26 +219,21 @@ static int launch_conv_io(const resr_generator* g, const Geo& q, int N, const Co
     ConvMaps m;
     memset(&a, 0, sizeof(a));
     memset(&m, 0, sizeof(m));
-    a.N = N; a.H = q.H; a.W = q.W; a.BW = q.BW; a.BN = q.BN;
-    a.nxs = (q.W + q.BW - 1) / q.BW;
-    a.ncg = ((N + q.BN - 1) / q.BN) * a.nxs;
+    conv3x3_init_geometry(&a, N, q.H, q.W, io.kvalid, -1);
     a.nchunks = io.nchunks;
-    a.tail_ksteps = io.kvalid ? conv3x3_tail_ksteps(io.kvalid) : 4;
-    a.mode = q.mode;
     a.fmt_in = io.fmt;
-    a.rows_total = static_cast<long long>(a.ncg) * q.H;
     a.wpack = io.wpack; a.bias = io.bias;
     a.ep_mode = io.ep_mode; a.lrelu = io.lrelu; a.clamp01 = io.clamp01;
-    int rc = conv3x3_make_tmap_act(&m.a, io.in16, N, q.H, q.W, io.in_c, q.mode, q.BW, q.BN, io.kvalid);
+    int rc = conv3x3_make_tmap_act(&m.a, io.in16, N, a.H, a.W, io.in_c, a.mode, a.BW, a.BN, io.kvalid);
     if (io.out16) {
         a.has_out16 = 1; a.out16_fmt = io.out16_fmt; a.out16_choff = io.out16_choff; a.out16_up2 = io.out16_up2;
         a.out16_slice_fixed = io.out16_fixed; a.slice_no16_mask = io.no16_mask;
-        rc |= conv3x3_make_tmap_out16(&m.o16, io.out16, N, q.H, q.W, io.out16_c, io.nout, q.BW, q.BN, io.out16_up2);
+        rc |= conv3x3_make_tmap_out16(&m.o16, io.out16, N, a.H, a.W, io.out16_c, io.nout, a.BW, a.BN, io.out16_up2);
     }
     if (io.outf) {
         a.has_outf = 1; a.outf_choff = io.outf_choff; a.slice_noutf_mask = io.noutf_mask;
         a.outf = io.outf; a.outf_cstride = io.outf_c;
-        rc |= conv3x3_make_tmap_f32(&m.of, io.outf, N, q.H, q.W, io.outf_c, q.BW, q.BN);
+        rc |= conv3x3_make_tmap_f32(&m.of, io.outf, N, a.H, a.W, io.outf_c, a.BW, a.BN);
     }
     if (io.res1) {
         a.has_res1 = 1; a.res_choff = io.res_choff; a.slice_nores_mask = io.nores_mask;
@@ -379,7 +365,7 @@ ConvIO fwd_io(const resr_generator* g, int k) {
 }
 
 int forward_train(resr_generator* g, const float* x, float* y, int N, int H, int W, const Bufs& B, cudaStream_t s) {
-    const Geo g0 = make_geo(g, H, W), g1 = make_geo(g, 2 * H, 2 * W), g2 = make_geo(g, 4 * H, 4 * W);
+    const Geo g0{H, W}, g1{2 * H, 2 * W}, g2{4 * H, 4 * W};
     // (no clearing of the concat buffers: a layer's activation tensor map ends at its last input channel, the rest of
     // the tail chunk is zero-filled by TMA, so never-written growth channels are never read)
     RESR_TRY(resr_nchw_to_nhwc16(x, B.xin, N, 3, H, W, 64, g->precision == 1 ? 1 : 0, s));
@@ -530,7 +516,7 @@ static void record_bucket(resr_generator* g, int i, cudaStream_t st) {
 
 // Common backward: B.biga holds conv4's output gradient (NHWC bf16 [16P][64], 3 channels used).
 int backward_common(resr_generator* g, float* grads, int N, int H, int W, const Bufs& B, cudaStream_t s) {
-    const Geo g0 = make_geo(g, H, W), g1 = make_geo(g, 2 * H, 2 * W), g2 = make_geo(g, 4 * H, 4 * W);
+    const Geo g0{H, W}, g1{2 * H, 2 * W}, g2{4 * H, 4 * W};
     const size_t P = static_cast<size_t>(N) * H * W;
     ensure_transposed_packs(g, s, true);
     g->ev_dyc_valid[0] = g->ev_dyc_valid[1] = g->ev_dyc_valid[2] = false;

@@ -1,4 +1,4 @@
-"""Sustained forward loop with NVML power / clock sampling (development aid). RESR_CONV_DBGFLAGS perturbs the kernel."""
+"""Sustained forward loop with NVML power / clock sampling (development aid)."""
 import sys, os, time, threading
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch, pynvml
@@ -31,6 +31,6 @@ while time.time() - t0 < secs:
 stop.set(); t.join()
 half = rows[len(rows) // 2:]
 med = lambda v: sorted(v)[len(v) // 2]
-print(f"flags={os.environ.get('RESR_CONV_DBGFLAGS','0')} nepi={os.environ.get('RESR_CONV_NEPI','-')}: first {times[0]:.2f} ms  last {times[-1]:.2f} ms  "
+print(f"first {times[0]:.2f} ms  last {times[-1]:.2f} ms  "
       f"power {med([r[0] for r in half]):.0f} W  sm {med([r[1] for r in half])} MHz  mem {med([r[2] for r in half])} MHz  "
       f"limit {pynvml.nvmlDeviceGetEnforcedPowerLimit(hd)/1e3:.0f} W")

@@ -21,5 +21,4 @@ ev1.record()
 torch.cuda.synchronize()
 ms = ev0.elapsed_time(ev1) / iters
 flop = 35853696.0 * n * h * w
-print(f"{n}x3x{h}x{w}: {ms:.3f} ms/forward  {n*h*w/ms/1e3:.3f} LR Mpix/s  {flop/ms/1e9:.1f} TFLOP/s  "
-      f"mode={os.environ.get('RESR_CONV_MODE','auto')}")
+print(f"{n}x3x{h}x{w}: {ms:.3f} ms/forward  {n*h*w/ms/1e3:.3f} LR Mpix/s  {flop/ms/1e9:.1f} TFLOP/s")
