@@ -339,6 +339,16 @@ int resr_niqe_num_blocks(int h, int w, int crop_border, int block);
 size_t resr_niqe_workspace_bytes(int b, int h, int w, int crop_border, int block);
 int resr_niqe_features(const float* image_rgb, double* features, int b, int h, int w, int crop_border, int block,
                        void* workspace, size_t workspace_bytes, void* stream);
+/* A list of differently sized images in one call: the reference's test.py / validate() score one image at a time, and
+ * benchmark sets differ in size. images[i] is fp32 NCHW [1,3,hs[i],ws[i]] in device memory; the pointer and size ARRAYS are
+ * host memory. features: float64 [total_blocks, 36]; image i's blocks are rows [block_offsets[i], block_offsets[i+1]) in
+ * the row-major order of resr_niqe_features, and each image's rows are bit-identical to its own resr_niqe_features call.
+ * block_offsets (host, count + 1 entries) is filled by the call. crop_border and block apply to every image; an image
+ * without a block after cropping, an empty or negative size or a bad block returns RESR_E_INVALID before any device work
+ * (the message names the image). resr_niqe_many_workspace_bytes returns 0 for any such argument. */
+size_t resr_niqe_many_workspace_bytes(const int* hs, const int* ws, int count, int crop_border, int block);
+int resr_niqe_features_many(const float* const* images, const int* hs, const int* ws, int count, int crop_border, int block,
+                            double* features, int* block_offsets, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- the whole degradation block in one call (train_realesrnet.py:267-377 == train_realesrgan.py:347-457) ---------------
  * A POD plan holds every host decision of one execution of the block; per-sample parameters and host-fed random draws

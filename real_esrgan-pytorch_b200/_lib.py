@@ -105,6 +105,9 @@ SIGNATURES = {
     "resr_niqe_num_blocks": (c_int, [c_int, c_int, c_int, c_int]),
     "resr_niqe_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int, c_int]),
     "resr_niqe_features": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_size_t, c_void_p]),
+    "resr_niqe_many_workspace_bytes": (c_size_t, [c_void_p, c_void_p, c_int, c_int, c_int]),
+    "resr_niqe_features_many": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_size_t,
+                                        c_void_p]),
     "resr_augment_batch_u8": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "resr_usm_backward_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int]),
     "resr_usm_sharp_backward": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_float, c_float,

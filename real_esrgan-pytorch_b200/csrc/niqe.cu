@@ -11,6 +11,7 @@
 #include <cmath>
 #include <cstdint>
 #include <cstring>
+#include <vector>
 #include <cuda_runtime.h>
 
 #include "../../include/resr.h"
@@ -23,27 +24,60 @@ static constexpr int kGamN = 9801;   // torch.arange(0.2, 10.001, 0.001)
 __constant__ double c_niqe_win[49];
 __constant__ double c_niqe_rw[10];   // resize weights
 
+// One image of a call. Every image is cropped to hh x ww = whole blocks after `crop_border`, so hh and ww are even and
+// each image's plane size is a multiple of 4: its arena offset at a level whose rows and / or columns are halved is
+// `off >> shift` (shift 0: full size, 1: rows halved, 2: both halved), and the planes of all images stay packed.
+struct NiqeImage {
+    const float* src;   // fp32 NCHW [1, 3, H, W]
+    int H, W, hh, ww;
+    size_t off;         // first element of this image's full-size plane in the packed fp64 arenas
+    int nbw, row0;      // blocks per row; first block (= feature row) of this image
+};
+
+// Image of arena element i at `shift`: the last image whose plane starts at or before i (planes are never empty).
+__device__ __forceinline__ int niqe_image_of_pixel(const NiqeImage* __restrict__ t, int count, size_t i, int shift) {
+    int lo = 0, hi = count - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if ((t[mid].off >> shift) <= i) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+
+__device__ __forceinline__ int niqe_image_of_block(const NiqeImage* __restrict__ t, int count, int blk) {
+    int lo = 0, hi = count - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (t[mid].row0 <= blk) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+
 // Y channel of rgb2ycbcr_torch(only_use_y_channel=True) in fp32, * 255, round (half to even), as float64; the crop of
 // `crop_border` pixels and the crop to whole blocks are folded into the indexing.
-__global__ void __launch_bounds__(256) niqe_y_kernel(const float* __restrict__ x, double* __restrict__ y, int B, int H, int W, int border,
-                                                     int h, int w) {
-    const size_t total = static_cast<size_t>(B) * h * w;
-    const size_t plane = static_cast<size_t>(H) * W;
+__global__ void __launch_bounds__(256) niqe_y_kernel(const NiqeImage* __restrict__ tab, int count, double* __restrict__ y, size_t total,
+                                                     int border) {
     for (size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; i < total; i += static_cast<size_t>(gridDim.x) * blockDim.x) {
-        const int xx = static_cast<int>(i % w), yy = static_cast<int>((i / w) % h), b = static_cast<int>(i / (static_cast<size_t>(w) * h));
-        const float* p = x + static_cast<size_t>(b) * 3 * plane + static_cast<size_t>(yy + border) * W + xx + border;
+        const NiqeImage& im = tab[niqe_image_of_pixel(tab, count, i, 0)];
+        const size_t li = i - im.off, plane = static_cast<size_t>(im.H) * im.W;
+        const int xx = static_cast<int>(li % im.ww), yy = static_cast<int>(li / im.ww);
+        const float* p = im.src + static_cast<size_t>(yy + border) * im.W + xx + border;
         float v = __fadd_rn(__fadd_rn(__fmul_rn(p[0], 65.481f), __fmul_rn(p[plane], 128.553f)), __fmul_rn(p[2 * plane], 24.966f));
         v = __fdiv_rn(__fadd_rn(v, 16.0f), 255.0f);            // imgproc.py:1830, 1838
         y[i] = static_cast<double>(rintf(__fmul_rn(v, 255.0f)));   // image_quality_assessment.py:984-985
     }
 }
 
-// structdis = (y - mu) / (sqrt(|E[y^2] - mu^2| + 1e-8) + 1), 7 x 7 window, replicate padding (image_quality_assessment.py:869-873)
-__global__ void __launch_bounds__(256) niqe_mscn_kernel(const double* __restrict__ y, double* __restrict__ sd, int B, int h, int w) {
-    const size_t total = static_cast<size_t>(B) * h * w;
+// structdis = (y - mu) / (sqrt(|E[y^2] - mu^2| + 1e-8) + 1), 7 x 7 window, replicate padding (image_quality_assessment.py:869-873).
+// lvl 0: full-size planes, 1: both sides halved (second scale).
+__global__ void __launch_bounds__(256) niqe_mscn_kernel(const NiqeImage* __restrict__ tab, int count, const double* __restrict__ y,
+                                                        double* __restrict__ sd, size_t total, int lvl) {
     for (size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; i < total; i += static_cast<size_t>(gridDim.x) * blockDim.x) {
-        const int xx = static_cast<int>(i % w), yy = static_cast<int>((i / w) % h);
-        const double* img = y + (i - static_cast<size_t>(yy) * w - xx);
+        const NiqeImage& im = tab[niqe_image_of_pixel(tab, count, i, 2 * lvl)];
+        const size_t base = im.off >> (2 * lvl);
+        const int h = im.hh >> lvl, w = im.ww >> lvl;
+        const int xx = static_cast<int>((i - base) % w), yy = static_cast<int>((i - base) / w);
+        const double* img = y + base;
         double mu = 0.0, e2 = 0.0;
         for (int dy = 0; dy < 7; ++dy) {
             const int sy = min(max(yy + dy - 3, 0), h - 1);
@@ -59,15 +93,18 @@ __global__ void __launch_bounds__(256) niqe_mscn_kernel(const double* __restrict
     }
 }
 
-// One CUDA block per image block of s x s MSCN coefficients. Map m = 0: the block; m = 1..4: block * roll(block, shift_m)
-// with shifts (0,1), (1,0), (1,1), (1,-1) (torch.roll: circular inside the block, image_quality_assessment.py:851-853).
-// stats[(block * 5 + m) * 6 + {count<0, count>0, sum v^2 over v<0, sum v^2 over v>0, sum |v|, sum v^2}].
-__global__ void __launch_bounds__(256) niqe_block_stats_kernel(const double* __restrict__ sd, double* __restrict__ stats, int h, int w, int s,
-                                                               int nbh, int nbw) {
+// One CUDA block per image block of s x s MSCN coefficients (s = block >> lvl). Map m = 0: the block; m = 1..4:
+// block * roll(block, shift_m) with shifts (0,1), (1,0), (1,1), (1,-1) (torch.roll: circular inside the block,
+// image_quality_assessment.py:851-853). stats[(block * 5 + m) * 6 + {count<0, count>0, sum v^2 over v<0, sum v^2 over v>0,
+// sum |v|, sum v^2}]; `block` counts over all images, in feature-row order.
+__global__ void __launch_bounds__(256) niqe_block_stats_kernel(const NiqeImage* __restrict__ tab, int count, const double* __restrict__ sd,
+                                                               double* __restrict__ stats, int s, int lvl) {
     __shared__ double red[8][30];
     const int blk = blockIdx.x;                       // (image, block row, block column)
-    const int bw_i = blk % nbw, bh_i = (blk / nbw) % nbh, img = blk / (nbw * nbh);
-    const double* base = sd + (static_cast<size_t>(img) * h + static_cast<size_t>(bh_i) * s) * w + static_cast<size_t>(bw_i) * s;
+    const NiqeImage& im = tab[niqe_image_of_block(tab, count, blk)];
+    const int w = im.ww >> lvl, local = blk - im.row0;
+    const int bw_i = local % im.nbw, bh_i = local / im.nbw;
+    const double* base = sd + (im.off >> (2 * lvl)) + static_cast<size_t>(bh_i) * s * w + static_cast<size_t>(bw_i) * s;
     double acc[30];
 #pragma unroll
     for (int i = 0; i < 30; ++i) acc[i] = 0.0;
@@ -105,7 +142,8 @@ __global__ void __launch_bounds__(256) niqe_block_stats_kernel(const double* __r
 }
 
 // AGGD fit of one (block, map) (image_quality_assessment.py:790-836 with get_sigma=True) and its slot of the 18 features
-// (:845-858): one CUDA block; the table search is a parallel arg-min (first minimum wins, like torch.argmin).
+// (:845-858): one CUDA block; the table search is a parallel arg-min (first minimum wins, like torch.argmin). Blocks
+// count over all images of the call, so block `blk` writes feature row `blk` and needs no image table.
 __global__ void __launch_bounds__(256) niqe_aggd_kernel(const double* __restrict__ stats, const double* __restrict__ r_gam,
                                                         double* __restrict__ feat, int s, int col0) {
     __shared__ double s_val[256];
@@ -154,14 +192,19 @@ __global__ void __launch_bounds__(256) niqe_aggd_kernel(const double* __restrict
 
 // MATLAB imresize(x / 255, 0.5) * 255 with antialiasing along one axis (image_quality_assessment.py:517-585 for scale 0.5:
 // ten taps, pos = 2 i + 0.5, base = 2 i - 4, one weight set, symmetric padding of four: the edge element is used twice).
-// axis 0: rows (h -> h / 2), axis 1: columns. div_in / scale_out fold the / 255 and * 255 of :877-878 into the passes.
-__global__ void __launch_bounds__(256) niqe_resize_half_kernel(const double* __restrict__ in, double* __restrict__ out, int B, int h, int w,
-                                                               int axis, double div_in, double scale_out) {
-    const int ho = axis == 0 ? h / 2 : h, wo = axis == 1 ? w / 2 : w;
-    const size_t total = static_cast<size_t>(B) * ho * wo;
+// axis 0: rows (hh x ww -> hh / 2 x ww), axis 1: columns (hh / 2 x ww -> hh / 2 x ww / 2); `total` counts output elements.
+// div_in / scale_out fold the / 255 and * 255 of :877-878 into the passes.
+__global__ void __launch_bounds__(256) niqe_resize_half_kernel(const NiqeImage* __restrict__ tab, int count, const double* __restrict__ in,
+                                                               double* __restrict__ out, size_t total, int axis, double div_in,
+                                                               double scale_out) {
     for (size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; i < total; i += static_cast<size_t>(gridDim.x) * blockDim.x) {
-        const int xx = static_cast<int>(i % wo), yy = static_cast<int>((i / wo) % ho), b = static_cast<int>(i / (static_cast<size_t>(wo) * ho));
-        const double* img = in + static_cast<size_t>(b) * h * w;
+        const NiqeImage& im = tab[niqe_image_of_pixel(tab, count, i, axis + 1)];
+        const size_t off = im.off;
+        const int h = im.hh >> axis, w = im.ww;
+        const int wo = w >> axis;
+        const size_t li = i - (off >> (axis + 1));
+        const int xx = static_cast<int>(li % wo), yy = static_cast<int>(li / wo);
+        const double* img = in + (off >> axis);
         const int n = axis == 0 ? h : w, o = axis == 0 ? yy : xx;
         double acc = 0.0;
 #pragma unroll
@@ -225,6 +268,77 @@ static int niqe_tables(double** r_gam_out, cudaStream_t s) {
     return RESR_OK;
 }
 
+// Workspace of one call: the packed fp64 arenas (Y, MSCN, the row-halved resize pass; `pixels` full-size elements each,
+// the second scale reuses their first quarter), the 30 block sums per block, then the image table.
+struct NiqeLayout {
+    size_t pixels = 0, stats = 0, table = 0, total = 0;
+    int blocks = 0;
+};
+
+// Table and layout of `count` images of sizes hs[i] x ws[i] (src pointers are filled by the caller). Rejects every bad
+// argument before any device work; an image without a block after cropping is named by its index.
+static int niqe_plan(const int* hs, const int* ws, int count, int crop_border, int block, std::vector<NiqeImage>& tab, NiqeLayout& L) {
+    if (!hs || !ws) return set_error(RESR_E_INVALID, "null argument");
+    if (count <= 0) return set_error(RESR_E_INVALID, "NIQE: %d images", count);
+    if (block <= 0 || (block & 1) || crop_border < 0)
+        return set_error(RESR_E_INVALID, "NIQE: block %d must be positive and even, crop_border %d non-negative", block, crop_border);
+    tab.assign(count, NiqeImage{});
+    size_t off = 0;
+    long long row = 0;
+    for (int i = 0; i < count; ++i) {
+        if (hs[i] <= 0 || ws[i] <= 0) return set_error(RESR_E_INVALID, "NIQE: image %d has size %d x %d", i, hs[i], ws[i]);
+        if (resr_niqe_num_blocks(hs[i], ws[i], crop_border, block) == 0)
+            return set_error(RESR_E_INVALID, "NIQE: image %d (%d x %d) is smaller than one %d x %d block after cropping %d pixels", i, hs[i],
+                             ws[i], block, block, crop_border);
+        const int nbh = (hs[i] - 2 * crop_border) / block, nbw = (ws[i] - 2 * crop_border) / block;
+        tab[i] = NiqeImage{nullptr, hs[i], ws[i], nbh * block, nbw * block, off, nbw, static_cast<int>(row)};
+        off += static_cast<size_t>(nbh * block) * (nbw * block);
+        row += static_cast<long long>(nbh) * nbw;
+        if (row > 0x7fffffff / 5) return set_error(RESR_E_INVALID, "NIQE: more than %d blocks in one call", 0x7fffffff / 5);
+    }
+    L.pixels = off;
+    L.blocks = static_cast<int>(row);
+    L.stats = 3 * off * sizeof(double);
+    L.table = (L.stats + static_cast<size_t>(L.blocks) * 30 * sizeof(double) + 255) & ~static_cast<size_t>(255);
+    L.total = L.table + static_cast<size_t>(count) * sizeof(NiqeImage) + 1024;   // + the alignment of the workspace to 256 bytes
+    return RESR_OK;
+}
+
+// Features of every image of `tab` into rows [row0, row0 + blocks) of `features`: five kernels per scale, whatever the
+// number of images.
+static int niqe_run(const std::vector<NiqeImage>& tab, const NiqeLayout& L, int crop_border, int block, double* features,
+                    void* workspace, size_t workspace_bytes, cudaStream_t s) {
+    if (workspace_bytes < L.total) return set_error(RESR_E_NOMEM, "NIQE workspace too small (need %zu bytes)", L.total);
+    double* r_gam = nullptr;
+    const int rc = niqe_tables(&r_gam, s);
+    if (rc != RESR_OK) return rc;
+    uint8_t* base = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~static_cast<uintptr_t>(255));
+    double* y = reinterpret_cast<double*>(base);
+    double* sd = y + L.pixels;
+    double* tmp = sd + L.pixels;
+    double* stats = reinterpret_cast<double*>(base + L.stats);
+    NiqeImage* tab_d = reinterpret_cast<NiqeImage*>(base + L.table);
+    const int count = static_cast<int>(tab.size());
+    // (pageable source: the copy is staged before the call returns, so `tab` may go out of scope)
+    if (cudaMemcpyAsync(tab_d, tab.data(), tab.size() * sizeof(NiqeImage), cudaMemcpyHostToDevice, s) != cudaSuccess)
+        return set_error(RESR_E_CUDA, "NIQE: table copy failed");
+    niqe_y_kernel<<<grid_of(L.pixels), 256, 0, s>>>(tab_d, count, y, L.pixels, crop_border);
+    for (int lvl = 0; lvl <= 1; ++lvl) {
+        const size_t cur = L.pixels >> (2 * lvl);
+        const int bs = block >> lvl;
+        niqe_mscn_kernel<<<grid_of(cur), 256, 0, s>>>(tab_d, count, y, sd, cur, lvl);
+        niqe_block_stats_kernel<<<L.blocks, 256, 0, s>>>(tab_d, count, sd, stats, bs, lvl);
+        niqe_aggd_kernel<<<L.blocks * 5, 256, 0, s>>>(stats, r_gam, features, bs, lvl * 18);
+        if (lvl == 0) {   // y = imresize(y / 255, 0.5) * 255: rows first, then columns (:877-878, :517-585)
+            niqe_resize_half_kernel<<<grid_of(cur / 2), 256, 0, s>>>(tab_d, count, y, tmp, cur / 2, 0, 255.0, 1.0);
+            niqe_resize_half_kernel<<<grid_of(cur / 4), 256, 0, s>>>(tab_d, count, tmp, y, cur / 4, 1, 1.0, 255.0);
+        }
+    }
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return set_error(RESR_E_CUDA, "NIQE launch: %s", cudaGetErrorString(e));
+    return RESR_OK;
+}
+
 }  // namespace resr
 
 using namespace resr;
@@ -238,47 +352,49 @@ int resr_niqe_num_blocks(int h, int w, int crop_border, int block) {
     return (hh / block) * (ww / block);
 }
 
+// A batch is a table of b equal images: one implementation for batches and lists.
+static int niqe_uniform_plan(int b, int h, int w, int crop_border, int block, std::vector<NiqeImage>& tab, NiqeLayout& L) {
+    const std::vector<int> hs(b > 0 ? b : 0, h), ws(b > 0 ? b : 0, w);
+    return niqe_plan(hs.data(), ws.data(), b, crop_border, block, tab, L);
+}
+
 size_t resr_niqe_workspace_bytes(int b, int h, int w, int crop_border, int block) {
-    const int nb = resr_niqe_num_blocks(h, w, crop_border, block);
-    if (b <= 0 || nb == 0) return 0;
-    const int hh = (h - 2 * crop_border) / block * block, ww = (w - 2 * crop_border) / block * block;
-    const size_t img = static_cast<size_t>(b) * hh * ww * sizeof(double);
-    return 3 * img + static_cast<size_t>(b) * nb * 30 * sizeof(double) + 1024;
+    std::vector<NiqeImage> tab;
+    NiqeLayout L;
+    return niqe_uniform_plan(b, h, w, crop_border, block, tab, L) == RESR_OK ? L.total : 0;
 }
 
 int resr_niqe_features(const float* image_rgb, double* features, int b, int h, int w, int crop_border, int block, void* workspace,
                        size_t workspace_bytes, void* stream) {
     if (!image_rgb || !features || !workspace) return set_error(RESR_E_INVALID, "null argument");
-    const int nb = resr_niqe_num_blocks(h, w, crop_border, block);
-    if (b <= 0 || nb == 0) return set_error(RESR_E_INVALID, "image smaller than one %d x %d block after cropping (or odd block size)", block, block);
-    if (workspace_bytes < resr_niqe_workspace_bytes(b, h, w, crop_border, block)) return set_error(RESR_E_NOMEM, "NIQE workspace too small");
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
-    double* r_gam = nullptr;
-    const int rc = niqe_tables(&r_gam, s);
+    std::vector<NiqeImage> tab;
+    NiqeLayout L;
+    const int rc = niqe_uniform_plan(b, h, w, crop_border, block, tab, L);
     if (rc != RESR_OK) return rc;
-    const int nbh = (h - 2 * crop_border) / block, nbw = (w - 2 * crop_border) / block;
-    int hh = nbh * block, ww = nbw * block;
-    const size_t img = static_cast<size_t>(b) * hh * ww;
-    double* y = reinterpret_cast<double*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~static_cast<uintptr_t>(255));
-    double* sd = y + img;
-    double* tmp = sd + img;
-    double* stats = tmp + img;
-    niqe_y_kernel<<<grid_of(img), 256, 0, s>>>(image_rgb, y, b, h, w, crop_border, hh, ww);
-    int bs = block;
-    for (int scale = 1; scale <= 2; ++scale) {
-        const size_t cur = static_cast<size_t>(b) * hh * ww;
-        niqe_mscn_kernel<<<grid_of(cur), 256, 0, s>>>(y, sd, b, hh, ww);
-        niqe_block_stats_kernel<<<b * nbh * nbw, 256, 0, s>>>(sd, stats, hh, ww, bs, nbh, nbw);
-        niqe_aggd_kernel<<<b * nbh * nbw * 5, 256, 0, s>>>(stats, r_gam, features, bs, (scale - 1) * 18);
-        if (scale == 1) {   // y = imresize(y / 255, 0.5) * 255: rows first, then columns (:877-878, :517-585)
-            niqe_resize_half_kernel<<<grid_of(cur / 2), 256, 0, s>>>(y, tmp, b, hh, ww, 0, 255.0, 1.0);
-            niqe_resize_half_kernel<<<grid_of(cur / 4), 256, 0, s>>>(tmp, y, b, hh / 2, ww, 1, 1.0, 255.0);
-            hh /= 2; ww /= 2; bs /= 2;
-        }
+    for (int i = 0; i < b; ++i) tab[i].src = image_rgb + static_cast<size_t>(i) * 3 * h * w;
+    return niqe_run(tab, L, crop_border, block, features, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
+}
+
+size_t resr_niqe_many_workspace_bytes(const int* hs, const int* ws, int count, int crop_border, int block) {
+    std::vector<NiqeImage> tab;
+    NiqeLayout L;
+    return niqe_plan(hs, ws, count, crop_border, block, tab, L) == RESR_OK ? L.total : 0;
+}
+
+int resr_niqe_features_many(const float* const* images, const int* hs, const int* ws, int count, int crop_border, int block,
+                            double* features, int* block_offsets, void* workspace, size_t workspace_bytes, void* stream) {
+    if (!images || !features || !block_offsets || !workspace) return set_error(RESR_E_INVALID, "null argument");
+    std::vector<NiqeImage> tab;
+    NiqeLayout L;
+    const int rc = niqe_plan(hs, ws, count, crop_border, block, tab, L);
+    if (rc != RESR_OK) return rc;
+    for (int i = 0; i < count; ++i) {
+        if (!images[i]) return set_error(RESR_E_INVALID, "NIQE: null image pointer %d", i);
+        tab[i].src = images[i];
+        block_offsets[i] = tab[i].row0;
     }
-    const cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return set_error(RESR_E_CUDA, "NIQE launch: %s", cudaGetErrorString(e));
-    return RESR_OK;
+    block_offsets[count] = L.blocks;
+    return niqe_run(tab, L, crop_border, block, features, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
 }
 
 }  // extern "C"
