@@ -125,8 +125,13 @@ int resr_generator_launches_per_forward(void);
 int resr_set_conv_pair_policy(int policy);
 
 /* One 3x3 convolution through the same tensor-core kernel (test / building block).
- * in16: NHWC 16-bit activations [n,h,w,c_total]; the first `cin` channels are convolved.
- * weight: OIHW fp32 [cout,cin,3,3]; bias: fp32 [cout] or NULL. */
+ * in16: NHWC 16-bit activations [n,h,w,c_total]; exactly the first `cin` channels are read (the tensor map ends there:
+ * whatever the channels [cin, c_total) hold, NaN included, does not reach the output). c_total is a multiple of 8 and
+ * at least cin rounded up to 64. weight: OIHW fp32 [cout,cin,3,3]; bias: fp32 [cout] or NULL.
+ * Outputs and residuals are addressed per 32-channel Cout slice: an NHWC output (out16 / outf) needs cout % 32 == 0 and
+ * choff + cout <= cstride; cout < 32 (the RGB convolution) writes out_nchw / out_nchw_raw / out_u8 only. 16-bit NHWC
+ * strides and offsets are multiples of 8 channels, fp32 ones multiples of 4 (16-byte vector accesses).
+ * Every argument is checked on the host before any device work; a bad one returns RESR_E_INVALID. */
 typedef struct resr_conv_desc {
     const void* in16;
     int n, h, w, c_total, cin, cout;
@@ -134,7 +139,8 @@ typedef struct resr_conv_desc {
     int mode;    /* -1 auto, 0 shifted-descriptor loads, 1 three loads per row */
     const float* weight;
     const float* bias;
-    int ep_mode; /* 0 plain, 1 rdb: 0.2*v+res1, 2 rrdb: 0.2*(0.2*v+res1)+res2, 3 skip: res1+v */
+    int ep_mode; /* 0 plain, 1 rdb: 0.2*v+res1, 2 rrdb: 0.2*(0.2*v+res1)+res2, 3 skip: res1+v,
+                    4 add2: v [+ res1] + res2_scale*res2 (fp32 res2) */
     int lrelu, clamp01;
     void* out16;
     int out16_fmt, out16_cstride, out16_choff, out16_up2;
@@ -145,9 +151,43 @@ typedef struct resr_conv_desc {
     int res_cstride, res_choff;
     int res16, res16_fmt;    /* res16 = 1: res1 / res2 are 16-bit tensors of format res16_fmt (0 fp16, 1 bf16) */
     float* out_nchw;
-    int out_nchw_c;
+    int out_nchw_c;          /* channels of out_nchw / out_nchw_raw / out_u8: must equal cout */
+    /* ---- what the generator's and the training step's launches set as well (zero: off) */
+    int reverse;             /* CTA-pair kernel: walk rows and column groups back to front (serpentine layer order) */
+    const uint32_t* vmask;   /* packed canvas: bit (x >> vmask_shift, y >> vmask_shift) of a row-major bitmap with */
+    int vmask_words;         /* vmask_words 32-bit words per row marks a valid pixel; every output of an invalid pixel */
+    int vmask_shift;         /* is written as 0 */
+    unsigned char* out_u8;   /* NHWC u8 [n,h,w,out_nchw_c]: (unsigned char)(255 * v) of the clamped value */
+    float* out_nchw_raw;     /* NCHW fp32 copy of the value before clamp01 */
+    const void* mask16;      /* LeakyReLU' mask: 16-bit NHWC activations (fp16 or bf16); out16 stores v where the */
+    int mask16_cstride, mask16_choff;  /* activation is > 0 and 0.2 v elsewhere (-0 and +0 count as not positive) */
+    float out16_scale;       /* != 0: out16 stores out16_scale * v (outf keeps v) */
+    float res2_scale;        /* ep_mode 4 */
+    int res2_cstride;        /* 0: res_cstride */
+    unsigned slice_nores_mask, slice_noutf_mask, slice_no16_mask;  /* bit s: 32-channel slice s skips res1 / outf / out16 */
+    int out16_slice_fixed;   /* 1: every writing slice stores at out16_choff instead of out16_choff + 32 s */
 } resr_conv_desc;
 int resr_conv3x3(const resr_conv_desc* d, void* stream);
+
+/* The launch configuration resr_conv3x3 uses for `d` on a device with `num_sms` SMs. Host only: needs no device, reads
+ * no pointer of `d` (only whether it is NULL), honours resr_set_conv_pair_policy. resr_conv3x3 plans through this very
+ * function, so the report cannot drift from what runs. Returns RESR_E_INVALID (and fills nothing) for every
+ * descriptor resr_conv3x3 would reject, including one whose weights and staging do not fit in shared memory. */
+typedef struct resr_conv_plan {
+    int pair;           /* 1: CTA-pair kernel (tcgen05 cta_group::2), 0: single-CTA kernel */
+    int nout;           /* accumulator channels per output row and launch slice: 64 (pairs only), 32 or 16 */
+    int nslices;        /* Cout slices of nout channels (grid y) */
+    int bw, bn;         /* one 128-lane tile = bw consecutive columns x bn consecutive images */
+    int mode;           /* 0: one activation load per (row, chunk); 1: one per (row, chunk, dx) */
+    int nxs, ncg;       /* column segments per image row, column groups */
+    int tail_ksteps;    /* K16 steps of the last 64-channel chunk (1, 2 or 4) */
+    int nepi, epi_bufs; /* epilogue warp groups, staging buffers per group */
+    int nstages;        /* activation pipeline stages */
+    int masked;         /* the packed-canvas (vmask) instantiation */
+    long long units;    /* work units: (column group, row), or (pair of column groups, row) for pairs */
+    long long clusters; /* clusters in the grid (one or two CTAs each) per Cout slice */
+} resr_conv_plan;
+int resr_conv3x3_plan(const resr_conv_desc* d, int num_sms, resr_conv_plan* plan);
 
 /* Layout helpers used by the generator (exposed for tests): NCHW fp32 -> NHWC 16-bit, channels zero-padded. */
 int resr_nchw_to_nhwc16(const float* x, void* out16, int n, int c, int h, int w, int c_pad, int fmt, void* stream);

@@ -28,7 +28,24 @@ class ConvDesc(Structure):
         ("res16", c_int), ("res16_fmt", c_int),
         ("out_nchw", c_void_p),
         ("out_nchw_c", c_int),
+        ("reverse", c_int),
+        ("vmask", c_void_p), ("vmask_words", c_int), ("vmask_shift", c_int),
+        ("out_u8", c_void_p),
+        ("out_nchw_raw", c_void_p),
+        ("mask16", c_void_p), ("mask16_cstride", c_int), ("mask16_choff", c_int),
+        ("out16_scale", c_float),
+        ("res2_scale", c_float),
+        ("res2_cstride", c_int),
+        ("slice_nores_mask", ctypes.c_uint), ("slice_noutf_mask", ctypes.c_uint), ("slice_no16_mask", ctypes.c_uint),
+        ("out16_slice_fixed", c_int),
     ]
+
+
+class ConvPlan(Structure):
+    """struct resr_conv_plan (include/resr.h)."""
+    _fields_ = [("pair", c_int), ("nout", c_int), ("nslices", c_int), ("bw", c_int), ("bn", c_int), ("mode", c_int),
+                ("nxs", c_int), ("ncg", c_int), ("tail_ksteps", c_int), ("nepi", c_int), ("epi_bufs", c_int),
+                ("nstages", c_int), ("masked", c_int), ("units", ctypes.c_longlong), ("clusters", ctypes.c_longlong)]
 
 
 class ResizeSpec(Structure):
@@ -99,6 +116,7 @@ SIGNATURES = {
     "resr_generator_launches_per_forward": (c_int, []),
     "resr_set_conv_pair_policy": (c_int, [c_int]),
     "resr_conv3x3": (c_int, [POINTER(ConvDesc), c_void_p]),
+    "resr_conv3x3_plan": (c_int, [POINTER(ConvDesc), c_int, POINTER(ConvPlan)]),
     "resr_nchw_to_nhwc16": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "resr_filter2d": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "resr_usm_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int]),

@@ -100,6 +100,16 @@ struct ConvLaunchCfg {
 // configuration does not fit in shared memory.
 int conv3x3_set_pair_policy(int policy);  // returns the previous policy; -1 only queries
 bool conv3x3_choose(ConvArgs* args, int pack_nout, int pack_nslices, ConvLaunchCfg* cfg);
+
+// Clusters of `cluster` CTAs per Cout slice of the persistent grid over `units` work units: as many as the SMs hold,
+// but at least 4 rows of work each (tiny problems are not shredded into 1-row strips with 2 halo rows each).
+inline long long conv3x3_clusters(long long units, int cluster, int nslices, int num_sms) {
+    long long nclusters = (num_sms / cluster) / nslices;
+    const long long min_rows = 4;
+    const long long cap = (units + min_rows - 1) / min_rows;
+    if (nclusters > cap) nclusters = cap;
+    return nclusters < 1 ? 1 : nclusters;
+}
 cudaError_t conv3x3_run(const ConvMaps& maps, const ConvArgs& args, const ConvLaunchCfg& cfg, int num_sms, cudaStream_t stream);
 
 // Tensor maps. base: NHWC tensor [N,H,W,C].

@@ -351,11 +351,7 @@ static cudaError_t conv3x3_launch_grid(const ConvMaps& maps, const ConvArgs& arg
     const int smem = 1024 + conv3x3_weight_bytes(args, nout, cluster) + args.nstages * kStageBytes +
                      args.nepi * epi_group_bytes(args, subw) + kMiscBytes;
     if (args.nstages < 2 || args.nepi < 1 || args.nepi > 3 || smem > kSmemMax) return cudaErrorInvalidConfiguration;
-    long long nclusters = (num_sms / cluster) / nslices;
-    const long long min_rows = 4;  // do not shred tiny problems into 1-row strips (2 halo rows each)
-    const long long cap = (units + min_rows - 1) / min_rows;
-    if (nclusters > cap) nclusters = cap;
-    if (nclusters < 1) nclusters = 1;
+    const long long nclusters = conv3x3_clusters(units, cluster, nslices, num_sms);
     if (units * (nclusters + 1) >= (1ll << 31)) return cudaErrorInvalidValue;   // the kernel's strip arithmetic is 32-bit
 
     static PerDevice<bool> attr;  // function attributes are per device

@@ -374,8 +374,11 @@ int conv3x3_make_tmap_act(CUtensorMap* out, const void* base, int N, int H, int 
     PFN_encodeTiled enc = get_encode_fn();
     if (!enc) return -1;
     // Channels at and beyond `cvalid` are out of bounds for the map: the 64-channel box of the tail chunk is zero-filled
-    // there instead of fetching the neighbouring (zero-weight) channels of the concat buffer from DRAM.
-    int cdim = cvalid > 0 ? (cvalid + 7) / 8 * 8 : C;
+    // there instead of fetching the neighbouring (zero-weight) channels of the concat buffer from DRAM. The map ends at
+    // exactly `cvalid` (TMA extents need no alignment, only the strides do): a zero weight times a NaN or Inf in a
+    // channel past `cvalid` would still be NaN. A caller that owns zeroed padding channels may pass cvalid rounded up
+    // to 8: a 16-byte row per pixel loads faster than a 6-byte one (the 3-channel first convolution).
+    int cdim = cvalid > 0 ? cvalid : C;
     if (cdim > C) cdim = C;
     const cuuint64_t dims[4] = {static_cast<cuuint64_t>(cdim), static_cast<cuuint64_t>(W), static_cast<cuuint64_t>(H),
                                 static_cast<cuuint64_t>(N)};

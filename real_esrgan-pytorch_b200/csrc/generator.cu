@@ -477,7 +477,8 @@ static int build_plan(resr_generator* g, Plan& p, int N, int H, int W, void* ws,
         a.wpack = g->wpack + cs.w_off;
         a.bias = g->bias + cs.b_off;
         if (vmask) { a.vmask = vmask; a.vmask_words = W / 32; a.vmask_shift = s; }
-        map_rc |= conv3x3_make_tmap_act(&st.maps.a, in16, N, a.H, a.W, cin_total, a.mode, a.BW, a.BN, cs.cin);
+        // the input's channels past cs.cin are zeros this library wrote: the map may end at the next multiple of 8
+        map_rc |= conv3x3_make_tmap_act(&st.maps.a, in16, N, a.H, a.W, cin_total, a.mode, a.BW, a.BN, (cs.cin + 7) / 8 * 8);
         return st;
     };
     auto set_out16 = [&](Step& st, void* dst, int c_total, int choff, int fmt, int up2) {
@@ -965,58 +966,146 @@ int resr_nchw_to_nhwc16(const float* x, void* out16, int n, int c, int h, int w,
     return RESR_OK;
 }
 
-int resr_conv3x3(const resr_conv_desc* d, void* stream) {
-    if (!d || !d->in16 || !d->weight) return set_error(RESR_E_INVALID, "null argument");
-    if (d->cin > d->c_total || d->c_total % 8 != 0) return set_error(RESR_E_INVALID, "bad channel counts");
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+// The one planning path of resr_conv3x3 and resr_conv3x3_plan: checks every field of `d`, then fills `a` (geometry,
+// epilogue flags and pointers; no tensor maps, no weight pack) and `cfg` exactly as the launch will use them. Host only.
+// Returns nullptr, or what is wrong with `d` (RESR_E_INVALID).
+static const char* conv_desc_plan(const resr_conv_desc* d, int num_sms, ConvArgs* a, ConvLaunchCfg* cfg, resr_conv_plan* out) {
+    if (!d || !d->in16 || !d->weight) return "null argument";
+    if (num_sms < 1) return "num_sms must be positive";
+    if (d->n < 1 || d->h < 1 || d->w < 1 || d->cin < 1 || d->cout < 1) return "empty or negative n / h / w / cin / cout";
+    if (d->cin > d->c_total || d->c_total % 8 != 0) return "bad channel counts: cin <= c_total, c_total % 8 == 0";
+    const int nchunks = (d->cin + 63) / 64;
+    if (static_cast<long long>(nchunks) * 64 > d->c_total) return "c_total must cover cin rounded up to 64";
+    if (d->fmt_in != 0 && d->fmt_in != 1) return "fmt_in must be 0 (fp16) or 1 (bf16)";
+    if (d->mode < -1 || d->mode > 1) return "mode must be -1, 0 or 1";
+    if (d->ep_mode < EP_PLAIN || d->ep_mode > EP_ADD2) return "ep_mode must be 0..4";
+    const bool mode_res1 = d->ep_mode == EP_RDB || d->ep_mode == EP_RRDB || d->ep_mode == EP_SKIP;
+    const bool mode_res2 = d->ep_mode == EP_RRDB || d->ep_mode == EP_ADD2;
+    if ((mode_res1 && !d->res1) || (mode_res2 && !d->res2)) return "ep_mode needs a residual that is NULL";
+    if (d->res16 != 0 && d->res16 != 1) return "res16 must be 0 or 1";
+    if (d->res16_fmt != 0 && d->res16_fmt != 1) return "res16_fmt must be 0 or 1";
+    if (d->ep_mode == EP_ADD2 && d->res16) return "ep_mode 4 reads fp32 residuals";
+    // one launch slice is 32 output channels (16 for the RGB convolution); NHWC stores and residual loads cover whole slices
     const int nout = d->cout >= 32 ? 32 : 16;
     const int nslices = (d->cout + nout - 1) / nout;
-    const int nchunks = (d->cin + 63) / 64;
-    if (nchunks * 64 > d->c_total) return set_error(RESR_E_INVALID, "c_total must cover cin rounded up to 64");
-    const size_t pack_bytes = static_cast<size_t>(nslices) * nchunks * 3 * (3 * nout) * 128;
-    uint8_t* wp = nullptr;
-    float* bp = nullptr;
-    if (cudaMalloc(&wp, pack_bytes) != cudaSuccess || cudaMalloc(&bp, nslices * nout * 4) != cudaSuccess)
-        return set_error(RESR_E_CUDA, "cudaMalloc failed");
-    launch_pack_conv(d->weight, d->bias, reinterpret_cast<uint16_t*>(wp), bp, d->cin, d->cout, nout, nslices, nchunks,
-                     d->fmt_in, 0, s);
-    cudaStreamSynchronize(s);  // the conv prefetches its weights before the programmatic grid dependency resolves
-    ConvArgs a;
-    ConvMaps maps;
-    memset(&a, 0, sizeof(a));
-    memset(&maps, 0, sizeof(maps));
-    conv3x3_init_geometry(&a, d->n, d->h, d->w, d->cin, d->mode);
-    a.nchunks = nchunks;
-    a.fmt_in = d->fmt_in;
-    a.wpack = wp; a.bias = bp;
-    a.ep_mode = d->ep_mode; a.lrelu = d->lrelu; a.clamp01 = d->clamp01;
-    int rc = conv3x3_make_tmap_act(&maps.a, d->in16, d->n, d->h, d->w, d->c_total, a.mode, a.BW, a.BN, d->cin);
+    if ((d->out16 || d->outf) && d->cout % 32 != 0)
+        return "an NHWC output (out16 / outf) needs cout % 32 == 0: the stores write whole 32-channel slices";
+    if (nout == 16 && (d->res1 || d->res2)) return "cout < 32 takes no residual";
+    if ((d->out_nchw || d->out_nchw_raw || d->out_u8) && d->out_nchw_c != d->cout) return "out_nchw_c must equal cout";
+    const long long span = static_cast<long long>(nslices) * nout;  // channels a residual / mask read covers
     if (d->out16) {
-        a.has_out16 = 1; a.out16_fmt = d->out16_fmt; a.out16_choff = d->out16_choff; a.out16_up2 = d->out16_up2;
-        rc |= conv3x3_make_tmap_out16(&maps.o16, d->out16, d->n, d->h, d->w, d->out16_cstride, nout, a.BW, a.BN, d->out16_up2);
+        if (d->out16_fmt != 0 && d->out16_fmt != 1) return "out16_fmt must be 0 or 1";
+        if (d->out16_up2 != 0 && d->out16_up2 != 1) return "out16_up2 must be 0 or 1";
+        if (d->out16_cstride < 1 || d->out16_cstride % 8 != 0) return "out16_cstride must be a positive multiple of 8";
+        if (d->out16_choff < 0 || d->out16_choff + (d->out16_slice_fixed ? 32ll : span) > d->out16_cstride)
+            return "out16 channels [choff, choff + cout) must lie inside out16_cstride";
     }
     if (d->outf) {
-        a.has_outf = 1; a.outf_choff = d->outf_choff; a.outf = static_cast<float*>(d->outf); a.outf_cstride = d->outf_cstride;
-        rc |= conv3x3_make_tmap_f32(&maps.of, d->outf, d->n, d->h, d->w, d->outf_cstride, a.BW, a.BN);
+        if (d->outf_cstride < 1 || d->outf_cstride % 4 != 0) return "outf_cstride must be a positive multiple of 4";
+        if (d->outf_choff < 0 || d->outf_choff + span > d->outf_cstride) return "outf channels [choff, choff + cout) must lie inside outf_cstride";
+    }
+    const int res_align = d->res16 ? 8 : 4;   // 16-byte vector loads
+    const int res2_cstride = d->res2_cstride ? d->res2_cstride : d->res_cstride;
+    if ((d->res1 || d->res2) && (d->res_choff < 0 || d->res_choff % res_align != 0))
+        return "res_choff must be a non-negative multiple of 8 (16-bit) / 4 (fp32) channels";
+    if (d->res1 && (d->res_cstride % res_align != 0 || d->res_choff + span > d->res_cstride))
+        return "res1: res_cstride must be a multiple of 8 (16-bit) / 4 (fp32) and hold res_choff + cout channels";
+    if (d->res2 && (res2_cstride % res_align != 0 || d->res_choff + span > res2_cstride))
+        return "res2: res2_cstride must be a multiple of 8 (16-bit) / 4 (fp32) and hold res_choff + cout channels";
+    if (d->mask16 && d->out16 && (d->mask16_cstride % 8 != 0 || d->mask16_choff < 0 || d->mask16_choff % 8 != 0 ||
+                                  d->mask16_choff + span > d->mask16_cstride))
+        return "mask16: stride and offset must be multiples of 8 holding mask16_choff + cout channels";
+    if (d->vmask && (d->vmask_shift < 0 || d->vmask_shift > 15 || d->vmask_words < 1 ||
+                     static_cast<long long>(d->vmask_words) * 32 <= ((d->w - 1) >> d->vmask_shift)))
+        return "vmask: vmask_shift must be 0..15 and vmask_words cover every column";
+
+    memset(a, 0, sizeof(*a));
+    conv3x3_init_geometry(a, d->n, d->h, d->w, d->cin, d->mode);
+    a->nchunks = nchunks;
+    a->fmt_in = d->fmt_in;
+    a->ep_mode = d->ep_mode; a->lrelu = d->lrelu; a->clamp01 = d->clamp01;
+    a->reverse = d->reverse != 0;
+    if (d->out16) {
+        a->has_out16 = 1; a->out16_fmt = d->out16_fmt; a->out16_choff = d->out16_choff; a->out16_up2 = d->out16_up2;
+        a->out16_slice_fixed = d->out16_slice_fixed; a->slice_no16_mask = d->slice_no16_mask;
+        a->mask16 = d->mask16; a->mask16_cstride = d->mask16_cstride; a->mask16_choff = d->mask16_choff;
+        a->out16_scale = d->out16_scale;
+    }
+    if (d->outf) {
+        a->has_outf = 1; a->outf_choff = d->outf_choff; a->outf = d->outf; a->outf_cstride = d->outf_cstride;
+        a->slice_noutf_mask = d->slice_noutf_mask;
     }
     if (d->res1) {
-        a.has_res1 = 1; a.res_choff = d->res_choff; a.res1 = d->res1; a.res1_cstride = d->res_cstride;
-        a.res16 = d->res16; a.res16_fmt = d->res16_fmt;
+        a->has_res1 = 1; a->res_choff = d->res_choff; a->res1 = d->res1; a->res1_cstride = d->res_cstride;
+        a->slice_nores_mask = d->slice_nores_mask;
     }
-    a.res2 = d->res2; a.res2_cstride = d->res_cstride;
-    a.out_nchw = d->out_nchw; a.out_nchw_c = d->out_nchw_c;
+    a->res16 = d->res16; a->res16_fmt = d->res16_fmt;
+    a->res2 = d->res2; a->res2_cstride = res2_cstride; a->res2_scale = d->res2_scale;
+    if (d->res2 && !d->res1) a->res_choff = d->res_choff;
+    a->out_nchw = d->out_nchw; a->out_nchw_raw = d->out_nchw_raw; a->out_u8 = d->out_u8; a->out_nchw_c = d->out_nchw_c;
+    a->vmask = d->vmask; a->vmask_words = d->vmask_words; a->vmask_shift = d->vmask_shift;
+    if (!conv3x3_choose(a, nout, nslices, cfg))
+        return "the weights of cin input channels and the output staging do not fit in shared memory";
+    const long long units = cfg->pair ? static_cast<long long>((a->ncg + 1) / 2) * a->H : a->rows_total;
+    const long long clusters = conv3x3_clusters(units, cfg->pair ? 2 : 1, cfg->nslices, num_sms);
+    if (units * (clusters + 1) >= (1ll << 31)) return "too many rows for the kernels' 32-bit strip arithmetic";
+    if (out) {
+        out->pair = cfg->pair; out->nout = cfg->nout; out->nslices = cfg->nslices;
+        out->bw = a->BW; out->bn = a->BN; out->mode = a->mode; out->nxs = a->nxs; out->ncg = a->ncg;
+        out->tail_ksteps = a->tail_ksteps;
+        out->nepi = a->nepi; out->epi_bufs = a->epi_bufs; out->nstages = a->nstages;
+        out->masked = a->vmask != nullptr;
+        out->units = units; out->clusters = clusters;
+    }
+    return nullptr;
+}
+
+int resr_conv3x3_plan(const resr_conv_desc* d, int num_sms, resr_conv_plan* plan) {
+    if (!plan) return set_error(RESR_E_INVALID, "null argument");
+    ConvArgs a;
     ConvLaunchCfg cfg;
-    if (!conv3x3_choose(&a, nout, nslices, &cfg)) rc |= 1 << 20;
-    if (nout == 16 && (d->out16 || d->outf || d->res1)) rc |= 1 << 21;  // the 16-wide slice only feeds the NCHW output
+    const char* bad = conv_desc_plan(d, num_sms, &a, &cfg, plan);
+    if (bad) return set_error(RESR_E_INVALID, "resr_conv3x3: %s", bad);
+    return RESR_OK;
+}
+
+int resr_conv3x3(const resr_conv_desc* d, void* stream) {
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    // the SM count only sizes the grid; without a device the descriptor is still checked (and a bad one rejected)
+    int dev = 0, sms = 0;
+    const bool have_dev = cudaGetDevice(&dev) == cudaSuccess &&
+                          cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && sms > 0;
+    if (!have_dev) { cudaGetLastError(); sms = 1; }
+    ConvArgs a;
+    ConvLaunchCfg cfg;
+    const char* bad = conv_desc_plan(d, sms, &a, &cfg, nullptr);
+    if (bad) return set_error(RESR_E_INVALID, "resr_conv3x3: %s", bad);
+    if (!have_dev) return set_error(RESR_E_CUDA, "resr_conv3x3: no CUDA device");
+    const int nout = d->cout >= 32 ? 32 : 16;   // the weight pack's slice width (a pair launch takes two 32-slices)
+    const int nslices = (d->cout + nout - 1) / nout;
+    const size_t pack_bytes = static_cast<size_t>(nslices) * a.nchunks * 3 * (3 * nout) * 128;
+    uint8_t* wp = nullptr;
+    float* bp = nullptr;
+    if (cudaMalloc(&wp, pack_bytes) != cudaSuccess) return set_error(RESR_E_CUDA, "cudaMalloc failed");
+    if (cudaMalloc(&bp, nslices * nout * 4) != cudaSuccess) {
+        cudaFree(wp);
+        return set_error(RESR_E_CUDA, "cudaMalloc failed");
+    }
+    launch_pack_conv(d->weight, d->bias, reinterpret_cast<uint16_t*>(wp), bp, d->cin, d->cout, nout, nslices, a.nchunks,
+                     d->fmt_in, 0, s);
+    cudaStreamSynchronize(s);  // the conv prefetches its weights before the programmatic grid dependency resolves
+    a.wpack = wp; a.bias = bp;
+    ConvMaps maps;
+    memset(&maps, 0, sizeof(maps));
+    int rc = conv3x3_make_tmap_act(&maps.a, d->in16, d->n, d->h, d->w, d->c_total, a.mode, a.BW, a.BN, d->cin);
+    if (d->out16) rc |= conv3x3_make_tmap_out16(&maps.o16, d->out16, d->n, d->h, d->w, d->out16_cstride, nout, a.BW, a.BN, d->out16_up2);
+    if (d->outf) rc |= conv3x3_make_tmap_f32(&maps.of, d->outf, d->n, d->h, d->w, d->outf_cstride, a.BW, a.BN);
     cudaError_t e = cudaSuccess;
     if (rc == 0) e = conv3x3_run(maps, a, cfg, sms, s);
     const cudaError_t e2 = cudaStreamSynchronize(s);
     cudaFree(wp);
     cudaFree(bp);
-    if (rc != 0) return set_error(RESR_E_CUDA, "tensor map / shared memory planning failed (%d)", rc);
+    if (rc != 0) return set_error(RESR_E_CUDA, "tensor map encoding failed (%d)", rc);
     if (e != cudaSuccess) return set_error(RESR_E_CUDA, "conv launch: %s", cudaGetErrorString(e));
     if (e2 != cudaSuccess) return set_error(RESR_E_CUDA, "conv run: %s", cudaGetErrorString(e2));
     return RESR_OK;

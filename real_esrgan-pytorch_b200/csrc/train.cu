@@ -224,7 +224,8 @@ static int launch_conv_io(const resr_generator* g, const Geo& q, int N, const Co
     a.fmt_in = io.fmt;
     a.wpack = io.wpack; a.bias = io.bias;
     a.ep_mode = io.ep_mode; a.lrelu = io.lrelu; a.clamp01 = io.clamp01;
-    int rc = conv3x3_make_tmap_act(&m.a, io.in16, N, a.H, a.W, io.in_c, a.mode, a.BW, a.BN, io.kvalid);
+    // channels past kvalid are zeros this library wrote: the map may end at the next multiple of 8
+    int rc = conv3x3_make_tmap_act(&m.a, io.in16, N, a.H, a.W, io.in_c, a.mode, a.BW, a.BN, (io.kvalid + 7) / 8 * 8);
     if (io.out16) {
         a.has_out16 = 1; a.out16_fmt = io.out16_fmt; a.out16_choff = io.out16_choff; a.out16_up2 = io.out16_up2;
         a.out16_slice_fixed = io.out16_fixed; a.slice_no16_mask = io.no16_mask;

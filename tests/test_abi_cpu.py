@@ -156,9 +156,10 @@ def test_pod_plan_layout_matches_the_header(tmp_path):
 #include <stddef.h>
 #include "resr.h"
 int main(void) {
-    printf("%zu %zu %zu %zu %zu %zu %zu\\n", sizeof(resr_degrade_plan), sizeof(resr_resize_spec), sizeof(resr_noise_spec),
-           offsetof(resr_degrade_plan, noise1), offsetof(resr_degrade_plan, rng_state), sizeof(resr_conv_desc),
-           sizeof(resr_kernel_params));
+    printf("%zu %zu %zu %zu %zu %zu %zu %zu %zu %zu %zu\\n", sizeof(resr_degrade_plan), sizeof(resr_resize_spec),
+           sizeof(resr_noise_spec), offsetof(resr_degrade_plan, noise1), offsetof(resr_degrade_plan, rng_state),
+           sizeof(resr_conv_desc), sizeof(resr_kernel_params), offsetof(resr_conv_desc, out16_scale),
+           offsetof(resr_conv_desc, out16_slice_fixed), sizeof(resr_conv_plan), offsetof(resr_conv_plan, units));
     return 0;
 }
 ''')
@@ -167,7 +168,9 @@ int main(void) {
     subprocess.run(["gcc", "-I", inc, str(src), "-o", str(exe)], check=True)
     got = [int(v) for v in subprocess.run([str(exe)], capture_output=True, text=True, check=True).stdout.split()]
     want = [ctypes.sizeof(L.DegradePlan), ctypes.sizeof(L.ResizeSpec), ctypes.sizeof(L.NoiseSpec), L.DegradePlan.noise1.offset,
-            L.DegradePlan.rng_state.offset, ctypes.sizeof(L.ConvDesc), ctypes.sizeof(L.KernelParams)]
+            L.DegradePlan.rng_state.offset, ctypes.sizeof(L.ConvDesc), ctypes.sizeof(L.KernelParams),
+            L.ConvDesc.out16_scale.offset, L.ConvDesc.out16_slice_fixed.offset, ctypes.sizeof(L.ConvPlan),
+            L.ConvPlan.units.offset]
     assert got == want
 
 
