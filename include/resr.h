@@ -321,9 +321,10 @@ int resr_draw_degradation_kernel_params(const resr_kernel_draw_config* cfg, int 
  * grads_flat: fp32 [resr_generator_num_params()] in state_dict order (layout of resr_generator_tensor_span); every
  * element is overwritten. The flat parameter vector given to resr_generator_load_params must stay alive (the
  * transposed weight packs of the data-gradient convolutions are built from it on the first backward).
- * Two recipes (resr_generator_set_precision): 0 = fp16 activations + bf16 gradients, weight gradients through
- * channels-first copies (w % 8 == 0 required); 1 = bf16 activations and gradients with an fp32 residual stream, weight
- * gradients straight from the NHWC buffers (csrc/wgrad_mn.cu; no shape rule, ~27 % faster per step).
+ * Two recipes (resr_generator_set_precision): 0 = fp16 activations + bf16 gradients; 1 = bf16 activations and gradients
+ * with an fp32 residual stream. Both take their weight gradients from the NHWC buffers (csrc/wgrad_mn.cu; the fp16
+ * recipe's activations pass through a bf16 copy first) and have no shape rule beyond n, h, w >= 1. Bias and weight
+ * gradients are summed in a fixed order: identical steps give bit-identical grads_flat.
  * ---------------------------------------------------------------------------------------------------------- */
 size_t resr_generator_train_workspace_bytes(int n, int h, int w);
 int resr_generator_forward_train(resr_generator_t* g, const float* x, float* y, int n, int h, int w, void* workspace,
@@ -351,18 +352,12 @@ int resr_generator_wait_grad_bucket(resr_generator_t* g, int bucket, void* strea
 int resr_generator_backward(resr_generator_t* g, const float* dy, float* grads_flat, int n, int h, int w, void* workspace,
                             size_t workspace_bytes, void* stream);
 
-/* Weight / bias gradient of one 3x3 convolution through the tensor-core wgrad kernel (test / building block).
- * x16: NHWC 16-bit input [n,h,w,x_cstride] (first cin channels; fmt_x 0 fp16 / 1 bf16); dy16_bf16: NHWC bf16 output
- * gradient [n,h,w,64] (first cout channels, cout <= 64). dw: OIHW fp32 [cout,cin,3,3]; db: [cout] or NULL. */
-size_t resr_conv3x3_wgrad_workspace_bytes(int n, int h, int w, int cin, int cout);
-int resr_conv3x3_wgrad(const void* x16, int x_cstride, int fmt_x, const void* dy16_bf16, int n, int h, int w, int cin,
-                       int cout, float* dw, float* db, void* workspace, size_t workspace_bytes, void* stream);
-
-/* The same gradients straight from NHWC bf16 operands (no channels-first copies): both operands are MN-major tcgen05
- * operands, pixel shifts are descriptor / TMA-coordinate shifts (csrc/wgrad_mn.cu). x_bf16: [n,h,w,x_cstride] (first cin
- * channels, cin <= 256); dy_bf16: [n,h,w,dy_cstride] (first cout channels, cout <= 192; when cout is not a multiple of 8
- * the channels up to the next multiple of 8 must be zero). No restriction on w. This is the kernel the bf16 training
- * recipe uses for every layer (autograd of model.py:75-79, 87-98). */
+/* Weight / bias gradient of one 3x3 convolution (test / building block) straight from NHWC bf16 operands: both operands
+ * are MN-major tcgen05 operands, pixel shifts are descriptor / TMA-coordinate shifts (csrc/wgrad_mn.cu).
+ * x_bf16: [n,h,w,x_cstride] (first cin channels, cin <= 256); dy_bf16: [n,h,w,dy_cstride] (first cout channels,
+ * cout <= 192; when cout is not a multiple of 8 the channels up to the next multiple of 8 must be zero). dw: OIHW fp32
+ * [cout,cin,3,3]; db: [cout] or NULL. No restriction on w. This is the kernel both training recipes use for every layer
+ * (autograd of model.py:75-79, 87-98). */
 size_t resr_conv3x3_wgrad_nhwc_workspace_bytes(void);
 int resr_conv3x3_wgrad_nhwc(const void* x_bf16, int x_cstride, const void* dy_bf16, int dy_cstride, int n, int h, int w,
                             int cin, int cout, float* dw, float* db, void* workspace, size_t workspace_bytes, void* stream);

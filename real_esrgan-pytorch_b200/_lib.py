@@ -162,14 +162,11 @@ SIGNATURES = {
                                              c_void_p, c_size_t, c_void_p]),
     "resr_generator_step_is_graph": (c_int, [c_void_p]),
     "resr_generator_backward": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_size_t, c_void_p]),
-    "resr_conv3x3_wgrad_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int, c_int]),
     "resr_generator_grad_buckets": (c_int, [c_void_p, c_int]),
     "resr_generator_wait_grad_bucket": (c_int, [c_void_p, c_int, c_void_p]),
     "resr_conv3x3_wgrad_nhwc_workspace_bytes": (c_size_t, []),
     "resr_conv3x3_wgrad_nhwc": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p,
                                         c_void_p, c_size_t, c_void_p]),
-    "resr_conv3x3_wgrad": (c_int, [c_void_p, c_int, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p,
-                                   c_void_p, c_size_t, c_void_p]),
     "resr_crop": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),
 }
 

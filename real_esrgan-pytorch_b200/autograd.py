@@ -40,8 +40,6 @@ class _GeneratorFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, gen, *params):
         n, _, h, w = x.shape
-        if w % 8 != 0 and gen.precision != "bf16":
-            raise _lib.ResrError(f"the fp16 training recipe needs W % 8 == 0 (got {w}); the bf16 recipe has no such limit")
         xc = x.detach().contiguous().float()
         gen._ensure_packed()
         y = torch.empty((n, 3, 4 * h, 4 * w), dtype=torch.float32, device=x.device)
@@ -92,8 +90,6 @@ def l1_loss_backward(gen, lr: torch.Tensor, hr: torch.Tensor, accumulate: bool =
     """Fused training step core: sr = G(lr); loss = mean|sr - hr|; d loss / d params. Returns (loss, sr, flat_grads);
     flat_grads (fp32, state_dict order) is also scattered into param.grad."""
     n, _, h, w = lr.shape
-    if w % 8 != 0 and gen.precision != "bf16":
-        raise _lib.ResrError(f"the fp16 training recipe needs W % 8 == 0 (got {w}); the bf16 recipe has no such limit")
     dev = lr.device
     xc = lr.detach().contiguous().float()
     hrc = hr.detach().contiguous().float()
@@ -119,8 +115,6 @@ class TrainStep:
     single NCCL all-reduce (data parallel, reference has none: SURVEY.md §2.1) before being scattered to param.grad."""
 
     def __init__(self, gen, n: int, h: int, w: int, device=None, process_group=None, world_size: int = 1):
-        if w % 8 != 0 and gen.precision != "bf16":
-            raise _lib.ResrError(f"the fp16 training recipe needs W % 8 == 0 (got {w}); the bf16 recipe has no such limit")
         self.gen, self.shape = gen, (n, h, w)
         dev = device or next(gen.parameters()).device
         self.lr = torch.zeros((n, 3, h, w), dtype=torch.float32, device=dev)

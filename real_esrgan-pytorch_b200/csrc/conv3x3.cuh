@@ -112,6 +112,12 @@ inline long long conv3x3_clusters(long long units, int cluster, int nslices, int
 }
 cudaError_t conv3x3_run(const ConvMaps& maps, const ConvArgs& args, const ConvLaunchCfg& cfg, int num_sms, cudaStream_t stream);
 
+// cuTensorMapEncodeTiled, looked up once through the runtime's driver entry point (null if the driver lacks it).
+typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
+                                    const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
+                                    CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+PFN_encodeTiled get_encode_fn();
+
 // Tensor maps. base: NHWC tensor [N,H,W,C].
 int conv3x3_make_tmap_act(CUtensorMap* out, const void* base, int N, int H, int W, int C, int mode, int BW, int BN,
                           int cvalid = 0);  // cvalid: channels the convolution reads (0 = all C)

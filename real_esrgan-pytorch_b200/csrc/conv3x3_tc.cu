@@ -353,11 +353,7 @@ void conv3x3_init_geometry(ConvArgs* a, int N, int H, int W, int cin, int mode) 
     a->tail_ksteps = r == 0 || r > 32 ? 4 : (r > 16 ? 2 : 1);
 }
 
-typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                    const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                    CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static PFN_encodeTiled get_encode_fn() {
+PFN_encodeTiled get_encode_fn() {
     static PFN_encodeTiled fn = nullptr;
     if (!fn) {
         void* p = nullptr;

@@ -1,7 +1,7 @@
 // Training path of the generator: forward that keeps every activation, L1 loss, and the full backward pass
-// (data gradients through the same tcgen05 convolution kernel with transposed weights, weight gradients through
-// wgrad_tc.cu). Reference: autograd of /root/reference/model.py:64-132, 206-275 and nn.L1Loss
-// (train_realesrnet.py:190-194, 383-388). See DESIGN.md §6.
+// (data gradients through the same tcgen05 convolution kernel with transposed weights, weight gradients through the
+// MN-major GEMM of wgrad_mn.cu in both recipes). Reference: autograd of /root/reference/model.py:64-132, 206-275 and
+// nn.L1Loss (train_realesrnet.py:190-194, 383-388). See DESIGN.md §6.
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
@@ -19,82 +19,19 @@ namespace resr {
 
 // ================================================================================================ small kernels
 
-// NHWC 16-bit [P][cstride], channels [c0, c0 + C) -> channels-first bf16 [Cpad][P]; rows C..Cpad-1 are zero-filled.
-// SHIFT3 additionally writes the copies shifted by one pixel along x (zero at the row ends),
-//     out[dx][c][n][y][x] = in[n][y][x - dx + 1][c]   (dx = 0, 1, 2; zero when x - dx + 1 is outside [0, W)),
-// because the weight-gradient kernel pairs X[.., x + dx - 1] with dY[.., x] and TMA cannot start a box at an odd 2-byte
-// offset of the innermost (pixel) dimension; and, when db is given, accumulates the bias gradient
-// db[c] += sum_p in[p][c] in the same pass (db zeroed by the caller).
-// One block = 32 channels x 256 pixels; all global traffic is 16-byte vectors (requires W % 8 == 0, c0 % 8 == 0,
-// cstride % 8 == 0).
-template <bool SHIFT3>
-__global__ void __launch_bounds__(256) nhwc16_to_cf_kernel(const uint16_t* __restrict__ in, int cstride, int c0, int C, int Cpad,
-                                                          size_t P, int W, int fmt_in, uint16_t* __restrict__ out,
-                                                          float* __restrict__ db) {
-    constexpr int kRow = 272;                   // halo pixel -1 at index 7, pixels 0..255 at 8..263, halo 256 at 264
-    __shared__ __align__(16) uint16_t tile[32][kRow];
-    const int cb = blockIdx.y * 32;
-    const long long p0 = static_cast<long long>(blockIdx.x) * 256;
-    for (int idx = threadIdx.x; idx < 258 * 4; idx += 256) {
-        const int px = idx >> 2, q = idx & 3;   // px 0..257 <-> pixel p0 - 1 + px
-        const long long p = p0 - 1 + px;
-        uint4 v = make_uint4(0u, 0u, 0u, 0u);
-        if (p >= 0 && p < static_cast<long long>(P) && cb + q * 8 < C)
-            v = *reinterpret_cast<const uint4*>(in + static_cast<size_t>(p) * cstride + c0 + cb + q * 8);
-        const uint32_t w4[4] = {v.x, v.y, v.z, v.w};
+// NHWC fp16 -> NHWC bf16 with the same channel stride, round to nearest even through fp32: the fp16 recipe's saved
+// activations as the X operand of the weight-gradient GEMM, which needs X and dY (bf16) in one format. n8: 16-byte vectors.
+__global__ void __launch_bounds__(256) fp16_to_bf16_kernel(const uint4* __restrict__ in, uint4* __restrict__ out, size_t n8) {
+    for (size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; i < n8; i += static_cast<size_t>(gridDim.x) * blockDim.x) {
+        uint4 v = in[i];
+        uint32_t* w = reinterpret_cast<uint32_t*>(&v);
 #pragma unroll
-        for (int j = 0; j < 8; ++j) {
-            uint16_t e = static_cast<uint16_t>(w4[j >> 1] >> ((j & 1) * 16));
-            if (fmt_in == 0) {  // fp16 -> bf16
-                const __half h = *reinterpret_cast<const __half*>(&e);
-                const __nv_bfloat16 bb = __float2bfloat16_rn(__half2float(h));
-                e = *reinterpret_cast<const uint16_t*>(&bb);
-            }
-            if (cb + q * 8 + j >= C) e = 0;
-            tile[q * 8 + j][7 + px] = e;
+        for (int j = 0; j < 4; ++j) {
+            const float2 f = __half22float2(*reinterpret_cast<const __half2*>(&w[j]));
+            const __nv_bfloat162 h = __floats2bfloat162_rn(f.x, f.y);
+            w[j] = *reinterpret_cast<const uint32_t*>(&h);
         }
-    }
-    __syncthreads();
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const size_t plane = static_cast<size_t>(Cpad) * P;
-    for (int c = warp; c < 32; c += 8) {
-        if (cb + c >= Cpad) break;
-        const long long p = p0 + 8 * lane;      // this lane's 8 pixels (never straddle an image row: W % 8 == 0)
-        const uint4 cur = *reinterpret_cast<const uint4*>(&tile[c][8 + 8 * lane]);
-        float bs = 0.f;
-        if (p < static_cast<long long>(P)) {
-            uint16_t* row = out + static_cast<size_t>(cb + c) * P + p;
-            if (!SHIFT3) {
-                *reinterpret_cast<uint4*>(row) = cur;
-            } else {
-                const uint32_t prev = *reinterpret_cast<const uint32_t*>(&tile[c][6 + 8 * lane]);   // pixels -2, -1
-                const uint32_t next = *reinterpret_cast<const uint32_t*>(&tile[c][16 + 8 * lane]);  // pixels 8, 9
-                const int x = static_cast<int>(p % W);
-                uint4 lo, hi;  // lo: out[dx=0][p + i] = in[p + i + 1];  hi: out[dx=2][p + i] = in[p + i - 1]
-                lo.x = __funnelshift_r(cur.x, cur.y, 16);
-                lo.y = __funnelshift_r(cur.y, cur.z, 16);
-                lo.z = __funnelshift_r(cur.z, cur.w, 16);
-                lo.w = __funnelshift_r(cur.w, next, 16);
-                hi.x = __funnelshift_r(prev, cur.x, 16);
-                hi.y = __funnelshift_r(cur.x, cur.y, 16);
-                hi.z = __funnelshift_r(cur.y, cur.z, 16);
-                hi.w = __funnelshift_r(cur.z, cur.w, 16);
-                if (x + 8 == W) lo.w &= 0x0000FFFFu;  // last pixel of an image row has no right neighbour
-                if (x == 0) hi.x &= 0xFFFF0000u;      // first pixel has no left neighbour
-                *reinterpret_cast<uint4*>(row) = lo;
-                *reinterpret_cast<uint4*>(row + plane) = cur;
-                *reinterpret_cast<uint4*>(row + 2 * plane) = hi;
-            }
-            if (SHIFT3 && db) {
-                const uint32_t w4[4] = {cur.x, cur.y, cur.z, cur.w};
-#pragma unroll
-                for (int j = 0; j < 4; ++j) bs += __uint_as_float(w4[j] << 16) + __uint_as_float(w4[j] & 0xFFFF0000u);
-            }
-        }
-        if (SHIFT3 && db) {
-            for (int o = 16; o > 0; o >>= 1) bs += __shfl_down_sync(0xffffffffu, bs, o);
-            if (lane == 0 && cb + c < C) atomicAdd(db + cb + c, bs);
-        }
+        out[i] = v;
     }
 }
 
@@ -258,8 +195,8 @@ static size_t up1k(size_t v) { return (v + 1023) / 1024 * 1024; }
 
 struct TrainWs {
     size_t xin, c[70], f[4], t1, t2, t3, t4, yraw;       // forward
-    size_t dycat[3], dbcat;
-    size_t g, dya, dyb, dx[3], dskip, biga, bigb, mida, midb, xt, dyt, partial, loss;  // backward
+    size_t dycat[3];
+    size_t g, dya, dyb, dx[3], dskip, biga, bigb, mida, midb, xbf16, partial, loss;  // backward
     size_t total;
 };
 
@@ -278,7 +215,6 @@ static TrainWs train_layout(size_t N, size_t H, size_t W, int num_sms) {
     L.yraw = take(16 * P * 3 * 4);
     L.g = take(P * 192 * 4);
     for (int i = 0; i < 3; ++i) L.dycat[i] = take(P * 192 * 2);
-    L.dbcat = take(192 * 4);
     L.dya = take(P * 64 * 2);
     L.dyb = take(P * 64 * 2);
     for (int i = 0; i < 3; ++i) L.dx[i] = take(P * 64 * 4);
@@ -287,12 +223,8 @@ static TrainWs train_layout(size_t N, size_t H, size_t W, int num_sms) {
     L.bigb = take(16 * P * 64 * 2);
     L.mida = take(4 * P * 64 * 2);
     L.midb = take(4 * P * 64 * 2);
-    L.xt = take(16 * P * 64 * 2 > P * 192 * 2 ? 16 * P * 64 * 2 : P * 192 * 2);
-    L.dyt = take(3 * 16 * P * 64 * 2);  // also holds the three 192-channel copies of a dense block's dYcat (3 * 192 * P)
-    {
-        const size_t pa = wgrad_partial_bytes(num_sms), pb = wgrad_mn_workspace_bytes(num_sms);
-        L.partial = take(pa > pb ? pa : pb);
-    }
+    L.xbf16 = take(16 * P * 64 * 2 > P * 192 * 2 ? 16 * P * 64 * 2 : P * 192 * 2);  // fp16 recipe: bf16 copy of a layer's X
+    L.partial = take(wgrad_mn_workspace_bytes(num_sms));
     L.loss = take(64);
     L.total = o;
     return L;
@@ -321,8 +253,7 @@ namespace {
 
 struct Bufs {
     uint16_t *dycat[3];
-    float* dbcat;
-    uint16_t *xin, *c[70], *t1, *t2, *t3, *t4, *dya, *dyb, *biga, *bigb, *mida, *midb, *xt, *dyt;
+    uint16_t *xin, *c[70], *t1, *t2, *t3, *t4, *dya, *dyb, *biga, *bigb, *mida, *midb, *xbf16;
     float *f[4], *yraw, *g, *dx[3], *dskip, *partial;
     double* loss;
 };
@@ -338,13 +269,12 @@ Bufs carve(void* ws, const TrainWs& L) {
     B.yraw = reinterpret_cast<float*>(b + L.yraw);
     B.g = reinterpret_cast<float*>(b + L.g);
     for (int i = 0; i < 3; ++i) B.dycat[i] = reinterpret_cast<uint16_t*>(b + L.dycat[i]);
-    B.dbcat = reinterpret_cast<float*>(b + L.dbcat);
     B.dya = reinterpret_cast<uint16_t*>(b + L.dya); B.dyb = reinterpret_cast<uint16_t*>(b + L.dyb);
     for (int i = 0; i < 3; ++i) B.dx[i] = reinterpret_cast<float*>(b + L.dx[i]);
     B.dskip = reinterpret_cast<float*>(b + L.dskip);
     B.biga = reinterpret_cast<uint16_t*>(b + L.biga); B.bigb = reinterpret_cast<uint16_t*>(b + L.bigb);
     B.mida = reinterpret_cast<uint16_t*>(b + L.mida); B.midb = reinterpret_cast<uint16_t*>(b + L.midb);
-    B.xt = reinterpret_cast<uint16_t*>(b + L.xt); B.dyt = reinterpret_cast<uint16_t*>(b + L.dyt);
+    B.xbf16 = reinterpret_cast<uint16_t*>(b + L.xbf16);
     B.partial = reinterpret_cast<float*>(b + L.partial);
     B.loss = reinterpret_cast<double*>(b + L.loss);
     return B;
@@ -426,14 +356,11 @@ int forward_train(resr_generator* g, const float* x, float* y, int N, int H, int
     return RESR_OK;
 }
 
-// weight + bias gradient of layer k. x16: NHWC input activations of the layer (first cin channels of a c_stride-wide
-// tensor, format fmt_x); dy16: NHWC bf16 output gradient (64-channel buffer). Both are transposed to channels-first.
-// The weight-gradient chain (transposes, split-K GEMM, reduction) of a layer only consumes the layer's dY and saved
-// input, nothing downstream on the data-gradient chain waits for it: it runs on a second stream (a parallel branch of
-// the captured graph) and fills the SMs the short data-gradient kernels leave idle. RESR_TRAIN_ONE_STREAM=1 disables it.
+// The weight-gradient chain of a layer (split-K GEMM, reduction) only consumes the layer's dY and saved input, nothing
+// downstream on the data-gradient chain waits for it: it runs on a second stream (a parallel branch of the captured
+// graph) and fills the SMs the short data-gradient kernels leave idle. The main stream serves if that stream cannot be
+// created.
 cudaStream_t wgrad_stream(resr_generator* g, cudaStream_t s) {
-    static const bool one = getenv("RESR_TRAIN_ONE_STREAM") != nullptr;
-    if (one) return s;
     if (!g->side_stream) {
         if (cudaStreamCreateWithFlags(&g->side_stream, cudaStreamNonBlocking) != cudaSuccess) { g->side_stream = nullptr; return s; }
         cudaEventCreateWithFlags(&g->ev_fork, cudaEventDisableTiming);
@@ -450,46 +377,39 @@ void fork_to(resr_generator* g, cudaStream_t s, cudaStream_t w) {
     cudaStreamWaitEvent(w, g->ev_fork, 0);
 }
 
-int layer_wgrad(resr_generator* g, int k, const uint16_t* x16, int x_cstride, int fmt_x, bool x_already_transposed, int xt_rows,
-                const uint16_t* dy16, int N, const Geo& q, const Bufs& B, float* grads, cudaStream_t s) {
+// X operand of the weight-gradient GEMM (wgrad_mn.cu), which reads X and dY in one format, bf16: the bf16 recipe's
+// activations in place, the fp16 recipe's converted into B.xbf16 on stream w. x16: NHWC [P][x_cstride].
+const uint16_t* wgrad_x(const resr_generator* g, const uint16_t* x16, size_t P, int x_cstride, const Bufs& B, cudaStream_t w) {
+    if (g->precision == 1) return x16;
+    const size_t n8 = P * x_cstride / 8;
+    fp16_to_bf16_kernel<<<egrid(n8), 256, 0, w>>>(reinterpret_cast<const uint4*>(x16), reinterpret_cast<uint4*>(B.xbf16), n8);
+    return B.xbf16;
+}
+
+// weight + bias gradient of layer k. x16: NHWC input activations of the layer (first cin channels of an x_cstride-wide
+// tensor, in the recipe's activation format); dy16: NHWC bf16 output gradient (64-channel buffer), which the MN-major
+// GEMM reads in place.
+int layer_wgrad(resr_generator* g, int k, const uint16_t* x16, int x_cstride, const uint16_t* dy16, int N, const Geo& q, const Bufs& B,
+                float* grads, cudaStream_t s) {
     const ConvSpec& c = table().c[k];
-    const size_t P = static_cast<size_t>(N) * q.H * q.W;
     cudaStream_t w = wgrad_stream(g, s);
     fork_to(g, s, w);  // dY of this layer (and everything before it) is complete on the main stream
-    if (g->precision == 1) {
-        // bf16 recipe: X and dY share one operand format, the MN-major kernel reads both NHWC buffers in place
-        WgradMnTable tb;
-        float* dw = grads + c.p_off;
-        for (int cs = 0; cs < 6; ++cs) {
-            tb.dw[cs] = dw; tb.db[cs] = dw + static_cast<size_t>(c.cout) * c.cin * 9;
-            tb.cin[cs] = c.cin; tb.cout[cs] = c.cout; tb.co_base[cs] = cs * 32;
-        }
-        const int dyc = (c.cout + 7) / 8 * 8 > 64 ? 64 : (c.cout + 7) / 8 * 8;
-        int units[2][3] = {{0, 0, 64}, {128, 0, 64}};
-        const int rc = wgrad_mn_launch(x16, x_cstride, c.cin, dy16, 64, dyc, N, q.H, q.W, units, c.cin > 128 ? 2 : 1, tb, true, B.partial,
-                                       g->num_sms, w);
-        if (rc != 0) return set_error(RESR_E_CUDA, "wgrad (nhwc) of layer %d failed (%d)", k, rc);
-        if (w != s) {  // the main stream overwrites this dY buffer two layers later: wait for its reader here
-            cudaEventRecord(g->ev_dy, w);
-            cudaStreamWaitEvent(s, g->ev_dy, 0);
-        }
-        return RESR_OK;
-    }
-    if (!x_already_transposed) {
-        xt_rows = (c.cin + 31) / 32 * 32;
-        nhwc16_to_cf_kernel<false><<<dim3(static_cast<unsigned>((P + 255) / 256), xt_rows / 32), 256, 0, w>>>(x16, x_cstride, 0, c.cin, xt_rows, P, q.W,
-                                                                                                               fmt_x, B.xt, nullptr);
-    }
-    const int dy_rows = (c.cout + 31) / 32 * 32;
+    const uint16_t* x = wgrad_x(g, x16, static_cast<size_t>(N) * q.H * q.W, x_cstride, B, w);
+    WgradMnTable tb;
     float* dw = grads + c.p_off;
-    float* db = dw + static_cast<size_t>(c.cout) * c.cin * 9;  // zeroed with the whole gradient vector at the start of the backward
-    nhwc16_to_cf_kernel<true><<<dim3(static_cast<unsigned>((P + 255) / 256), dy_rows / 32), 256, 0, w>>>(dy16, 64, 0, c.cout, dy_rows, P, q.W, 1, B.dyt, db);
-    if (w != s) {  // the main stream may overwrite the dY buffer once its channels-first copies exist
+    for (int cs = 0; cs < 6; ++cs) {
+        tb.dw[cs] = dw; tb.db[cs] = dw + static_cast<size_t>(c.cout) * c.cin * 9;
+        tb.cin[cs] = c.cin; tb.cout[cs] = c.cout; tb.co_base[cs] = cs * 32;
+    }
+    const int dyc = (c.cout + 7) / 8 * 8 > 64 ? 64 : (c.cout + 7) / 8 * 8;
+    int units[2][3] = {{0, 0, 64}, {128, 0, 64}};
+    const int rc = wgrad_mn_launch(x, x_cstride, c.cin, dy16, 64, dyc, N, q.H, q.W, units, c.cin > 128 ? 2 : 1, tb, true, B.partial,
+                                   g->num_sms, w);
+    if (rc != 0) return set_error(RESR_E_CUDA, "wgrad of layer %d failed (%d)", k, rc);
+    if (w != s) {  // the main stream overwrites this dY buffer two layers later: wait for its reader here
         cudaEventRecord(g->ev_dy, w);
         cudaStreamWaitEvent(s, g->ev_dy, 0);
     }
-    const int rc = wgrad_launch(B.xt, xt_rows, B.dyt, dy_rows, N, q.H, q.W, c.cin, c.cout, B.partial, dw, nullptr, g->num_sms, w);
-    if (rc != 0) return set_error(RESR_E_CUDA, "wgrad of layer %d failed (%d)", k, rc);
     return RESR_OK;
 }
 
@@ -521,39 +441,41 @@ int backward_common(resr_generator* g, float* grads, int N, int H, int W, const 
     const size_t P = static_cast<size_t>(N) * H * W;
     ensure_transposed_packs(g, s, true);
     g->ev_dyc_valid[0] = g->ev_dyc_valid[1] = g->ev_dyc_valid[2] = false;
-    cudaMemsetAsync(grads, 0, table().n_params * sizeof(float), s);  // bias gradients are accumulated with atomics
+    // every element is written by one of the weight-gradient reductions below; cleared first so that none can carry the
+    // previous step's value
+    cudaMemsetAsync(grads, 0, table().n_params * sizeof(float), s);
     cudaMemsetAsync(B.dya, 0, P * 64 * 2, s);
     cudaMemsetAsync(B.dyb, 0, P * 64 * 2, s);
     const int kConv2 = 346, kUp1 = 347, kUp2 = 348, kConv3 = 349, kConv4 = 350;
 
     // ---- tail (model.py:264-270 backwards)
-    RESR_TRY(layer_wgrad(g, kConv4, B.t4, 64, g->precision, false, 0, B.biga, N, g2, B, grads, s));
+    RESR_TRY(layer_wgrad(g, kConv4, B.t4, 64, B.biga, N, g2, B, grads, s));
     {   // d(T4) masked by LeakyReLU'(conv3 out) -> conv3's dY
         ConvIO io = bwd_io(g, kConv4);
         io.in16 = B.biga; io.out16 = B.bigb; io.mask16 = B.t4;
         RESR_TRY(launch_conv_io(g, g2, N, io, s));
     }
-    RESR_TRY(layer_wgrad(g, kConv3, B.t3, 64, g->precision, false, 0, B.bigb, N, g2, B, grads, s));
+    RESR_TRY(layer_wgrad(g, kConv3, B.t3, 64, B.bigb, N, g2, B, grads, s));
     {
         ConvIO io = bwd_io(g, kConv3);
         io.in16 = B.bigb; io.out16 = B.biga; io.mask16 = B.t3;
         RESR_TRY(launch_conv_io(g, g2, N, io, s));
     }
-    RESR_TRY(layer_wgrad(g, kUp2, B.t2, 64, g->precision, false, 0, B.biga, N, g2, B, grads, s));
+    RESR_TRY(layer_wgrad(g, kUp2, B.t2, 64, B.biga, N, g2, B, grads, s));
     {   // d(T2) at 4x, masked by LeakyReLU'(up1 out) (T2 holds its upsampled copy), then the 2x2 sum of nearest x2
         ConvIO io = bwd_io(g, kUp2);
         io.in16 = B.biga; io.out16 = B.bigb; io.mask16 = B.t2;
         RESR_TRY(launch_conv_io(g, g2, N, io, s));
         sum2x2_kernel<<<egrid(4 * P * 32), 256, 0, s>>>(B.bigb, nullptr, B.mida, N, 2 * H, 2 * W);
     }
-    RESR_TRY(layer_wgrad(g, kUp1, B.t1, 64, g->precision, false, 0, B.mida, N, g1, B, grads, s));
+    RESR_TRY(layer_wgrad(g, kUp1, B.t1, 64, B.mida, N, g1, B, grads, s));
     {   // d(T1) at 2x (no activation on the skip sum), 2x2 sum -> d(out) at LR: fp32 (skip branch) + bf16 (conv2's dY)
         ConvIO io = bwd_io(g, kUp1);
         io.in16 = B.mida; io.out16 = B.midb;
         RESR_TRY(launch_conv_io(g, g1, N, io, s));
         sum2x2_kernel<<<egrid(P * 32), 256, 0, s>>>(B.midb, B.dskip, B.dya, N, H, W);
     }
-    RESR_TRY(layer_wgrad(g, kConv2, B.c[69], 192, g->precision, false, 0, B.dya, N, g0, B, grads, s));
+    RESR_TRY(layer_wgrad(g, kConv2, B.c[69], 192, B.dya, N, g0, B, grads, s));
     {   // d(trunk output), fp32, and its bf16 copy x 0.2 x 0.2 = dY5 of the last dense block (trunk.22.rdb3)
         ConvIO io = bwd_io(g, kConv2);
         io.in16 = B.dya; io.outf = B.dx[0];
@@ -612,52 +534,28 @@ int backward_common(resr_generator* g, float* grads, int N, int H, int W, const 
                 }
                 RESR_TRY(launch_conv_io(g, g0, N, io, s));
             }
-            {   // weight + bias gradients of the five layers (side stream): dYcat is complete once conv2's launch is done
+            {   // weight + bias gradients of the five layers (side stream): dYcat is complete once conv2's launch is done.
+                // ONE MN-major GEMM straight from the concat buffer and dYcat' (no transposed copies).
+                // Units (128 ci x n co'): [0,128) x [0,128), [0,128) x [128,192), [128,192(+64 zero rows)) x [0,128);
+                // the reduction keeps ci < cin of the layer owning each 32-channel slice of dYcat'.
                 fork_to(g, s, wst);
-                if (g->precision == 1) {
-                    // bf16 recipe: ONE MN-major GEMM straight from the concat buffer and dYcat' (no transposed copies).
-                    // Units (128 ci x n co'): [0,128) x [0,128), [0,128) x [128,192), [128,192(+64 zero rows)) x [0,128);
-                    // the reduction keeps ci < cin of the layer owning each 32-channel slice of dYcat'.
-                    WgradMnTable tb;
-                    for (int cs = 0; cs < 6; ++cs) {
-                        const int kl = 1 + 5 * r + (cs < 2 ? 4 : 5 - cs);
-                        const ConvSpec& c = table().c[kl];
-                        tb.dw[cs] = grads + c.p_off;
-                        tb.db[cs] = grads + c.p_off + static_cast<size_t>(c.cout) * c.cin * 9;
-                        tb.cin[cs] = c.cin; tb.cout[cs] = c.cout;
-                        tb.co_base[cs] = cs < 2 ? cs * 32 : 0;
-                    }
-                    const int units[3][3] = {{0, 0, 128}, {0, 128, 64}, {128, 0, 128}};
-                    const int rc = wgrad_mn_launch(B.c[r], 192, 192, dyc, 192, 192, N, H, W, units, 3, tb, true, B.partial, g->num_sms, wst);
-                    if (rc != 0) return set_error(RESR_E_CUDA, "dense-block wgrad (nhwc) failed (%d)", rc);
-                    if (wst != s) {
-                        cudaEventRecord(g->ev_dyc[r % 3], wst);
-                        g->ev_dyc_valid[r % 3] = true;
-                    }
-                    continue;
-                }
-                const dim3 tg(static_cast<unsigned>((P + 255) / 256), 6);
-                nhwc16_to_cf_kernel<false><<<tg, 256, 0, wst>>>(B.c[r], 192, 0, 192, 192, P, W, 0, B.xt, nullptr);
-                cudaMemsetAsync(B.dbcat, 0, 192 * sizeof(float), wst);
-                nhwc16_to_cf_kernel<true><<<tg, 256, 0, wst>>>(dyc, 192, 0, 192, 192, P, W, 1, B.dyt, B.dbcat);
-                if (wst != s) {
-                    cudaEventRecord(g->ev_dyc[r % 3], wst);
-                    g->ev_dyc_valid[r % 3] = true;
-                }
-                WgradRdbTable tb;
+                const uint16_t* x = wgrad_x(g, B.c[r], P, 192, B, wst);
+                WgradMnTable tb;
                 for (int cs = 0; cs < 6; ++cs) {   // slices of dYcat': conv5 (two halves), conv4, conv3, conv2, conv1
                     const int kl = 1 + 5 * r + (cs < 2 ? 4 : 5 - cs);
                     const ConvSpec& c = table().c[kl];
                     tb.dw[cs] = grads + c.p_off;
-                    tb.cin[cs] = c.cin;
+                    tb.db[cs] = grads + c.p_off + static_cast<size_t>(c.cout) * c.cin * 9;
+                    tb.cin[cs] = c.cin; tb.cout[cs] = c.cout;
                     tb.co_base[cs] = cs < 2 ? cs * 32 : 0;
-                    tb.db[cs] = grads + c.p_off + static_cast<size_t>(c.cout) * c.cin * 9 + tb.co_base[cs];
                 }
-                tb.dbcat = B.dbcat;
-                // (giving the two chains disjoint SM subsets instead of letting them interleave was tried: 22.6 - 24.4 ms
-                // against 21.5 ms, profiles/r02_train_sm_partition_ab.txt)
-                const int rc = wgrad_launch_rdb(B.xt, B.dyt, N, H, W, B.partial, tb, g->num_sms, wst);
+                const int units[3][3] = {{0, 0, 128}, {0, 128, 64}, {128, 0, 128}};
+                const int rc = wgrad_mn_launch(x, 192, 192, dyc, 192, 192, N, H, W, units, 3, tb, true, B.partial, g->num_sms, wst);
                 if (rc != 0) return set_error(RESR_E_CUDA, "dense-block wgrad failed (%d)", rc);
+                if (wst != s) {
+                    cudaEventRecord(g->ev_dyc[r % 3], wst);
+                    g->ev_dyc_valid[r % 3] = true;
+                }
             }
         }
         for (int bi = 0; bi < 3; ++bi)   // every gradient from RRDB i upwards has been enqueued on the weight-gradient stream
@@ -666,8 +564,8 @@ int backward_common(resr_generator* g, float* grads, int N, int H, int W, const 
     }
     // ---- conv1 (model.py:258): dY = d(trunk input) + d(skip)
     scale_f32_to_bf16_kernel<<<egrid(P * 64), 256, 0, s>>>(B.dx[0], 1.f, B.dskip, 1.f, B.dya, P * 64);
-    RESR_TRY(layer_wgrad(g, 0, B.xin, 64, g->precision, false, 0, B.dya, N, g0, B, grads, s));
-    if (g->side_stream && wgrad_stream(g, s) != s) {  // join: the gradient vector is complete when the main stream continues
+    RESR_TRY(layer_wgrad(g, 0, B.xin, 64, B.dya, N, g0, B, grads, s));
+    if (g->side_stream) {  // join: the gradient vector is complete when the main stream continues
         cudaEventRecord(g->ev_join, g->side_stream);
         cudaStreamWaitEvent(s, g->ev_join, 0);
     }
@@ -679,8 +577,6 @@ int backward_common(resr_generator* g, float* grads, int N, int H, int W, const 
 int check_train_args(resr_generator_t* g, int n, int h, int w, void* ws, size_t ws_bytes) {
     if (!g || !ws) return set_error(RESR_E_INVALID, "null argument");
     if (n <= 0 || h <= 0 || w <= 0) return set_error(RESR_E_INVALID, "bad shape");
-    if (g->precision != 1 && w % 8 != 0)
-        return set_error(RESR_E_INVALID, "the fp16 training recipe needs W %% 8 == 0 (channels-first TMA strides), got %d; the bf16 recipe has no such limit", w);
     if (!g->loaded || !g->flat_params) return set_error(RESR_E_INVALID, "resr_generator_load_params has not been called");
     if (ws_bytes < resr_generator_train_workspace_bytes(n, h, w)) return set_error(RESR_E_NOMEM, "training workspace too small");
     if ((reinterpret_cast<uintptr_t>(ws) & 1023) != 0) return set_error(RESR_E_INVALID, "workspace must be 1024-byte aligned");
@@ -795,29 +691,6 @@ int resr_generator_wait_grad_bucket(resr_generator_t* g, int bucket, void* strea
     return RESR_OK;
 }
 
-int resr_conv3x3_wgrad(const void* x16, int x_cstride, int fmt_x, const void* dy16_bf16, int n, int h, int w, int cin, int cout,
-                       float* dw, float* db, void* workspace, size_t workspace_bytes, void* stream) {
-    if (!x16 || !dy16_bf16 || !dw || !workspace) return set_error(RESR_E_INVALID, "null argument");
-    if (w % 8 != 0 || cout > 64 || cin > x_cstride) return set_error(RESR_E_INVALID, "unsupported wgrad shape");
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
-    const size_t P = static_cast<size_t>(n) * h * w;
-    const int xr = (cin + 31) / 32 * 32, yr = (cout + 31) / 32 * 32;
-    const size_t need = up1k(P * xr * 2) + up1k(3 * P * yr * 2) + wgrad_partial_bytes(160);
-    if (workspace_bytes < need) return set_error(RESR_E_NOMEM, "wgrad workspace too small (need %zu)", need);
-    uint16_t* xt = static_cast<uint16_t*>(workspace);
-    uint16_t* dyt = reinterpret_cast<uint16_t*>(static_cast<uint8_t*>(workspace) + up1k(P * xr * 2));
-    float* partial = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(dyt) + up1k(3 * P * yr * 2));
-    nhwc16_to_cf_kernel<false><<<dim3(static_cast<unsigned>((P + 255) / 256), xr / 32), 256, 0, s>>>(static_cast<const uint16_t*>(x16), x_cstride, 0, cin, xr, P, w, fmt_x, xt, nullptr);
-    if (db) cudaMemsetAsync(db, 0, cout * sizeof(float), s);
-    nhwc16_to_cf_kernel<true><<<dim3(static_cast<unsigned>((P + 255) / 256), yr / 32), 256, 0, s>>>(static_cast<const uint16_t*>(dy16_bf16), 64, 0, cout, yr, P, w, 1, dyt, db);
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const int rc = wgrad_launch(xt, xr, dyt, yr, n, h, w, cin, cout, partial, dw, nullptr, sms, s);
-    if (rc != 0) return set_error(RESR_E_CUDA, "wgrad failed (%d)", rc);
-    return RESR_OK;
-}
-
 size_t resr_conv3x3_wgrad_nhwc_workspace_bytes(void) { return wgrad_mn_workspace_bytes(160) + 1024; }
 
 int resr_conv3x3_wgrad_nhwc(const void* x_bf16, int x_cstride, const void* dy_bf16, int dy_cstride, int n, int h, int w, int cin, int cout,
@@ -847,12 +720,6 @@ int resr_conv3x3_wgrad_nhwc(const void* x_bf16, int x_cstride, const void* dy_bf
                                    n, h, w, units, nu, tb, db != nullptr, static_cast<float*>(workspace), sms, static_cast<cudaStream_t>(stream));
     if (rc != 0) return set_error(RESR_E_CUDA, "wgrad (nhwc) failed (%d)", rc);
     return RESR_OK;
-}
-
-size_t resr_conv3x3_wgrad_workspace_bytes(int n, int h, int w, int cin, int cout) {
-    const size_t P = static_cast<size_t>(n) * h * w;
-    const int xr = (cin + 31) / 32 * 32, yr = (cout + 31) / 32 * 32;
-    return up1k(P * xr * 2) + up1k(3 * P * yr * 2) + wgrad_partial_bytes(160);
 }
 
 }  // extern "C"

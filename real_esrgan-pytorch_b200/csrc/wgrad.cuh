@@ -1,4 +1,5 @@
-// Internal interface of the tensor-core weight-gradient kernel (wgrad_tc.cu).
+// Internal interface of the tensor-core weight-gradient kernel (wgrad_mn.cu): operands straight from the NHWC buffers,
+// one 16-bit format (bf16) for X and dY.
 #pragma once
 #include <cstddef>
 #include <cstdint>
@@ -6,41 +7,6 @@
 
 namespace resr {
 
-struct WgradArgs {
-    int N, H, W;
-    int cin, cout;
-    int n_mb;             // input-channel blocks of 128
-    int n_cs;             // output-channel slices of 32
-    int segs_per_row;     // ceil(W / 64)
-    long long kstages_total;  // N * H * segs_per_row (one stage = 64 pixels of one row)
-    float* partial;       // [nsplit][n_mb][n_cs][3 dy][128 ci][96 = (dx, co)] fp32
-    int nstages;
-    int dy_rows;          // channel rows of one shifted copy of dY^T
-    int nunits;           // > 0: explicit (ci block, co slice) list instead of the full n_mb x n_cs grid
-    unsigned char unit_mb[16], unit_cs[16];
-};
-
-// One dense block at once: the five layers share X (the 192-channel concat buffer) and their output gradients sit side by
-// side in one 192-channel buffer [dY1 | dY2 | dY3 | dY4 | dY5], so ONE split-K GEMM X^T x dYcat yields all five weight
-// gradients; slice cs (32 output-gradient channels) belongs to layer `layer[cs]`.
-struct WgradRdbTable {
-    float* dw[6];      // OIHW gradient of the layer that owns slice cs
-    float* db[6];      // its bias gradient (first element of the slice)
-    int cin[6];        // the layer's input channels (rows >= cin are not part of that layer)
-    int co_base[6];    // first output channel of the slice inside its layer
-    const float* dbcat;  // [192] bias gradients of the concatenated buffer (from the transpose pass)
-};
-
-size_t wgrad_partial_bytes(int num_sms);
-
-// xt: channels-first bf16 activations [x_channels][N][H][W]; dyt: three x-shifted channels-first bf16 copies of the
-// output gradient [3][dy_channels][N][H][W] (dy_channels >= ceil(cout/32)*32; copy dx holds dY[.., x - dx + 1]). dw: OIHW fp32 [cout][cin][3][3]; db: [cout] or null.
-int wgrad_launch_rdb(const uint16_t* xt, const uint16_t* dyt, int N, int H, int W, float* partial, const WgradRdbTable& tb,
-                     int num_sms, cudaStream_t s);
-int wgrad_launch(const uint16_t* xt, int x_channels, const uint16_t* dyt, int dy_channels, int N, int H, int W, int cin, int cout,
-                 float* partial, float* dw, float* db, int num_sms, cudaStream_t s);
-
-// ---- MN-major variant (wgrad_mn.cu): operands straight from the NHWC buffers, one 16-bit format (bf16) for X and dY
 static constexpr int kMnMaxKinds = 12;
 struct WgradMnKind { int ci0, co0, n, dy, cta0, nsplit; };   // unit (128 input channels from ci0) x (n = 64 / 128 dY channels from co0), one dy
 struct WgradMnArgs {

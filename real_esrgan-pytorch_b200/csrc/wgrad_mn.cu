@@ -16,7 +16,7 @@
 // A CTA owns one unit (ci block, co chunk), ONE dy, and a contiguous range of pixel stages (split-K); its three
 // accumulators go to a partial buffer and wgrad_mn_reduce_kernel sums the splits into the OIHW gradients of the layers
 // that own the channel slices (a dense block's five layers share X and sit side by side in dYcat', train.cu).
-// Requires X and dY in ONE 16-bit format (bf16 here: the bf16 recipe of the training path).
+// Requires X and dY in ONE 16-bit format, bf16 (train.cu converts the fp16 recipe's saved activations first).
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -251,24 +251,10 @@ __global__ void __launch_bounds__(256) wgrad_mn_reduce_kernel(const WgradMnArgs 
     }
 }
 
-typedef CUresult (*PFN_encodeTiledMn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                      const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                      CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static PFN_encodeTiledMn mn_encode_fn() {
-    static PFN_encodeTiledMn fn = nullptr;
-    if (!fn) {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<PFN_encodeTiledMn>(p);
-    }
-    return fn;
-}
-
 // NHWC 16-bit tensor [N][H][W][cstride], channels [0, C) visible (the rest of a 64-channel box is zero-filled);
 // box = 64 channels x `rows` pixels of one image row.
 static int make_nhwc_map(CUtensorMap* out, const void* base, int C, int cstride, int N, int H, int W, int rows) {
-    PFN_encodeTiledMn enc = mn_encode_fn();
+    PFN_encodeTiled enc = get_encode_fn();
     if (!enc) return -1;
     const cuuint64_t dims[4] = {static_cast<cuuint64_t>(C), static_cast<cuuint64_t>(W), static_cast<cuuint64_t>(H), static_cast<cuuint64_t>(N)};
     const cuuint64_t strides[3] = {static_cast<cuuint64_t>(cstride) * 2, static_cast<cuuint64_t>(W) * cstride * 2,

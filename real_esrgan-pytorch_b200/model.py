@@ -175,10 +175,11 @@ class Generator(nn.Module):
 
     def set_precision(self, precision: str):
         """Recipe of the forward and of the training path: "fp16" (default: fp16 tensor-core operands, the trunk's residual
-        stream is the fp16 conv input; training keeps fp16 activations + bf16 gradients and needs W % 8 == 0) or "bf16"
-        (BASELINE.json north_star: bf16 operands and activations + fp32 masters of the residual stream; training keeps bf16
-        activations and gradients and takes its weight gradients straight from the NHWC buffers: 27 % faster per step, no
-        shape rule). Both run at the same tensor-core rate; fp16 is ~2-3x closer to the fp32 reference."""
+        stream is the fp16 conv input; training keeps fp16 activations + bf16 gradients and takes its weight gradients
+        from a bf16 copy of each layer's input) or "bf16" (BASELINE.json north_star: bf16 operands and activations + fp32
+        masters of the residual stream; training keeps bf16 activations and gradients and takes its weight gradients
+        straight from the NHWC buffers, faster per step). Neither has a shape rule. Both run at the same tensor-core
+        rate; fp16 is ~2-3x closer to the fp32 reference."""
         if precision not in _PRECISIONS:
             raise ValueError(f"precision must be one of {sorted(_PRECISIONS)}")
         if precision != self._precision:

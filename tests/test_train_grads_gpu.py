@@ -111,9 +111,9 @@ def pair_policy(request):
     lib.resr_set_conv_pair_policy(prev)
 
 
-SHAPES = [(1, 3, 16, 24), (2, 3, 16, 64), (3, 3, 5, 8), (1, 3, 1, 8), (1, 3, 9, 136)]
-BF16_SHAPES = SHAPES + [(2, 3, 7, 13), (1, 3, 3, 257)]  # W % 8 != 0: the fp16 recipe refuses these (test_train_gpu.py)
-CASES = [("fp16", s) for s in SHAPES] + [("bf16", s) for s in BF16_SHAPES]
+SHAPES = [(1, 3, 16, 24), (2, 3, 16, 64), (3, 3, 5, 8), (1, 3, 1, 8), (1, 3, 9, 136), (2, 3, 7, 13), (1, 3, 3, 257)]
+# every shape in both recipes; the fp16 cases with W % 8 != 0 come last so that each earlier case keeps its test id
+CASES = [("fp16", s) for s in SHAPES[:5]] + [("bf16", s) for s in SHAPES] + [("fp16", s) for s in SHAPES[5:]]
 
 
 @pytest.mark.parametrize("pair_policy", [1, 2], indirect=True)
@@ -121,7 +121,7 @@ CASES = [("fp16", s) for s in SHAPES] + [("bf16", s) for s in BF16_SHAPES]
 def test_l1_gradients_per_tensor_vs_float64(oracle, precision, shape, pair_policy):
     """The fused training step (autograd.l1_loss_backward: resr_generator_forward_train + resr_generator_backward_l1)."""
     import resr_b200
-    case = (BF16_SHAPES.index(shape), shape, "l1")
+    case = (SHAPES.index(shape), shape, "l1")
     sd = oracle.state_dict(case[0])
     x, hr = _inputs(case)
     g = _generator(sd, precision)

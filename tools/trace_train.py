@@ -25,14 +25,14 @@ print("streams", streams)
 # overlap between conv kernels and wgrad kernels
 import bisect
 conv = [(e["ts"], e["ts"] + e["dur"]) for e in ev if "conv3x3" in e["name"]]
-wg = [(e["ts"], e["ts"] + e["dur"]) for e in ev if ("wgrad_tc" in e["name"] or "wgrad_mn_kernel" in e["name"])]
+wg = [(e["ts"], e["ts"] + e["dur"]) for e in ev if "wgrad_mn_kernel" in e["name"]]
 ov = 0.0
 for a0, a1 in wg:
     for b0, b1 in conv:
         if b0 >= a1: break
         if b1 <= a0: continue
         ov += min(a1, b1) - max(a0, b0)
-print(f"wgrad_tc total {sum(b-a for a,b in wg)/1e3:.2f} ms, conv total {sum(b-a for a,b in conv)/1e3:.2f} ms, overlapped {ov/1e3:.2f} ms")
+print(f"wgrad total {sum(b-a for a,b in wg)/1e3:.2f} ms, conv total {sum(b-a for a,b in conv)/1e3:.2f} ms, overlapped {ov/1e3:.2f} ms")
 # print a window of the backward timeline
 mid = len(ev) // 2
 t0 = ev[mid]["ts"]
