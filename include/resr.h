@@ -433,6 +433,35 @@ int resr_adam_ema_step(float* params, const float* grads, float* exp_avg, float*
                        float lr, float beta1, float beta2, float eps, long long step, float ema_decay, float grad_scale,
                        void* stream);
 
+/* ---- VGG19 content loss of the RealESRGAN generator step (ContentLoss, model.py:278-335; train_realesrgan.py:473-487) -----
+ * losses[k] = mean |F_k(Normalize(sr)) - F_k(Normalize(gt))| for each requested node k, F_k = vgg19().features up to
+ * features.<node> as create_feature_extractor returns it: the conv output, rewritten by the in-place ReLU that follows it
+ * unless it is the deepest requested node. Weights are frozen; the backward gives d/d sr only.
+ *
+ * resr_vgg_create takes the node list as features indices (host; any of 0, 2, 5, 7, 10, 12, 14, 16, 19, 21, 23, 25, 28,
+ * 30, 32, 34, no repeats; losses come out in this order) and Normalize's mean / std (host, 3 floats each). It allocates
+ * nothing on the device. resr_vgg_load_params packs the 16 convolutions from one flat fp32 device vector of
+ * resr_vgg_num_params() (20,024,384) values: features.{0,2,...,34}.weight then .bias, torchvision order; it needs an sm_100a
+ * device (RESR_E_CUDA otherwise) and binds the handle to the current device. Convolutions past the deepest node never run.
+ *
+ * resr_vgg_forward: sr, gt [n,3,h,w] fp32 NCHW; losses: device fp32 [count]. SR and GT run as one 2n batch; the workspace
+ * (resr_vgg_workspace_bytes, 1024-byte aligned) keeps the activations the backward needs. The sums are fp64 in a fixed
+ * order: two identical calls give identical bits. h and w must leave at least one pixel at the deepest node (2x2 / stride 2
+ * floor pooling); resr_vgg_workspace_bytes returns 0 for a shape that does not.
+ * resr_vgg_backward: grad_losses (device fp32 [count], read on the device: no host sync) -> grad_sr fp32 NCHW [n,3,h,w].
+ * It needs the workspace and shape of the handle's last forward; anything else is RESR_E_INVALID.
+ * Every argument is checked on the host before any device work; a bad one returns RESR_E_INVALID. */
+typedef struct resr_vgg resr_vgg_t;
+size_t resr_vgg_num_params(void);
+int resr_vgg_create(resr_vgg_t** out, const int* features_host, int count, const float* mean_host, const float* std_host);
+void resr_vgg_destroy(resr_vgg_t* v);
+int resr_vgg_load_params(resr_vgg_t* v, const float* flat_params, void* stream);
+size_t resr_vgg_workspace_bytes(const resr_vgg_t* v, int n, int h, int w);
+int resr_vgg_forward(resr_vgg_t* v, const float* sr, const float* gt, float* losses, int n, int h, int w, void* workspace,
+                     size_t workspace_bytes, void* stream);
+int resr_vgg_backward(resr_vgg_t* v, const float* grad_losses, float* grad_sr, int n, int h, int w, void* workspace,
+                      size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

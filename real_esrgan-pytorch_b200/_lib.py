@@ -168,6 +168,13 @@ SIGNATURES = {
     "resr_conv3x3_wgrad_nhwc": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p,
                                         c_void_p, c_size_t, c_void_p]),
     "resr_crop": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),
+    "resr_vgg_num_params": (c_size_t, []),
+    "resr_vgg_create": (c_int, [POINTER(c_void_p), POINTER(c_int), c_int, POINTER(c_float), POINTER(c_float)]),
+    "resr_vgg_destroy": (None, [c_void_p]),
+    "resr_vgg_load_params": (c_int, [c_void_p, c_void_p, c_void_p]),
+    "resr_vgg_workspace_bytes": (c_size_t, [c_void_p, c_int, c_int, c_int]),
+    "resr_vgg_forward": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_size_t, c_void_p]),
+    "resr_vgg_backward": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_size_t, c_void_p]),
 }
 
 _lib = None

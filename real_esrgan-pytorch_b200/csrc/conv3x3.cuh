@@ -75,6 +75,9 @@ struct ConvArgs {
     int vmask_words;
     int vmask_shift;            // this layer's resolution: pixel (x, y) is valid iff LR bit (x >> shift, y >> shift) is set;
                                 // every output of an invalid pixel is written as 0, so a zero gutter between images stays zero
+    // ---- VGG19 content loss (vgg.cu); zero everywhere else
+    int relu;                   // v = max(v, 0) where `lrelu` applies LeakyReLU 0.2 (before every output)
+    int mask16_relu;            // mask16 is ReLU' (v *= act > 0 ? 1 : 0) instead of LeakyReLU' 0.2
 };
 
 // Fills the launch geometry of an N x H x W convolution: N / H / W, the lane split BW x BN, mode (-1: automatic, i.e. 0

@@ -234,6 +234,10 @@ __device__ __forceinline__ void epi_pass(const ConvArgs& a, const CUtensorMap* t
             val[2 * i + 1] = fmaxf(val[2 * i + 1], t.y);
         }
     }
+    if (a.relu) {
+#pragma unroll
+        for (int i = 0; i < W; ++i) val[i] = fmaxf(val[i], 0.f);
+    }
     if (MASKED && !p.inside) {   // gutter / canvas margin: 0 in every output, as the zero padding around an image
 #pragma unroll
         for (int i = 0; i < W; ++i) val[i] = 0.f;
@@ -257,7 +261,7 @@ __device__ __forceinline__ void epi_pass(const ConvArgs& a, const CUtensorMap* t
             *reinterpret_cast<float4*>(tileR + m * 128 + ((i ^ (m & 7)) << 4)) =
                 make_float4(val[4 * i], val[4 * i + 1], val[4 * i + 2], val[4 * i + 3]);
     }
-    if (use_o16 && a.mask16) {  // LeakyReLU backward: slope 1 where the saved activation is > 0, else 0.2
+    if (use_o16 && a.mask16) {  // LeakyReLU backward: slope 1 where the saved activation is > 0, else 0.2 (0: ReLU)
         const uint4* mk = reinterpret_cast<const uint4*>(static_cast<const uint16_t*>(a.mask16) + p.pix * a.mask16_cstride +
                                                          a.mask16_choff + ls * W);
 #pragma unroll
@@ -268,7 +272,7 @@ __device__ __forceinline__ void epi_pass(const ConvArgs& a, const CUtensorMap* t
             for (int e = 0; e < 8; ++e) {
                 const uint32_t h16 = (w4[e >> 1] >> ((e & 1) * 16)) & 0xFFFFu;
                 const bool pos = ((h16 & 0x8000u) == 0) && ((h16 & 0x7FFFu) != 0);
-                if (!pos) val[8 * i + e] = __fmul_rn(val[8 * i + e], 0.2f);
+                if (!pos) val[8 * i + e] = a.mask16_relu ? 0.f : __fmul_rn(val[8 * i + e], 0.2f);
             }
         }
     }

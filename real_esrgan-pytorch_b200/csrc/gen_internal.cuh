@@ -136,6 +136,26 @@ struct resr_generator {
 
 namespace resr {
 int grid_for(size_t total, int block);
+
+// One convolution of the training path (train.cu) or of the VGG19 content loss (vgg.cu), launched with tensor maps encoded
+// per call: what goes in, which weights, which epilogue, what comes out.
+struct Geo { int H, W; };  // resolution of one convolution
+
+struct ConvIO {
+    const void* in16 = nullptr; int in_c = 64;
+    const uint8_t* wpack = nullptr; const float* bias = nullptr;
+    int nout = 32, nslices = 1, nchunks = 1, fmt = 1;
+    int kvalid = 0;  // real input channels (0: every chunk is full)
+    void* out16 = nullptr; int out16_c = 64, out16_choff = 0, out16_fmt = 1, out16_up2 = 0, out16_fixed = 0; unsigned no16_mask = 0;
+    float* outf = nullptr; int outf_c = 64, outf_choff = 0; unsigned noutf_mask = 0;
+    const float* res1 = nullptr; int res1_c = 64, res_choff = 0; unsigned nores_mask = 0;
+    const float* res2 = nullptr; int res2_c = 64; float res2_scale = 1.f;
+    const void* mask16 = nullptr; int mask16_c = 64, mask16_choff = 0, mask16_relu = 0;
+    int ep_mode = EP_PLAIN, lrelu = 0, clamp01 = 0, relu = 0;
+    float out16_scale = 0.f;
+    float* out_nchw = nullptr; float* out_nchw_raw = nullptr; int out_nchw_c = 3;
+};
+int launch_conv_io(int num_sms, const Geo& q, int N, const ConvIO& io, cudaStream_t s);
 // OIHW fp32 -> packed 16-bit tiles (generator.cu). transposed=1 packs the data-gradient convolution
 // W'[ci][co][dy][dx] = W[co][ci][2-dy][2-dx] (cin/cout are the FORWARD channel counts; bias ignored).
 // (re)builds the transposed packs if the handle has them allocated or `force` is set (train.cu)

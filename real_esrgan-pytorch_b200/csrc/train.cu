@@ -134,24 +134,7 @@ static int egrid(size_t total) {
 
 // ================================================================================================ conv launcher
 
-struct Geo { int H, W; };  // resolution of one convolution
-
-struct ConvIO {
-    const void* in16 = nullptr; int in_c = 64;
-    const uint8_t* wpack = nullptr; const float* bias = nullptr;
-    int nout = 32, nslices = 1, nchunks = 1, fmt = 1;
-    int kvalid = 0;  // real input channels (0: every chunk is full)
-    void* out16 = nullptr; int out16_c = 64, out16_choff = 0, out16_fmt = 1, out16_up2 = 0, out16_fixed = 0; unsigned no16_mask = 0;
-    float* outf = nullptr; int outf_c = 64, outf_choff = 0; unsigned noutf_mask = 0;
-    const float* res1 = nullptr; int res1_c = 64, res_choff = 0; unsigned nores_mask = 0;
-    const float* res2 = nullptr; int res2_c = 64; float res2_scale = 1.f;
-    const void* mask16 = nullptr; int mask16_c = 64, mask16_choff = 0;
-    int ep_mode = EP_PLAIN, lrelu = 0, clamp01 = 0;
-    float out16_scale = 0.f;
-    float* out_nchw = nullptr; float* out_nchw_raw = nullptr; int out_nchw_c = 3;
-};
-
-static int launch_conv_io(const resr_generator* g, const Geo& q, int N, const ConvIO& io, cudaStream_t s) {
+int launch_conv_io(int num_sms, const Geo& q, int N, const ConvIO& io, cudaStream_t s) {
     ConvArgs a;
     ConvMaps m;
     memset(&a, 0, sizeof(a));
@@ -160,7 +143,7 @@ static int launch_conv_io(const resr_generator* g, const Geo& q, int N, const Co
     a.nchunks = io.nchunks;
     a.fmt_in = io.fmt;
     a.wpack = io.wpack; a.bias = io.bias;
-    a.ep_mode = io.ep_mode; a.lrelu = io.lrelu; a.clamp01 = io.clamp01;
+    a.ep_mode = io.ep_mode; a.lrelu = io.lrelu; a.clamp01 = io.clamp01; a.relu = io.relu;
     // channels past kvalid are zeros this library wrote: the map may end at the next multiple of 8
     int rc = conv3x3_make_tmap_act(&m.a, io.in16, N, a.H, a.W, io.in_c, a.mode, a.BW, a.BN, (io.kvalid + 7) / 8 * 8);
     if (io.out16) {
@@ -179,12 +162,12 @@ static int launch_conv_io(const resr_generator* g, const Geo& q, int N, const Co
     }
     a.res2 = io.res2; a.res2_cstride = io.res2_c; a.res2_scale = io.res2_scale;
     a.out16_scale = io.out16_scale;
-    a.mask16 = io.mask16; a.mask16_cstride = io.mask16_c; a.mask16_choff = io.mask16_choff;
+    a.mask16 = io.mask16; a.mask16_cstride = io.mask16_c; a.mask16_choff = io.mask16_choff; a.mask16_relu = io.mask16_relu;
     a.out_nchw = io.out_nchw; a.out_nchw_raw = io.out_nchw_raw; a.out_nchw_c = io.out_nchw_c;
     ConvLaunchCfg cfg;  // CTA-pair kernel whenever two column groups can be paired (conv3x3_pair.cu)
     if (!conv3x3_choose(&a, io.nout, io.nslices, &cfg)) rc |= 1 << 20;
     if (rc != 0) return set_error(RESR_E_CUDA, "conv planning failed (%d)", rc);
-    const cudaError_t e = conv3x3_run(m, a, cfg, g->num_sms, s);
+    const cudaError_t e = conv3x3_run(m, a, cfg, num_sms, s);
     if (e != cudaSuccess) return set_error(RESR_E_CUDA, "conv launch: %s", cudaGetErrorString(e));
     return RESR_OK;
 }
@@ -305,7 +288,7 @@ int forward_train(resr_generator* g, const float* x, float* y, int N, int H, int
         ConvIO io = fwd_io(g, k++);
         io.in16 = B.xin; io.in_c = 64;
         io.outf = B.f[0]; io.out16 = B.c[0]; io.out16_c = 192;
-        RESR_TRY(launch_conv_io(g, g0, N, io, s));
+        RESR_TRY(launch_conv_io(g->num_sms, g0, N, io, s));
     }
     for (int i = 0; i < kNumRRDB; ++i) {
         float* X0 = (i == 0) ? B.f[0] : B.f[3];
@@ -316,7 +299,7 @@ int forward_train(resr_generator* g, const float* x, float* y, int N, int H, int
                 ConvIO io = fwd_io(g, k++);
                 io.in16 = B.c[r]; io.in_c = 192; io.lrelu = 1;
                 io.out16 = B.c[r]; io.out16_c = 192; io.out16_choff = 64 + 32 * q;
-                RESR_TRY(launch_conv_io(g, g0, N, io, s));
+                RESR_TRY(launch_conv_io(g->num_sms, g0, N, io, s));
             }
             ConvIO io = fwd_io(g, k++);
             io.in16 = B.c[r]; io.in_c = 192;
@@ -324,34 +307,34 @@ int forward_train(resr_generator* g, const float* x, float* y, int N, int H, int
             if (j < 2) { io.ep_mode = EP_RDB; io.outf = B.f[j + 1]; }
             else { io.ep_mode = EP_RRDB; io.res2 = X0; io.res2_c = 64; io.outf = B.f[3]; }
             io.out16 = B.c[r + 1]; io.out16_c = 192;
-            RESR_TRY(launch_conv_io(g, g0, N, io, s));
+            RESR_TRY(launch_conv_io(g->num_sms, g0, N, io, s));
         }
     }
     {   // conv2 + skip, stored nearest-upsampled x2 (fp16)
         ConvIO io = fwd_io(g, k++);
         io.in16 = B.c[69]; io.in_c = 192; io.ep_mode = EP_SKIP; io.res1 = B.f[0];
         io.out16 = B.t1; io.out16_c = 64; io.out16_up2 = 1;
-        RESR_TRY(launch_conv_io(g, g0, N, io, s));
+        RESR_TRY(launch_conv_io(g->num_sms, g0, N, io, s));
     }
     {
         ConvIO io = fwd_io(g, k++);
         io.in16 = B.t1; io.lrelu = 1; io.out16 = B.t2; io.out16_up2 = 1;
-        RESR_TRY(launch_conv_io(g, g1, N, io, s));
+        RESR_TRY(launch_conv_io(g->num_sms, g1, N, io, s));
     }
     {
         ConvIO io = fwd_io(g, k++);
         io.in16 = B.t2; io.lrelu = 1; io.out16 = B.t3;
-        RESR_TRY(launch_conv_io(g, g2, N, io, s));
+        RESR_TRY(launch_conv_io(g->num_sms, g2, N, io, s));
     }
     {
         ConvIO io = fwd_io(g, k++);
         io.in16 = B.t3; io.lrelu = 1; io.out16 = B.t4;
-        RESR_TRY(launch_conv_io(g, g2, N, io, s));
+        RESR_TRY(launch_conv_io(g->num_sms, g2, N, io, s));
     }
     {
         ConvIO io = fwd_io(g, k++);
         io.in16 = B.t4; io.clamp01 = 1; io.out_nchw = y; io.out_nchw_raw = B.yraw; io.out_nchw_c = 3;
-        RESR_TRY(launch_conv_io(g, g2, N, io, s));
+        RESR_TRY(launch_conv_io(g->num_sms, g2, N, io, s));
     }
     return RESR_OK;
 }
@@ -453,26 +436,26 @@ int backward_common(resr_generator* g, float* grads, int N, int H, int W, const 
     {   // d(T4) masked by LeakyReLU'(conv3 out) -> conv3's dY
         ConvIO io = bwd_io(g, kConv4);
         io.in16 = B.biga; io.out16 = B.bigb; io.mask16 = B.t4;
-        RESR_TRY(launch_conv_io(g, g2, N, io, s));
+        RESR_TRY(launch_conv_io(g->num_sms, g2, N, io, s));
     }
     RESR_TRY(layer_wgrad(g, kConv3, B.t3, 64, B.bigb, N, g2, B, grads, s));
     {
         ConvIO io = bwd_io(g, kConv3);
         io.in16 = B.bigb; io.out16 = B.biga; io.mask16 = B.t3;
-        RESR_TRY(launch_conv_io(g, g2, N, io, s));
+        RESR_TRY(launch_conv_io(g->num_sms, g2, N, io, s));
     }
     RESR_TRY(layer_wgrad(g, kUp2, B.t2, 64, B.biga, N, g2, B, grads, s));
     {   // d(T2) at 4x, masked by LeakyReLU'(up1 out) (T2 holds its upsampled copy), then the 2x2 sum of nearest x2
         ConvIO io = bwd_io(g, kUp2);
         io.in16 = B.biga; io.out16 = B.bigb; io.mask16 = B.t2;
-        RESR_TRY(launch_conv_io(g, g2, N, io, s));
+        RESR_TRY(launch_conv_io(g->num_sms, g2, N, io, s));
         sum2x2_kernel<<<egrid(4 * P * 32), 256, 0, s>>>(B.bigb, nullptr, B.mida, N, 2 * H, 2 * W);
     }
     RESR_TRY(layer_wgrad(g, kUp1, B.t1, 64, B.mida, N, g1, B, grads, s));
     {   // d(T1) at 2x (no activation on the skip sum), 2x2 sum -> d(out) at LR: fp32 (skip branch) + bf16 (conv2's dY)
         ConvIO io = bwd_io(g, kUp1);
         io.in16 = B.mida; io.out16 = B.midb;
-        RESR_TRY(launch_conv_io(g, g1, N, io, s));
+        RESR_TRY(launch_conv_io(g->num_sms, g1, N, io, s));
         sum2x2_kernel<<<egrid(P * 32), 256, 0, s>>>(B.midb, B.dskip, B.dya, N, H, W);
     }
     RESR_TRY(layer_wgrad(g, kConv2, B.c[69], 192, B.dya, N, g0, B, grads, s));
@@ -480,7 +463,7 @@ int backward_common(resr_generator* g, float* grads, int N, int H, int W, const 
         ConvIO io = bwd_io(g, kConv2);
         io.in16 = B.dya; io.outf = B.dx[0];
         io.out16 = B.dycat[(3 * kNumRRDB - 1) % 3]; io.out16_c = 192; io.out16_choff = 0; io.out16_fmt = 1; io.out16_scale = 0.2f * 0.2f;
-        RESR_TRY(launch_conv_io(g, g0, N, io, s));
+        RESR_TRY(launch_conv_io(g->num_sms, g0, N, io, s));
     }
 
     // ---- trunk, RRDB 22 .. 0 (model.py:123-132 and 87-98 backwards)
@@ -532,7 +515,7 @@ int backward_common(resr_generator* g, float* grads, int N, int H, int W, const 
                         io.out16_scale = jj == 2 ? 0.2f * 0.2f : 0.2f;
                     }
                 }
-                RESR_TRY(launch_conv_io(g, g0, N, io, s));
+                RESR_TRY(launch_conv_io(g->num_sms, g0, N, io, s));
             }
             {   // weight + bias gradients of the five layers (side stream): dYcat is complete once conv2's launch is done.
                 // ONE MN-major GEMM straight from the concat buffer and dYcat' (no transposed copies).

@@ -14,7 +14,7 @@ from torch import nn
 
 from . import _lib
 
-__all__ = ["ResidualDenseBlock", "ResidualResidualDenseBlock", "Generator", "plan_tiles", "infer_tiled"]
+__all__ = ["ResidualDenseBlock", "ResidualResidualDenseBlock", "Generator", "ContentLoss", "plan_tiles", "infer_tiled"]
 
 
 _PRECISIONS = {"fp16": 0, "bf16": 1}
@@ -485,3 +485,184 @@ def infer_tiled(gen: "Generator", x: torch.Tensor, tile_h: int = 512, tile_w: in
         out[:, :, s * y0:s * y1, s * x0:s * x1] = piece
         mine.append((s * y0, s * x0, piece))
     return out, mine
+
+
+# ----------------------------------------------------------------------------------------------------------------------
+# VGG19 content loss of the RealESRGAN generator step (reference ContentLoss, model.py:278-335): forward and d/d sr in
+# libresr.so (C ABI resr_vgg_*, include/resr.h).
+
+VGG19_CONV_FEATURES = (0, 2, 5, 7, 10, 12, 14, 16, 19, 21, 23, 25, 28, 30, 32, 34)
+_VGG19_CHANNELS = ((3, 64), (64, 64), (64, 128), (128, 128), (128, 256), (256, 256), (256, 256), (256, 256), (256, 512),
+                   (512, 512), (512, 512), (512, 512), (512, 512), (512, 512), (512, 512), (512, 512))
+_VGG19_POOLS_BEFORE = (0, 0, 1, 1, 2, 2, 2, 2, 3, 3, 3, 3, 4, 4, 4, 4)
+VGG19_CHECKPOINT = "vgg19-dcbb9e9d.pth"   # torchvision's ImageNet weights (models.vgg19(True), reference model.py:296)
+
+
+def parse_vgg19_nodes(nodes):
+    """Node names ("features.<i>") -> features indices, in the caller's order. Only the convolution outputs of
+    vgg19().features are supported; anything else raises ValueError naming the supported nodes."""
+    if isinstance(nodes, str) or len(nodes) == 0:
+        raise ValueError("feature_model_extractor_nodes must be a non-empty list of node names")
+    out = []
+    for name in nodes:
+        idx = None
+        if isinstance(name, str) and name.startswith("features."):
+            tail = name[len("features."):]
+            if tail.isdigit() and str(int(tail)) == tail:
+                idx = int(tail)
+        if idx not in VGG19_CONV_FEATURES:
+            supported = ", ".join(f"features.{i}" for i in VGG19_CONV_FEATURES)
+            raise ValueError(f"unsupported content-loss node {name!r}: the supported nodes are {supported}")
+        if idx in out:
+            raise ValueError(f"content-loss node {name!r} is listed twice")
+        out.append(idx)
+    return out
+
+
+def _vgg19_min_size(features):
+    """Smallest H (and W) that leaves one pixel at the deepest of `features` (2x2 / stride 2 floor pooling)."""
+    return 1 << _VGG19_POOLS_BEFORE[VGG19_CONV_FEATURES.index(max(features))]
+
+
+class _ContentLossFn(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, sr, gt, mod):
+        n, _, h, w = sr.shape
+        src, gtc = sr.detach().contiguous().float(), gt.detach().contiguous().float()
+        mod._ensure_packed()
+        losses = torch.empty(len(mod.nodes), dtype=torch.float32, device=sr.device)
+        wp, wbytes = mod._workspace(n, h, w, sr.device)
+        with torch.cuda.device(sr.device):
+            _lib.check(_lib.lib().resr_vgg_forward(mod._native(), _lib.ptr(src), _lib.ptr(gtc), _lib.ptr(losses), n, h, w, wp,
+                                                   wbytes, _lib.stream_ptr(sr.device)))
+        # the saved activations live in the module's single workspace: stamp this forward (as Generator does)
+        mod._fwd_generation += 1
+        ctx.mod, ctx.shape, ctx.generation, ctx.packed_version = mod, (n, h, w), mod._fwd_generation, mod._packed_version
+        return losses
+
+    @staticmethod
+    def backward(ctx, grad_losses):
+        mod = ctx.mod
+        n, h, w = ctx.shape
+        if mod._fwd_generation != ctx.generation:
+            raise _lib.ResrError(
+                "backward of a stale forward: another forward of this ContentLoss ran in between and overwrote the saved "
+                "activations (one shared workspace per module). Call backward() before the next forward.")
+        if mod._packed_version != ctx.packed_version:
+            raise _lib.ResrError("the VGG weights were repacked between forward and backward (parameters changed)")
+        g = grad_losses.detach().contiguous().float()
+        grad_sr = torch.empty((n, 3, h, w), dtype=torch.float32, device=g.device)
+        wp, wbytes = mod._workspace(n, h, w, g.device)
+        with torch.cuda.device(g.device):
+            _lib.check(_lib.lib().resr_vgg_backward(mod._native(), _lib.ptr(g), _lib.ptr(grad_sr), n, h, w, wp, wbytes,
+                                                    _lib.stream_ptr(g.device)))
+        return grad_sr, None, None
+
+
+class ContentLoss(nn.Module):
+    """VGG19 content loss (reference model.py:278-335). `forward(sr, gt)` returns the 1-D tensor of the per-node L1 losses
+    (mean), in node order; the caller weights and sums them. Semantics are those of torchvision:
+    `create_feature_extractor(vgg19, nodes)` on `Normalize(mean, std)` inputs, so a node other than the deepest is the
+    conv output after the in-place ReLU that follows it, and the deepest node is the raw conv output. The gradient flows
+    to `sr` only; the VGG weights are frozen.
+
+    `vgg`: a torchvision vgg19 module or its state_dict; None loads `vgg19-dcbb9e9d.pth` from
+    `torch.hub.get_dir()/checkpoints` if that file exists and raises FileNotFoundError otherwise (nothing is downloaded).
+    The 16 convolutions are held as `features.<i>` nn.Conv2d modules, so torchvision's state_dict keys load unchanged."""
+
+    def __init__(self, feature_model_extractor_nodes, feature_model_normalize_mean, feature_model_normalize_std, vgg=None):
+        super().__init__()
+        self.nodes = list(feature_model_extractor_nodes)
+        self.features_idx = parse_vgg19_nodes(self.nodes)
+        self.mean = [float(v) for v in feature_model_normalize_mean]
+        self.std = [float(v) for v in feature_model_normalize_std]
+        if len(self.mean) != 3 or len(self.std) != 3:
+            raise ValueError("feature_model_normalize_mean / _std need 3 values (RGB)")
+        if any(s == 0 or s != s for s in self.std):
+            raise ValueError("feature_model_normalize_std must be non-zero")
+        self.features = nn.ModuleDict({str(i): nn.Conv2d(ci, co, 3, 1, 1) for i, (ci, co) in zip(VGG19_CONV_FEATURES, _VGG19_CHANNELS)})
+        if vgg is None:
+            import os
+            path = os.path.join(torch.hub.get_dir(), "checkpoints", VGG19_CHECKPOINT)
+            if not os.path.isfile(path):
+                raise FileNotFoundError(
+                    f"ContentLoss(vgg=None) loads the torchvision VGG19 weights from {path}, which does not exist; place "
+                    f"{VGG19_CHECKPOINT} there or pass vgg= (a torchvision vgg19 module or its state_dict). Nothing is downloaded.")
+            vgg = torch.load(path, map_location="cpu", weights_only=True)
+        sd = vgg.state_dict() if isinstance(vgg, nn.Module) else vgg
+        self.load_state_dict({k: v for k, v in sd.items() if k.startswith("features.")})
+        for p in self.parameters():
+            p.requires_grad_(False)   # reference model.py:301-303: the feature extractor is frozen
+        self._handle = None
+        self._handle_device = None
+        self._packed_version = None
+        self._ws = None
+        self._fwd_generation = 0
+
+    def _device(self):
+        return next(self.parameters()).device
+
+    def _native(self):
+        dev = self._device()
+        if dev.type != "cuda":
+            raise _lib.ResrError("resr_b200.ContentLoss runs on a CUDA (sm_100a) device only; move it with .cuda() / .to(device)")
+        if self._handle is not None and self._handle_device != dev:
+            self._release()
+        if self._handle is None:
+            h = ctypes.c_void_p()
+            feats = (ctypes.c_int * len(self.features_idx))(*self.features_idx)
+            _lib.check(_lib.lib().resr_vgg_create(ctypes.byref(h), feats, len(self.features_idx), (ctypes.c_float * 3)(*self.mean),
+                                                  (ctypes.c_float * 3)(*self.std)))
+            self._handle, self._handle_device = h, dev
+        return self._handle
+
+    def _release(self):
+        with torch.cuda.device(self._handle_device):
+            torch.cuda.synchronize()
+            _lib.lib().resr_vgg_destroy(self._handle)
+        self._handle, self._packed_version, self._ws = None, None, None
+
+    def __del__(self):
+        h = getattr(self, "_handle", None)
+        if h is not None:
+            try:
+                with torch.cuda.device(self._handle_device):
+                    _lib.lib().resr_vgg_destroy(h)
+            except Exception:
+                pass
+
+    def _param_version(self):
+        return tuple((p._version, p.data_ptr(), p.dtype) for p in self.parameters()) + (self._device(),)
+
+    def _ensure_packed(self):
+        ver = self._param_version()
+        if self._packed_version != ver:
+            flat = torch.cat([p.detach().reshape(-1).float() for p in self.parameters()])
+            assert flat.numel() == _lib.lib().resr_vgg_num_params()
+            dev = self._device()
+            h = self._native()
+            with torch.cuda.device(dev):
+                _lib.check(_lib.lib().resr_vgg_load_params(h, _lib.ptr(flat), _lib.stream_ptr(dev)))
+                torch.cuda.current_stream(dev).synchronize()   # `flat` is a temporary
+            self._packed_version = ver
+
+    def _workspace(self, n, h, w, device):
+        need = _lib.lib().resr_vgg_workspace_bytes(self._native(), n, h, w)
+        if need == 0:
+            raise ValueError(_lib.lib().resr_last_error().decode())
+        if self._ws is None or self._ws.numel() < need + 1024 or self._ws.device != device:
+            self._ws = torch.empty(need + 1024, dtype=torch.uint8, device=device)
+        return Generator._aligned(self._ws)
+
+    def forward(self, sr: torch.Tensor, gt: torch.Tensor) -> torch.Tensor:
+        if sr.dim() != 4 or sr.size(1) != 3 or sr.shape != gt.shape:
+            raise ValueError(f"expected sr and gt of one [N, 3, H, W] shape, got {tuple(sr.shape)} and {tuple(gt.shape)}")
+        if not (sr.is_cuda and gt.is_cuda):
+            raise _lib.ResrError("resr_b200.ContentLoss runs on a CUDA (sm_100a) device only; there is no CPU path")
+        if sr.device != self._device() or gt.device != self._device():
+            raise _lib.ResrError(f"inputs on {sr.device} / {gt.device} but the loss lives on {self._device()}")
+        m = _vgg19_min_size(self.features_idx)
+        if sr.size(2) < m or sr.size(3) < m:
+            raise ValueError(f"{sr.size(2)} x {sr.size(3)} leaves no pixel at features.{max(self.features_idx)}: "
+                             f"H and W must be at least {m}")
+        return _ContentLossFn.apply(sr, gt, self)
