@@ -5,6 +5,7 @@
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
+#include <atomic>
 #include <cstring>
 
 #include "conv3x3.cuh"
@@ -358,11 +359,14 @@ static cudaError_t conv3x3_launch_grid(const ConvMaps& maps, const ConvArgs& arg
     const long long nclusters = conv3x3_clusters(units, cluster, nslices, num_sms);
     if (units * (nclusters + 1) >= (1ll << 31)) return cudaErrorInvalidValue;   // the kernel's strip arithmetic is 32-bit
 
-    static PerDevice<bool> attr;  // function attributes are per device
-    if (!attr.cur()) {
+    // Function attributes are per device. Host threads driving different devices (or the same one) may get here at
+    // once: the flag is atomic, and two threads that both see it unset both set the same attribute, which is harmless.
+    static PerDevice<std::atomic<bool>> attr;
+    std::atomic<bool>& done = attr.cur();
+    if (!done.load(std::memory_order_acquire)) {
         const cudaError_t e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax);
         if (e != cudaSuccess) return e;
-        attr.cur() = true;
+        done.store(true, std::memory_order_release);
     }
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof(cfg));

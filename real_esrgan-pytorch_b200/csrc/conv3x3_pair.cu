@@ -405,12 +405,14 @@ static bool plan_smem(ConvArgs* a, int wbytes, int subw, int max_bufs) {
 }
 
 // 0: never pair, 1: pair when the problem is large enough (default), 2: pair whenever two column groups exist
-static int g_pair_policy = -1;
+// Read by every plan, possibly from several host threads at once: an atomic, initialised once from the environment.
+static std::atomic<int>& pair_policy() {
+    static std::atomic<int> p{getenv("RESR_CONV_PAIR") ? atoi(getenv("RESR_CONV_PAIR")) : 1};
+    return p;
+}
 int conv3x3_set_pair_policy(int policy) {
-    if (g_pair_policy < 0) g_pair_policy = getenv("RESR_CONV_PAIR") ? atoi(getenv("RESR_CONV_PAIR")) : 1;
-    const int prev = g_pair_policy;
-    if (policy >= 0 && policy <= 2) g_pair_policy = policy;
-    return prev;
+    std::atomic<int>& p = pair_policy();
+    return policy >= 0 && policy <= 2 ? p.exchange(policy) : p.load();
 }
 
 bool conv3x3_choose(ConvArgs* a, int pack_nout, int pack_nslices, ConvLaunchCfg* cfg) {

@@ -354,14 +354,16 @@ void conv3x3_init_geometry(ConvArgs* a, int N, int H, int W, int cin, int mode) 
 }
 
 PFN_encodeTiled get_encode_fn() {
-    static PFN_encodeTiled fn = nullptr;
-    if (!fn) {
+    // looked up once per process; the initialisation of a function-local static is thread-safe (several host threads
+    // plan forwards at once)
+    static const PFN_encodeTiled fn = [] {
         void* p = nullptr;
         cudaDriverEntryPointQueryResult q;
         if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
             q == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<PFN_encodeTiled>(p);
-    }
+            return reinterpret_cast<PFN_encodeTiled>(p);
+        return static_cast<PFN_encodeTiled>(nullptr);
+    }();
     return fn;
 }
 

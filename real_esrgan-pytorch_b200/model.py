@@ -8,18 +8,36 @@ the reference weights and reference checkpoints load unchanged), but whose forwa
 convolution (`resr_conv3x3`). There is no PyTorch fallback path.
 """
 import ctypes
+import threading
+import time
 
 import torch
 from torch import nn
 
 from . import _lib
 
-__all__ = ["ResidualDenseBlock", "ResidualResidualDenseBlock", "Generator", "ContentLoss", "plan_tiles", "infer_tiled"]
+__all__ = ["ResidualDenseBlock", "ResidualResidualDenseBlock", "Generator", "ContentLoss", "plan_tiles", "infer_tiled",
+           "canvas_groups", "default_band_rows", "deal_groups", "MultiDeviceInference"]
 
 
 _PRECISIONS = {"fp16": 0, "bf16": 1}
 # LR pixels per packed canvas of infer_many: cfg3's 64 x 128 x 128 batch, about 8 GB of workspace in the fp16 recipe
 CANVAS_MAX_PIXELS = 1 << 20
+
+
+def canvas_groups(sizes, max_pixels: int = CANVAS_MAX_PIXELS):
+    """The canvases of Generator.infer_many: lists of indices into `sizes` ((h, w) LR sizes), consecutive images up to
+    `max_pixels` LR pixels per canvas (an image larger than that runs alone)."""
+    groups, cur, px = [], [], 0
+    for i, (hh, ww) in enumerate(sizes):
+        if cur and px + hh * ww > max_pixels:
+            groups.append(cur)
+            cur, px = [], 0
+        cur.append(i)
+        px += hh * ww
+    if cur:
+        groups.append(cur)
+    return groups
 
 
 def _conv(cin: int, cout: int) -> nn.Conv2d:
@@ -422,17 +440,9 @@ class Generator(nn.Module):
         self._ensure_packed()
         h = self._native()
         dev = xs[0].device
-        groups, cur, px = [], [], 0
-        for i, (hh, ww) in enumerate(sizes):   # consecutive images, up to max_pixels LR pixels per canvas
-            if cur and px + hh * ww > max_pixels:
-                groups.append(cur)
-                cur, px = [], 0
-            cur.append(i)
-            px += hh * ww
-        groups.append(cur)
         call = getattr(_lib.lib(), fn)
         with torch.cuda.device(dev):
-            for idx in groups:
+            for idx in canvas_groups(sizes, max_pixels):
                 n = len(idx)
                 hs = (ctypes.c_int * n)(*[sizes[i][0] for i in idx])
                 ws_ = (ctypes.c_int * n)(*[sizes[i][1] for i in idx])
@@ -485,6 +495,286 @@ def infer_tiled(gen: "Generator", x: torch.Tensor, tile_h: int = 512, tile_w: in
         out[:, :, s * y0:s * y1, s * x0:s * x1] = piece
         mine.append((s * y0, s * x0, piece))
     return out, mine
+
+
+# ----------------------------------------------------------------------------------------------------------------------
+# Several GPUs from one process: one Generator replica per device and one host thread per replica for the length of a
+# call. The work is dealt out, never recomputed differently: every band and every canvas is the forward one GPU runs.
+
+
+def default_band_rows(h: int, w: int, replicas: int, max_pixels: int = CANVAS_MAX_PIXELS) -> int:
+    """Interior LR rows per full-width band of MultiDeviceInference.infer_large: at least two bands per replica whenever
+    h >= 2 * replicas (a replica uploads band k + 1 while band k computes), and at most `max_pixels` LR pixels per band
+    interior (the forward's workspace grows with the band, about 8 KB per LR pixel)."""
+    return max(1, min(h // (2 * replicas), max_pixels // w))
+
+
+def deal_groups(sizes, replicas: int, max_pixels: int = CANVAS_MAX_PIXELS):
+    """The canvases of a list of (h, w) LR sizes (canvas_groups: the canvases Generator.infer_many runs) dealt to
+    `replicas`: largest canvas (in LR pixels) first, onto the replica with the least work so far; ties go to the earlier
+    canvas and the lower replica. Returns (groups, dealt): dealt[r] lists the indices into `groups` replica r runs."""
+    groups = canvas_groups(sizes, max_pixels)
+    work = [sum(sizes[i][0] * sizes[i][1] for i in g) for g in groups]
+    load, dealt = [0] * replicas, [[] for _ in range(replicas)]
+    for k in sorted(range(len(groups)), key=lambda k: (-work[k], k)):
+        r = min(range(replicas), key=lambda r: (load[r], r))
+        dealt[r].append(k)
+        load[r] += work[k]
+    return groups, dealt
+
+
+class MultiDeviceInference:
+    """Inference of one Generator on several GPUs from one process: a large image as full-width halo bands
+    (infer_large / infer_u8_large) or a list of images as packed canvases (infer_many / infer_u8_many), dealt to one
+    replica of `gen` per entry of `devices` (default: every visible CUDA device). Entries may repeat: [0, 0] runs two
+    replicas on one GPU. Inputs are host tensors (pinned or not) or CUDA tensors on any device; results are written to
+    page-locked host memory.
+
+    Every replica is an ordinary Generator on its device with gen's precision recipe and static weights. Each call
+    compares gen's weights with the ones the replicas hold and reloads them when they changed (an optimizer step,
+    EMA.apply_shadow); when gen.assume_static_weights() is set that walk is skipped, and invalidate() forces a reload.
+    A call runs one host thread per replica, each with its device current and on the replica's own streams (compute,
+    upload, download), and joins them all before it returns. ctypes releases the GIL around every library call, so the
+    launches to different GPUs are enqueued in parallel. If a replica fails, every thread is still joined, then the
+    first error is raised naming the replica's device; the contents of the output are unspecified in that case.
+
+    `last_enqueue` holds, per replica of the last call, (device, bands or canvases, host seconds spent enqueuing them)."""
+
+    def __init__(self, gen: Generator, devices=None):
+        if not isinstance(gen, Generator):
+            raise ValueError(f"expected a resr_b200 Generator, got {type(gen).__name__}")
+        if devices is not None:
+            devices = [torch.device("cuda", d) if isinstance(d, int) else torch.device(d) for d in devices]
+            if not devices or any(d.type != "cuda" or d.index is None for d in devices):
+                raise ValueError(f"devices must be a non-empty list of CUDA device indices, got {devices}")
+        self.gen = gen
+        self.devices = devices
+        self._replicas = None
+        self._streams = None
+        self._loaded = None
+        self.last_enqueue = None
+
+    def invalidate(self):
+        """Reload the replicas' weights from gen on the next call (for a gen with assume_static_weights set)."""
+        self._loaded = None
+
+    # ------------------------------------------------------------------ large images
+    @torch.no_grad()
+    def infer_large(self, x: torch.Tensor, out: torch.Tensor = None, band_rows: int = None, halo: int = 16) -> torch.Tensor:
+        """SR of one fp32 [1, 3, H, W] image into `out`, a page-locked host tensor [1, 3, 4H, 4W] (allocated if None;
+        callers that loop pass their own: pinning 805 MB costs more than the forward of a 2048^2 image).
+
+        The image is cut into full-width bands plan_tiles(H, W, band_rows, W, halo) (band_rows: default_band_rows),
+        dealt round-robin to the replicas in infer_tiled's order. Per band: one upload of the window rows per channel
+        plane, the replica's infer(), and one download per channel plane of the interior rows straight into `out`.
+
+        The result is torch.equal to infer_tiled(gen, x, band_rows, W, halo)[0] on one GPU: every band is the same
+        forward at the same shape with the same kernels. That holds across devices of one GPU model, because a forward's
+        plan depends only on the shape, the SM count and the pair policy. Against the whole-image forward the error is
+        infer_tiled's (DESIGN §6)."""
+        if x.dim() != 4 or x.size(0) != 1 or x.size(1) != 3 or x.dtype != torch.float32:
+            raise ValueError(f"expected a float32 [1, 3, H, W] image, got {tuple(x.shape)} {x.dtype}")
+        return self._large(x, out, band_rows, halo, u8=False)
+
+    @torch.no_grad()
+    def infer_u8_large(self, img: torch.Tensor, out: torch.Tensor = None, band_rows: int = None, halo: int = 16) -> torch.Tensor:
+        """infer_large for a uint8 [H, W, 3] image (what cv2.imread + cvtColor hold) into a page-locked uint8
+        [4H, 4W, 3] host tensor: per band one upload of the window rows, infer_u8(), one download of the interior rows.
+        Equal to assembling Generator.infer_u8 of the same bands on one GPU."""
+        if img.dim() != 3 or img.size(2) != 3 or img.dtype != torch.uint8:
+            raise ValueError(f"expected a uint8 [H, W, 3] image, got {tuple(img.shape)} {img.dtype}")
+        return self._large(img, out, band_rows, halo, u8=True)
+
+    def _large(self, x, out, band_rows, halo, u8):
+        h, w = (x.size(0), x.size(1)) if u8 else (x.size(2), x.size(3))
+        if h == 0 or w == 0:
+            raise ValueError(f"empty image {tuple(x.shape)}")
+        if band_rows is not None and band_rows < 1 or halo < 0:
+            raise ValueError(f"band_rows must be >= 1 and halo >= 0, got {band_rows} and {halo}")
+        shape = (4 * h, 4 * w, 3) if u8 else (1, 3, 4 * h, 4 * w)
+        if out is not None and (tuple(out.shape) != shape or out.dtype != x.dtype or out.is_cuda or not out.is_contiguous()):
+            raise ValueError(f"out must be a contiguous {x.dtype} host tensor of shape {shape}, got {tuple(out.shape)} "
+                             f"{out.dtype} on {out.device}")
+        self._check_devices()
+        if out is not None and not out.is_pinned():
+            raise ValueError("out must be page-locked host memory (tensor.pin_memory())")
+        self._prepare()
+        if out is None:
+            out = torch.empty(shape, dtype=x.dtype, pin_memory=True)
+        nrep = len(self._replicas)
+        bands = plan_tiles(h, w, band_rows or default_band_rows(h, w, nrep), w, halo)
+        x = x.detach().contiguous()
+        if x.is_cuda:
+            torch.cuda.current_stream(x.device).synchronize()   # the caller's work on x is done before the copies
+        self._run(lambda rep, streams, mine: _run_bands(rep, streams, mine, x, out, u8), [bands[r::nrep] for r in range(nrep)])
+        return out
+
+    # ------------------------------------------------------------------ lists of differently sized images
+    @torch.no_grad()
+    def infer_many(self, images, max_pixels: int = CANVAS_MAX_PIXELS):
+        """Generator.infer_many on several GPUs: floating-point [1, 3, h, w] or [3, h, w] images, host or CUDA, in; one
+        page-locked fp32 host tensor per image ([1, 3, 4h, 4w] or [3, 4h, 4w]) out, in input order. The canvases are
+        canvas_groups(...) of the list, dealt by deal_groups, so each result is torch.equal to the matching element of
+        gen.infer_many(images, max_pixels) on one GPU."""
+        for x in images:
+            if x.dim() not in (3, 4) or x.size(-3) != 3 or (x.dim() == 4 and x.size(0) != 1) or not x.is_floating_point():
+                raise ValueError(f"expected a floating-point [1, 3, H, W] or [3, H, W] image, got {tuple(x.shape)} {x.dtype}")
+        return self._many(list(images), [tuple(x.shape[-2:]) for x in images], max_pixels, u8=False)
+
+    @torch.no_grad()
+    def infer_u8_many(self, images_u8, max_pixels: int = CANVAS_MAX_PIXELS):
+        """infer_many for uint8 [h, w, 3] images: page-locked uint8 [4h, 4w, 3] results in input order, each torch.equal
+        to the matching element of gen.infer_u8_many(images_u8, max_pixels) on one GPU."""
+        for x in images_u8:
+            if x.dim() != 3 or x.size(2) != 3 or x.dtype != torch.uint8:
+                raise ValueError(f"expected a uint8 [H, W, 3] image, got {tuple(x.shape)} {x.dtype}")
+        return self._many(list(images_u8), [tuple(x.shape[:2]) for x in images_u8], max_pixels, u8=True)
+
+    def _many(self, xs, sizes, max_pixels, u8):
+        if not xs:
+            raise ValueError("empty image list")
+        if any(hh == 0 or ww == 0 for hh, ww in sizes):
+            raise ValueError(f"empty image among {sizes}")
+        if max_pixels < 1:
+            raise ValueError(f"max_pixels must be >= 1, got {max_pixels}")
+        self._check_devices()
+        self._prepare()
+        outs = [torch.empty((4 * x.size(0), 4 * x.size(1), 3) if u8 else x.shape[:-2] + (4 * x.size(-2), 4 * x.size(-1)),
+                            dtype=torch.uint8 if u8 else torch.float32, pin_memory=True) for x in xs]
+        for dev in {x.device for x in xs if x.is_cuda}:
+            torch.cuda.current_stream(dev).synchronize()   # the caller's work on the inputs is done before the copies
+        groups, dealt = deal_groups(sizes, len(self._replicas), max_pixels)
+        self._run(lambda rep, streams, mine: _run_canvases(rep, streams, mine, xs, outs, max_pixels, u8),
+                  [[groups[k] for k in d] for d in dealt])
+        return outs
+
+    # ------------------------------------------------------------------ replicas and threads
+    def _check_devices(self):
+        if not torch.cuda.is_available():
+            raise _lib.ResrError("MultiDeviceInference needs CUDA (sm_100a) devices; none is visible")
+        count = torch.cuda.device_count()
+        if self.devices is None:
+            self.devices = [torch.device("cuda", i) for i in range(count)]
+        for d in self.devices:
+            if d.index >= count:
+                raise _lib.ResrError(f"{d} is not visible ({count} CUDA device(s))")
+
+    def _prepare(self):
+        """Builds the replicas once and brings their weights up to date with gen's."""
+        gen = self.gen
+        _lib.lib()   # loaded here, not by racing worker threads
+        if self._replicas is None:
+            self._replicas = [self._replica(d) for d in self.devices]
+            self._streams = [tuple(torch.cuda.Stream(d) for _ in range(3)) for d in self.devices]
+        if self._loaded is not None and gen._static_weights and self._loaded[1] == gen.precision:
+            return
+        ver = (gen._param_version(), gen.precision)
+        if ver != self._loaded:
+            flat = gen.flat_parameters()
+            for rep, d in zip(self._replicas, self.devices):
+                rep.set_precision(gen.precision)
+                with torch.cuda.device(d):
+                    rep._flat_master.copy_(flat)
+                rep.invalidate()
+            for d in set(self.devices):
+                torch.cuda.synchronize(d)   # the workers pack from these vectors on their own streams
+            self._loaded = ver
+
+    @staticmethod
+    def _replica(dev) -> Generator:
+        with torch.device("meta"):
+            rep = Generator(3, 3, 4)   # on meta: no initialisation, no draw from the global RNG
+        rep = rep.to_empty(device=dev).eval().requires_grad_(False)
+        flat = torch.empty(_lib.lib().resr_generator_num_params(), dtype=torch.float32, device=dev)
+        off = 0
+        for p in rep.parameters():
+            p.data = flat[off:off + p.numel()].view_as(p)
+            off += p.numel()
+        rep._flat_master = flat   # the replica packs straight from this vector (Generator._ensure_packed)
+        return rep.assume_static_weights(True)
+
+    def _run(self, job, work):
+        """job(replica, (compute, upload, download) streams, items) on one thread per replica with work; all joined."""
+        n = len(self._replicas)
+        errors, spent = [None] * n, [0.0] * n
+
+        def worker(r):
+            streams = self._streams[r]
+            try:
+                with torch.cuda.device(self.devices[r]), torch.cuda.stream(streams[0]):
+                    try:
+                        t0 = time.perf_counter()
+                        job(self._replicas[r], streams, work[r])
+                        spent[r] = time.perf_counter() - t0
+                    finally:
+                        for s in streams:
+                            s.synchronize()
+            except BaseException as e:   # noqa: B036 -- handed to the calling thread
+                errors[r] = e
+
+        threads = [threading.Thread(target=worker, args=(r,), name=f"resr-replica-{r}") for r in range(n) if work[r]]
+        try:
+            for t in threads:
+                t.start()
+        finally:
+            for t in threads:
+                if t.ident is not None:
+                    t.join()
+        self.last_enqueue = [(self.devices[r], len(work[r]), spent[r]) for r in range(n)]
+        for r, e in enumerate(errors):
+            if e is not None:
+                raise _lib.ResrError(f"replica {r} on {self.devices[r]} failed: {type(e).__name__}: {e}") from e
+
+
+def _run_bands(rep, streams, bands, x, out, u8):
+    """One replica's bands: upload band k + 1 (upload stream) while band k computes (compute stream) and band k - 1
+    downloads (download stream). Two window slots; events order each slot's reuse."""
+    s, up, down = streams
+    w = x.size(1) if u8 else x.size(3)
+    most = max(b[5] - b[4] for b in bands) * 3 * w
+    slots = [torch.empty(most, dtype=x.dtype, device=s.device) for _ in range(2)]
+    landed, read = [torch.cuda.Event() for _ in range(2)], [torch.cuda.Event() for _ in range(2)]
+    for k, (y0, y1, _, _, wy0, wy1, _, _) in enumerate(bands):
+        i, rows = k % 2, wy1 - wy0
+        if k >= 2:
+            up.wait_event(read[i])   # the forward of band k - 2 has read this slot
+        with torch.cuda.stream(up):
+            if u8:
+                win = slots[i][:rows * w * 3].view(1, rows, w, 3)
+                win[0].copy_(x[wy0:wy1], non_blocking=True)
+            else:
+                win = slots[i][:3 * rows * w].view(1, 3, rows, w)
+                for c in range(3):
+                    win[0, c].copy_(x[0, c, wy0:wy1], non_blocking=True)
+            landed[i].record(up)
+        s.wait_event(landed[i])
+        y = rep.infer_u8(win) if u8 else rep.infer(win)
+        read[i].record(s)
+        down.wait_event(read[i])
+        oy, n = 4 * (y0 - wy0), 4 * (y1 - y0)
+        with torch.cuda.stream(down):
+            if u8:
+                out[4 * y0:4 * y1].copy_(y[0, oy:oy + n], non_blocking=True)
+            else:
+                for c in range(3):
+                    out[0, c, 4 * y0:4 * y1].copy_(y[0, c, oy:oy + n], non_blocking=True)
+        y.record_stream(down)   # the next band's output must not take this memory before the download has read it
+
+
+def _run_canvases(rep, streams, groups, xs, outs, max_pixels, u8):
+    """One replica's canvases: inputs to the device on the compute stream, results downloaded on the download stream
+    while the next canvas computes."""
+    s, _, down = streams
+    for idx in groups:
+        src = [xs[i].to(s.device, non_blocking=True) for i in idx]
+        # one canvas: the group fits max_pixels (or is one image), so infer_many regroups it into itself
+        ys = rep.infer_u8_many(src, max_pixels) if u8 else rep.infer_many(src, max_pixels)
+        down.wait_stream(s)
+        with torch.cuda.stream(down):
+            for i, y in zip(idx, ys):
+                outs[i].copy_(y, non_blocking=True)
+        for y in ys:
+            y.record_stream(down)
 
 
 # ----------------------------------------------------------------------------------------------------------------------
